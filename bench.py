@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # CUDA path (this repo)
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host cores
     python bench.py --workload c4|c5 ...                      # BASELINE.json configs[3] / configs[4] instead of configs[1]
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's results as DIR/<name>.npy
 
 A "step" is one pass of analyze_audio over one batch of synthetic tracks.  Default workload C2 = BASELINE.json configs[1]:
 1024 three-minute 44.1 kHz tracks per B200 (BPM 70-180, random keys; SURVEY.md §8d).  The batch is generated ON the device
@@ -291,6 +292,56 @@ def pinned_empty(torch, n_elems: int, np_dtype):
         return None
 
 
+DUMP_CAP_BYTES = 60_000_000  # data bytes; with the .npy headers the dump stays below 64 MB
+# per-track scalars of StratumResult; processing_time_ms is left out: it is a wall time and differs from run to run
+DUMP_SCALARS = ("status", "bpm", "bpm_confidence", "key_is_minor", "key_index", "key_confidence", "key_clarity", "grid_stability",
+                "duration_seconds", "sample_rate", "onset_method_consensus", "warnings", "flags", "tempogram_multi_res_triggered",
+                "tempogram_multi_res_used", "tempogram_percussive_triggered", "tempogram_percussive_used", "trim_start", "trim_end",
+                "time_sig_beats_per_bar", "beats_refined", "n_tempogram_candidates")
+# per-track arrays: (pointer field, count field, dtype written)
+DUMP_ARRAYS = (("beats", "n_beats", np.float32), ("downbeats", "n_downbeats", np.float32), ("bars", "n_bars", np.float32),
+               ("onsets", "n_onsets", np.float64), ("hmm_beat_frames", "n_hmm_beat_frames", np.float64))
+
+
+def dump_outputs(results, out_dir, seed: int = 0) -> int:
+    """Writes the StratumResult array of one batch call as out_dir/<name>.npy, for comparing two builds output for output.
+
+    Scalars are one float64 per track (integers stay exact).  A per-track array is written concatenated in track order with
+    <name>_offsets.npy (track i = <name>[offsets[i]:offsets[i+1]]); tempogram_candidates has one row of (bpm, score, fft_norm,
+    autocorr_norm, selected) per candidate.  An array that no track returned is not written: tempogram candidates, for one, exist only
+    when the configuration emits them (n_tempogram_candidates is -1 otherwise).  If the whole batch exceeds DUMP_CAP_BYTES, a fixed,
+    seeded sample of tracks is written; track_index.npy names the tracks written.  Returns the number of bytes written."""
+    def arr(r, ptr, n, dtype):
+        return np.ctypeslib.as_array(getattr(r, ptr), shape=(n,)).astype(dtype) if n and getattr(r, ptr) else np.zeros(0, dtype)
+
+    def cands(r):
+        n = max(r.n_tempogram_candidates, 0)
+        return np.array([[c.bpm, c.score, c.fft_norm, c.autocorr_norm, c.selected] for c in r.tempogram_candidates[:n]], np.float32).reshape(n, 5)
+
+    n = len(results)
+    per_track = np.array([8 * (len(DUMP_SCALARS) + 1 + 6) + 4 * (r.n_beats + r.n_downbeats + r.n_bars) + 8 * (r.n_onsets + r.n_hmm_beat_frames)
+                          + 20 * max(r.n_tempogram_candidates, 0) for r in results], np.int64)
+    idx = np.arange(n)
+    if per_track.sum() > DUMP_CAP_BYTES:
+        order = np.random.default_rng(seed).permutation(n)
+        idx = np.sort(order[np.cumsum(per_track[order]) <= DUMP_CAP_BYTES])
+    picked = [results[int(i)] for i in idx]
+    out = {"track_index": idx.astype(np.float64)}
+    for f in DUMP_SCALARS:
+        out[f] = np.array([getattr(r, f) for r in picked], np.float64)
+    parts = {f: [arr(r, f, getattr(r, cnt), dt) for r in picked] for f, cnt, dt in DUMP_ARRAYS}
+    parts["tempogram_candidates"] = [cands(r) for r in picked]
+    for f, p in parts.items():
+        if sum(len(a) for a in p) == 0:
+            continue
+        out[f"{f}_offsets"] = np.concatenate([[0], np.cumsum([len(a) for a in p])]).astype(np.float64)
+        out[f] = np.concatenate(p)
+    Path(out_dir).mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(Path(out_dir) / f"{name}.npy", a)
+    return sum(a.nbytes for a in out.values())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -303,7 +354,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-multi-device-call", action="store_true", help="skip the one-process, one-call multi-device e2e leg at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (rank 0's tracks) as DIR/<name>.npy; the inputs are the same on every run")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's results; the reference arm has none to write")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -387,6 +444,8 @@ def main():
         if r.status == 0 and b > 0 and min(abs(b - t), abs(2 * b - t), abs(b - 2 * t)) <= tol:
             bpm_hit += 1
     n_escalated = sum(1 for r in last if r.status == 0 and r.tempogram_multi_res_triggered == 1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
     S.free_results(last)
     L = S.lib()
     L.stratum_b200_fp32_peak_tflops.restype = C.c_double
@@ -434,7 +493,7 @@ def main():
         h0, d0 = S.transfer_bytes()
         barrier()
         te0 = time.perf_counter()
-        e_steps = max(1, min(args.steps, 3))
+        e_steps = args.steps
         for _ in range(e_steps):
             host_step()
         barrier()
@@ -661,7 +720,7 @@ def multi_device_call(S, torch, wl, world, ne, args):
         return n_ok
 
     call()  # warm-up: contexts, arenas and staging buffers of every device
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps
     h0, d0 = S.transfer_bytes()
     t0 = time.perf_counter()
     n_ok = 0

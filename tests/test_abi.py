@@ -120,13 +120,6 @@ def test_metadata_literals_are_the_reference_literals():
     # AnalysisMetadata fields the wrappers synthesise (the C result carries the numbers): quoted from the reference
     assert S.ALGORITHM_VERSION == "0.1.0-alpha"  # src/lib.rs:1603
     assert list(S.METHODS_USED) == ["energy_flux", "chroma_extraction", "key_detection"]  # src/lib.rs:1604-1608
-    ref = ROOT.parent / "reference" / "src" / "lib.rs"
-    if ref.exists():  # this container only; the literals above are what the GPU box checks
-        txt = ref.read_text()
-        blk = txt[txt.index("methods_used: vec!["):]
-        blk = blk[:blk.index("]")]
-        assert re.findall(r'"([a-z_]+)"\.to_string\(\)', blk) == list(S.METHODS_USED)
-        assert 'algorithm_version: "0.1.0-alpha".to_string()' in txt
     rs = (ROOT / "rust" / "stratum-dsp-b200" / "src" / "lib.rs").read_text()
     assert 'vec!["energy_flux".to_string(), "chroma_extraction".to_string(), "key_detection".to_string()]' in rs
     assert 'algorithm_version: "0.1.0-alpha".to_string()' in rs

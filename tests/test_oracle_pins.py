@@ -1,24 +1,12 @@
 """Pins the CPU oracle to every known answer the reference's own tests hold for this path
 (SURVEY.md §8c).  The Rust reference cannot be built here, so these are the anchors."""
 import ctypes as C
-import wave
-from pathlib import Path
 
 import numpy as np
 import pytest
 
 import oracle_lib as O
 import synth
-
-REF_FIXTURES = Path("/root/reference/tests/fixtures")
-
-
-def _wav(path):
-    with wave.open(str(path), "rb") as w:
-        assert w.getnchannels() == 1 and w.getsampwidth() == 2
-        sr = w.getframerate()
-        x = np.frombuffer(w.readframes(w.getnframes()), dtype="<i2").astype(np.float32) / 32768.0
-    return x, sr
 
 
 # ---- tests/integration_tests.rs:46-275 on re-created fixtures (scripts/generate_fixtures.py) ----------
@@ -56,19 +44,6 @@ def test_all_silence_is_an_error():
 def test_empty_and_bad_rate():
     assert O.analyze(np.zeros(0, np.float32), 44100).status == 1  # lib.rs:100-104
     assert O.analyze(np.ones(10, np.float32), 0).status == 1  # lib.rs:106-110
-
-
-@pytest.mark.skipif(not REF_FIXTURES.exists(), reason="reference checkout not present (GPU box)")
-@pytest.mark.parametrize("name,check", [
-    ("120bpm_4bar.wav", lambda r: r.bpm == 0 or abs(r.bpm - 120) <= 2),
-    ("128bpm_4bar.wav", lambda r: r.bpm == 0 or abs(r.bpm - 128) <= 2),
-    ("cmajor_scale.wav", lambda r: r.key == 0 or r.key_confidence < 0.3),
-    ("mixed_silence.wav", lambda r: 4.0 <= r.duration_seconds <= 6.0),
-])
-def test_reference_wav_fixtures(name, check):
-    x, sr = _wav(REF_FIXTURES / name)
-    r = O.analyze(x, sr)
-    assert r.status == 0 and check(r)
 
 
 def test_criterion_bench_shape_returns():
