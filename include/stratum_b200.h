@@ -293,6 +293,12 @@ uint32_t stratum_b200_debug_plan_waves(const uint64_t* offsets, const uint32_t* 
  * starts (padded to 256).  Lets the chunking be tested without a GPU. */
 void stratum_b200_debug_mel_schedule(const int32_t* mel_off, uint32_t n_mels, int32_t* schedule256);
 
+/* Host-side BPM hypothesis grid on its own (no device work; csrc/engine.cu: bpm_grid): the values of the reference's f32 loop
+ * `bpm = min_bpm; while bpm <= max_bpm { ..; bpm += bpm_resolution }` (tempogram_autocorr.rs:79-178).  Writes the first
+ * min(count, cap) values to out (may be NULL) and returns the count, or -1 for an invalid range or a grid of more than 32768
+ * hypotheses (which includes every grid whose accumulation stalls).  Such grids are rejected with STRATUM_NOT_IMPLEMENTED. */
+int32_t stratum_b200_debug_bpm_grid(float min_bpm, float max_bpm, float bpm_resolution, float* out, int32_t cap);
+
 /* Per-stage device time (ms) accumulated since the last reset; names newline separated. */
 int32_t stratum_b200_stage_times(char* names, size_t cap, double* ms, int32_t max_stages);
 void stratum_b200_stage_times_reset(void);

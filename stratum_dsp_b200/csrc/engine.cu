@@ -9,6 +9,7 @@
 // hop-256 / hop-1024 spectrograms and processed as a compacted sub-batch.
 // There is no CPU fallback: without a usable CUDA device every compute entry point fails.
 #include <algorithm>
+#include <array>
 #include <atomic>
 #include <chrono>
 #include <condition_variable>
@@ -218,6 +219,7 @@ struct DeviceCtx {
     std::vector<void*> owned;                 // table allocations
     std::map<uint32_t, float2*> tw_tables;    // size -> TW table (Stockham twiddles, oracle/so_fft.cpp)
     std::map<uint32_t, const float*> hann_tables;  // frame size -> Hann window of the generic STFT
+    std::map<std::array<float, 3>, const float*> bpm_tabs;  // (min_bpm, max_bpm, bpm_resolution) -> hypothesis table of a fine BPM grid
     std::vector<SrTables> sr_host;
     std::vector<StratumConfig> sr_cfg;        // configuration each sr_host entry was built for (the tables depend on it)
     SrTables* d_srtab = nullptr;
@@ -370,6 +372,34 @@ static GenStft get_gen_stft(DeviceCtx& c, uint32_t n) {
     g.rw = get_tw(c, n);
     g.n = (g.win && g.tw && g.rw) ? n : 0;
     return g;
+}
+
+// The BPM hypotheses of the reference's grid loops, `bpm = min_bpm; while bpm <= limit { ..; bpm += bpm_resolution }` in f32:
+// limit = max_bpm in the autocorrelation tempogram (tempogram_autocorr.rs:79-178), max_bpm + 1e-10 in the comb filterbank
+// (comb_filter.rs:96-215).  The count and the values come from the accumulation, not from (max - min) / res: 40..240 at 0.1 gives
+// 2000 hypotheses, and at 0.01 the last values are 5 steps away from min + i * res.  Writes the first min(count, cap) values and
+// returns the count, or -1 beyond BPM_GRID_MAX hypotheses.  That includes every grid whose accumulation stalls (bpm_resolution
+// below half an ulp of bpm), on which the reference never terminates.
+static int bpm_grid(float min_bpm, float limit, float res, float* out, int cap) {
+    int n = 0;
+    for (float bpm = min_bpm; bpm <= limit; bpm = bpm + res) {
+        if (n == BPM_GRID_MAX) return -1;
+        if (n < cap) out[n] = bpm;
+        ++n;
+    }
+    return n;
+}
+
+// Hypothesis table of a fine BPM grid (the comb filterbank's loop: it covers the tempogram's), uploaded once per grid.
+static const float* get_bpm_tab(DeviceCtx& c, const DevCfg& d) {
+    const std::array<float, 3> key{d.min_bpm, d.max_bpm, d.bpm_resolution};
+    auto it = c.bpm_tabs.find(key);
+    if (it != c.bpm_tabs.end()) return it->second;
+    std::vector<float> tab(std::max(d.n_bpm, d.n_comb));
+    bpm_grid(d.min_bpm, d.max_bpm + 1e-10f, d.bpm_resolution, tab.data(), (int)tab.size());
+    const float* p = dev_upload(c, tab);
+    if (p) c.bpm_tabs[key] = p;
+    return p;
 }
 
 static int ctx_init(DeviceCtx& c, int device) {
@@ -941,7 +971,9 @@ static int config_validate(const StratumConfig& c) {
         set_error("Invalid BPM range");
         return STRATUM_INVALID_INPUT;
     }
-    if ((c.max_bpm - c.min_bpm) / c.bpm_resolution > 250.0f) return ni("more than 256 BPM hypotheses");
+    // the comb filterbank's loop bound is the larger one, so its count bounds both grids
+    if (bpm_grid(c.min_bpm, c.max_bpm + 1e-10f, c.bpm_resolution, nullptr, 0) < 0)
+        return ni(("more than " + std::to_string(BPM_GRID_MAX) + " BPM hypotheses (bpm_resolution too fine for the BPM range)").c_str());
     if (!(c.onset_threshold_percentile >= 0.0f && c.onset_threshold_percentile <= 1.0f)) {
         set_error("Threshold percentile must be in [0, 1]");
         return STRATUM_INVALID_INPUT;
@@ -958,6 +990,10 @@ static DevCfg make_devcfg(const StratumConfig& c) {
     d.min_bpm = c.min_bpm;
     d.max_bpm = c.max_bpm;
     d.bpm_resolution = c.bpm_resolution;
+    d.n_bpm = (uint32_t)std::max(bpm_grid(c.min_bpm, c.max_bpm, c.bpm_resolution, nullptr, 0), 0);
+    d.n_comb = (uint32_t)std::max(bpm_grid(c.min_bpm, c.max_bpm + 1e-10f, c.bpm_resolution, nullptr, 0), 0);
+    d.ac_stride = std::max<uint32_t>(AC_CAP, d.n_bpm);
+    d.bpm_tab = nullptr;  // device table: Session::open, for grids of more than AC_CAP hypotheses
     d.silence_thr_linear = powf(10.0f, c.min_amplitude_db / 20.0f);
     d.silence_min_ms = 500;
     d.energy_thr_mul = powf(10.0f, -20.0f / 20.0f);
@@ -1090,7 +1126,7 @@ struct Bump {
     }
 };
 
-static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, bool with_spec = true) {
+static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, uint32_t ac_stride, bool with_spec = true) {
     H.fmax = fcap;
     H.hop = hop;
     H.fft_cap = std::max<uint32_t>(next_pow2_u32(fcap > 1 ? fcap - 1 : 1), 4);
@@ -1099,26 +1135,25 @@ static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, bool w
     H.pair = fa.take((uint64_t)PAIR_Q * fcap);
     H.nov = fa.take((uint64_t)MAX_VARIANTS * fcap);
     H.tgfft = fa.take((uint64_t)MAX_VARIANTS * (H.fft_cap / 2 + 1));
-    H.tgac = fa.take((uint64_t)MAX_VARIANTS * AC_CAP);
+    H.tgac = fa.take((uint64_t)MAX_VARIANTS * ac_stride);
     H.tgwork = fa.take((uint64_t)MAX_VARIANTS * 2 * H.fft_cap);
     H.tgtw = nullptr;
     H.pad_ = 0;
 }
 
 // Base (always needed) work areas of one track.
-static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumConfig& cfg) {
+static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumConfig& cfg, const DevCfg& kd) {
     const uint64_t n = T.n;
     const uint32_t F512 = frames_of(n, 2048, 512), F256 = frames_of(n, 2048, 256), F1024 = frames_of(n, 2048, 1024);
-    const DevCfg kd = make_devcfg(cfg);
     const uint32_t Fk = frames_of(n, kd.key_frame, kd.key_hop);
     const uint32_t Fsil = n >= 2048 ? frames_of(n, 2048, 1024) : 1;
     const uint32_t Fb = frames_of(n, 2048, kd.hop);  // frames of the base path (= F512 at the default hop_size)
     T.fall = std::max(std::max(std::max(F256, F512), std::max(F1024, 1u)), Fb);
     T.fkmax = Fk;
-    plan_hop(fa, T.hop[0], std::max(F512, 1u), 512);
+    plan_hop(fa, T.hop[0], std::max(F512, 1u), 512, kd.ac_stride);
     T.cands[0] = fa.take((uint64_t)MAX_CANDS * 4);
     if (kd.bs != 0) {  // hop_size other than 512: the base path gets a slot of its own
-        plan_hop(fa, T.hop[SLOT_BASE_ALT], std::max(Fb, 1u), kd.hop);
+        plan_hop(fa, T.hop[SLOT_BASE_ALT], std::max(Fb, 1u), kd.hop, kd.ac_stride);
         T.cands[SLOT_BASE_ALT] = fa.take((uint64_t)MAX_CANDS * 4);
     }
     T.sil_rms = fa.take(Fsil + 1);
@@ -1168,7 +1203,7 @@ static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumC
             T.hpss_h[q] = fa.take((uint64_t)std::max(Fb, 1u) * 1025);
             T.hpss_p[q] = fa.take((uint64_t)std::max(Fb, 1u) * 1025);
         }
-        plan_hop(fa, T.hop[SLOT_PERC], std::max(Fb, 1u), kd.hop, false);
+        plan_hop(fa, T.hop[SLOT_PERC], std::max(Fb, 1u), kd.hop, kd.ac_stride, false);
         T.cands[SLOT_PERC] = fa.take((uint64_t)MAX_CANDS * 4);
     }
     T.on_final = ia.take((uint64_t)(hpss ? 4 : 3) * on_cap);
@@ -1189,6 +1224,7 @@ static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumC
     // legacy ACF: next_pow2(2 * (max_frame + 1)), max_frame <= n / 512
     T.lg_fft = next_pow2_u32((uint32_t)(2 * (n / kd.hop + 1)));
     T.lg_work = fa.take((uint64_t)4 * T.lg_fft);
+    T.lg_comb = fa.take(std::max(kd.n_comb, 1u));
     T.lg_tw = nullptr;
     T.lg_pad = 0;
     T.lufs_nb = T.lufs_block = 0;
@@ -1205,10 +1241,10 @@ static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumC
     }
 }
 
-static void plan_escalation(Bump& fa, TrackDev& T) {
-    plan_hop(fa, T.hop[1], std::max(frames_of(T.n, 2048, 256), 1u), 256);
+static void plan_escalation(Bump& fa, TrackDev& T, uint32_t ac_stride) {
+    plan_hop(fa, T.hop[1], std::max(frames_of(T.n, 2048, 256), 1u), 256, ac_stride);
     T.cands[1] = fa.take((uint64_t)MAX_CANDS * 4);
-    plan_hop(fa, T.hop[2], std::max(frames_of(T.n, 2048, 1024), 1u), 1024);
+    plan_hop(fa, T.hop[2], std::max(frames_of(T.n, 2048, 1024), 1u), 1024, ac_stride);
     T.cands[2] = fa.take((uint64_t)MAX_CANDS * 4);
 }
 
@@ -1341,11 +1377,11 @@ static void debug_put_i(const char* name, const int32_t* d, size_t n, cudaStream
     g_debug_arrays[name] = std::move(f);
 }
 
-static uint64_t esc_floats(uint64_t n) {
+static uint64_t esc_floats(uint64_t n, uint32_t ac_stride) {
     TrackDev T{};
     T.n = n;
     Bump b;
-    plan_escalation(b, T);
+    plan_escalation(b, T, ac_stride);
     return align_up(b.pos, 64);
 }
 
@@ -1456,7 +1492,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
             T.n = 0;
             T.sr = T.sr ? T.sr : 1;
         }
-        plan_track(fa, oa, ia, T, cfg);
+        plan_track(fa, oa, ia, T, cfg, dcfg);
         if (T.status == 0 && T.kband_stride != w.kband_stride_common) w.kband_stride_common = kband_seen ? 0u : T.kband_stride;
         if (T.status == 0) kband_seen = true;
         T.hop[0].tgtw = get_tw(c, T.hop[0].fft_cap);
@@ -1465,7 +1501,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
         T.lg_tw = get_tw(c, T.lg_fft);
         if (mr_on) {  // escalation work areas, relative to the start of whichever arena slot escalation_compact_kernel assigns
             Bump b;
-            plan_escalation(b, T);
+            plan_escalation(b, T, dcfg.ac_stride);
             T.hop[1].tgtw = get_tw(c, T.hop[1].fft_cap);
             T.hop[2].tgtw = get_tw(c, T.hop[2].fft_cap);
         }
@@ -1495,7 +1531,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
     const uint64_t fa_base_end = align_up(fa.pos, 64);
     // escalation pool: whatever is left of the budget (at least one track's worth)
     uint64_t esc_each = 0;
-    for (int i = 0; i < nt; ++i) esc_each = std::max<uint64_t>(esc_each, esc_floats(tracks[i].n));
+    for (int i = 0; i < nt; ++i) esc_each = std::max<uint64_t>(esc_each, esc_floats(tracks[i].n, dcfg.ac_stride));
     uint64_t esc_slots = 0;
     if (mr_on) {
         const uint64_t room = fa_budget > fa_base_end ? fa_budget - fa_base_end : 0;
@@ -1713,7 +1749,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
                     const std::string tag = h == 1 ? "h256." : "h1024.";
                     debug_put((tag + "nov.full").c_str(), c.fa + T.hop[h].nov, L, s);
                     debug_put((tag + "tg.fft.full").c_str(), c.fa + T.hop[h].tgfft, T.hop[h].fft_cap / 2 + 1, s);
-                    debug_put((tag + "tg.ac.full").c_str(), c.fa + T.hop[h].tgac, AC_CAP, s);
+                    debug_put((tag + "tg.ac.full").c_str(), c.fa + T.hop[h].tgac, dcfg.n_bpm, s);
                     debug_put((tag + "cands").c_str(), c.fa + T.cands[h], (size_t)MAX_CANDS * 4, s);
                 }
             }
@@ -1807,7 +1843,8 @@ static void debug_dump_wave(DeviceCtx& c, const WaveJob& job) {
     const char* vn[5] = {"base.nov.full", "base.nov.low", "base.nov.mid", "base.nov.high", "base.nov.mel"};
     for (int v = 0; v < 5; ++v) debug_put(vn[v], c.fa + H.nov + (uint64_t)v * fm, L, s);
     debug_put("base.tg.fft.full", c.fa + H.tgfft, H.fft_cap / 2 + 1, s);
-    debug_put("base.tg.ac.full", c.fa + H.tgac, AC_CAP, s);
+    debug_put("base.tg.ac.full", c.fa + H.tgac, dcfg.n_bpm, s);
+    if (T.n_on_final >= 2) debug_put("legacy.comb_raw", c.fa + T.lg_comb, dcfg.n_comb, s);  // hypothesis order; not computed with fewer onsets
     debug_put("base.cands", c.fa + T.cands[bs], (size_t)MAX_CANDS * 4, s);
     float est[12] = {T.est[bs].bpm, T.est[bs].confidence, (float)T.est[bs].agreement, (float)T.est[bs].ok, (float)T.est[bs].n_cands,
                      T.legacy.bpm, T.legacy.confidence, (float)T.legacy.ok, (float)T.escalate, T.est[1].bpm, T.est[2].bpm, 0.0f};
@@ -1826,12 +1863,12 @@ static void debug_dump_wave(DeviceCtx& c, const WaveJob& job) {
 }
 
 // Footprint (floats) of a track's base work areas.
-static uint64_t track_floats(uint64_t n, uint32_t sr, const StratumConfig& cfg) {
+static uint64_t track_floats(uint64_t n, uint32_t sr, const StratumConfig& cfg, const DevCfg& kd) {
     TrackDev T{};
     T.n = n;
     T.sr = sr ? sr : 1;
     Bump fa, oa, ia;
-    plan_track(fa, oa, ia, T, cfg);
+    plan_track(fa, oa, ia, T, cfg, kd);
     return align_up(fa.pos, 64) + 64;
 }
 
@@ -1847,7 +1884,8 @@ struct WaveLimits {
 constexpr uint32_t WAVE_MAX_TRACKS = 65535;
 constexpr uint64_t WAVE_CAP_SAMPLES = (uint64_t)208 * 7938000;  // device-resident wave cap: 208 three-minute tracks (see Session::open)
 
-static void pack_wave(uint32_t& i, uint32_t n_tracks, const uint64_t* lens, const uint32_t* srs, const StratumConfig& cfg, WaveLimits& L, WavePlan& wp) {
+static void pack_wave(uint32_t& i, uint32_t n_tracks, const uint64_t* lens, const uint32_t* srs, const StratumConfig& cfg, const DevCfg& kd, WaveLimits& L,
+                      WavePlan& wp) {
     uint64_t used = 0, esc_max = 0, wave_samples = 0, remaining = 0;
     for (uint32_t q = i; q < n_tracks; ++q) remaining += lens[q];
     uint64_t wave_target = L.wave_max_samples;
@@ -1857,8 +1895,8 @@ static void pack_wave(uint32_t& i, uint32_t n_tracks, const uint64_t* lens, cons
     }
     while (i < n_tracks && wp.idx.size() < std::min(L.wave_max, WAVE_MAX_TRACKS)) {
         if (!wp.idx.empty() && wave_samples + lens[i] / 2 > wave_target) break;
-        const uint64_t need = track_floats(lens[i], srs[i], cfg);
-        const uint64_t esc = esc_floats(lens[i]);
+        const uint64_t need = track_floats(lens[i], srs[i], cfg, kd);
+        const uint64_t esc = esc_floats(lens[i], kd.ac_stride);
         const uint64_t esc_new = std::max(esc_max, esc);
         // keep room for escalating about a quarter of the wave at a time (at least one track)
         const uint64_t esc_room = esc_new * std::max<uint64_t>(1, (wp.idx.size() + 4) / 4);
@@ -1919,6 +1957,13 @@ struct Session {
             wave_max_samples = ~0ull;
         }
         lim = WaveLimits{budget_floats, wave_max, wave_max_samples};
+        if (dcfg.n_bpm > (uint32_t)AC_CAP || dcfg.n_comb > (uint32_t)AC_CAP) {  // fine BPM grid: its kernels read the hypotheses from a table
+            dcfg.bpm_tab = get_bpm_tab(c, dcfg);
+            if (!dcfg.bpm_tab) {
+                set_error("BPM grid table allocation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
+        }
         CUDA_OK(cudaEventCreate(&call_a));
         CUDA_OK(cudaEventCreate(&call_b));
         cudaEventRecord(call_a, c.stream);
@@ -1938,7 +1983,7 @@ struct Session {
             WavePlan wp;
             {
                 HostSpan span_pack("host_wave_pack");
-                pack_wave(i, n, lens, srs, cfg, lim, wp);
+                pack_wave(i, n, lens, srs, cfg, dcfg, lim, wp);
             }
             WaveJob& job = c.jobs[cur];
             WaveJob& prev = c.jobs[cur ^ 1];
@@ -2281,6 +2326,11 @@ void stratum_b200_debug_mel_schedule(const int32_t* mel_off, uint32_t n_mels, in
     mel_fold_schedule(mel_off, n_mels, schedule256);
 }
 
+int32_t stratum_b200_debug_bpm_grid(float min_bpm, float max_bpm, float bpm_resolution, float* out, int32_t cap) {
+    if (!(min_bpm > 0.0f) || !(max_bpm > min_bpm) || !(bpm_resolution > 0.0f)) return -1;
+    return bpm_grid(min_bpm, max_bpm, bpm_resolution, out, out ? cap : 0);
+}
+
 uint32_t stratum_b200_debug_plan_waves(const uint64_t* offsets, const uint32_t* sample_rates, uint32_t n_tracks, const StratumConfig* cfg, double budget_gb,
                                        uint32_t* wave_of_track) {
     StratumConfig def;
@@ -2289,10 +2339,11 @@ uint32_t stratum_b200_debug_plan_waves(const uint64_t* offsets, const uint32_t* 
     std::vector<uint64_t> lens(n_tracks);
     for (uint32_t q = 0; q < n_tracks; ++q) lens[q] = offsets[q + 1] - offsets[q];
     WaveLimits lim{(uint64_t)(budget_gb * 1e9 / 4), WAVE_MAX_TRACKS, WAVE_CAP_SAMPLES};
+    const DevCfg kd = make_devcfg(c);
     uint32_t i = 0, nw = 0;
     while (i < n_tracks) {
         WavePlan wp;
-        pack_wave(i, n_tracks, lens.data(), sample_rates, c, lim, wp);
+        pack_wave(i, n_tracks, lens.data(), sample_rates, c, kd, lim, wp);
         for (uint32_t q : wp.idx) wave_of_track[q] = nw;
         ++nw;
     }

@@ -133,6 +133,55 @@ __device__ __forceinline__ float block_max(float v, float* sm /* >= 32 */) {
     return r;
 }
 
+// top K by (value desc, index asc) of val(i) over i in [lo, hi] (values >= 0); all threads participate; result in out_idx[0..cnt).
+// sval / sidx: one slot per warp.
+template <int K, class F>
+__device__ inline int block_topk(F val, int lo, int hi, int* out_idx, float* sval, int* sidx) {
+    int cnt = 0;
+    for (int r = 0; r < K; ++r) {
+        float bv = -1.0f;
+        int bi = 0x7fffffff;
+        for (int i = lo + (int)threadIdx.x; i <= hi; i += blockDim.x) {
+            bool taken = false;
+            for (int q = 0; q < cnt; ++q) taken |= (out_idx[q] == i);
+            if (taken) continue;
+            float x = val(i);
+            if (x > bv || (x == bv && i < bi)) {
+                bv = x;
+                bi = i;
+            }
+        }
+        for (int o = 16; o > 0; o >>= 1) {
+            float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+            int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+            if (ov > bv || (ov == bv && oi < bi)) {
+                bv = ov;
+                bi = oi;
+            }
+        }
+        if ((threadIdx.x & 31) == 0) {
+            sval[threadIdx.x >> 5] = bv;
+            sidx[threadIdx.x >> 5] = bi;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
+                if (sval[w] > bv || (sval[w] == bv && sidx[w] < bi)) {
+                    bv = sval[w];
+                    bi = sidx[w];
+                }
+            if (bi != 0x7fffffff) out_idx[cnt] = bi;
+            sidx[0] = (bi != 0x7fffffff) ? 1 : 0;
+        }
+        __syncthreads();
+        int ok = sidx[0];
+        __syncthreads();
+        if (!ok) break;
+        ++cnt;
+    }
+    return cnt;
+}
+
 // Exact k-th smallest (0-based) of n non-negative floats: 4-pass MSB radix select on the bit
 // patterns (order-preserving for x >= 0).  All threads of the block call it; result broadcast.
 __device__ inline float block_select_kth(const float* __restrict__ v, uint32_t n, uint32_t k, uint32_t* hist /* 256 */, uint32_t* bcast /* 2 */) {

@@ -1,6 +1,6 @@
 // Legacy BPM estimator — reference period/mod.rs:216-404 (estimate_bpm_with_guardrails):
 //   onset-list autocorrelation via FFT        period/autocorrelation.rs:99-338
-//   comb-filterbank scoring of 201 BPMs       period/comb_filter.rs:96-215, 342-397
+//   comb-filterbank scoring of the BPM grid   period/comb_filter.rs:96-215, 342-397
 //   candidate merge + boosts + guardrails     period/candidate_filter.rs:51-443, period/mod.rs:242-404
 // Always computed (lib.rs:294-329); its estimate is used only when the tempogram produced nothing,
 // but its hard errors propagate to the caller.
@@ -9,7 +9,8 @@
 // next_pow2(2 len); both transforms are the SFFT DAG over ping-pong buffers in global memory.  The
 // comb filterbank is a nearest-neighbour search per (BPM, beat) — not a dense contraction — so one
 // thread walks one BPM hypothesis with a moving cursor over the sorted onsets (first-minimum rule of
-// `min_by_key` on the truncated distance, comb_filter.rs:371-386).
+// `min_by_key` on the truncated distance, comb_filter.rs:371-386).  Grids of more than AC_CAP hypotheses are scored
+// beforehand by comb_kernel across CTAs; legacy_kernel then only selects the head of the confidence order.
 #include "fft.cuh"
 #include "framed.cuh"
 #include "kernels.h"
@@ -18,6 +19,7 @@ namespace sb {
 
 constexpr int LG_MAX_ACF = 160;   // ACF peak candidates kept
 constexpr int LG_MAX_GROUPS = 192;
+constexpr int LG_COMB_TOP = 10;   // comb candidates legacy_merge reads (candidate_filter.rs:228-262 keeps the top 10)
 
 struct LgCand {
     float bpm, conf;
@@ -214,8 +216,52 @@ __device__ inline void legacy_merge(LgCand* ac, int n_ac, const LgCand* comb, in
     }
 }
 
+// score_bpm_candidate (comb_filter.rs:342-397): share of the expected beats k * period that have an onset within tol * period.  The
+// nearest onset is found with a cursor moving over the sorted onsets (first minimum of `min_by_key` on the truncated distance, :371-386).
+__device__ inline float comb_score(const int32_t* on, uint32_t n_on, uint32_t sr, float bpm) {
+    const float tol = clamp_rs(0.1f * (120.0f / bpm), 0.05f, 0.15f);
+    const float period = (60.0f * (float)sr) / bpm;
+    float score = 0.0f;
+    if (period >= 1.0f) {  // `period < 1` is a NumericalError in the reference; unreachable for sr >= 240 / 60
+        const float tol_s = period * tol;
+        const float last = (float)on[n_on - 1];
+        const uint32_t num_beats = as_u32(ceilf(last / period)) + 1;
+        uint32_t aligned = 0, cur = 0;
+        for (uint32_t k = 0; k < num_beats; ++k) {
+            const float eb = (float)k * period;
+            while (cur + 1 < n_on && (float)on[cur + 1] <= eb) ++cur;
+            const uint32_t lo = cur >= 3 ? cur - 3 : 0, hi = min(cur + 4, n_on);
+            uint32_t best_i = lo;
+            uint64_t best_k = ~0ull;
+            for (uint32_t i = lo; i < hi; ++i) {
+                const uint64_t key = as_u64(fabsf((float)on[i] - eb));
+                if (key < best_k) {
+                    best_k = key;
+                    best_i = i;
+                }
+            }
+            const float d = fabsf((float)on[best_i] - eb);
+            if (d <= tol_s) ++aligned;
+        }
+        score = num_beats > 0 ? (float)aligned / (float)num_beats : 0.0f;
+    }
+    return score;
+}
+
+// ---- comb filterbank of a fine BPM grid: one thread per hypothesis, one CTA per (256 hypotheses, track) -------------------------
+// A 60-minute mix at 0.01 BPM is about 20 000 hypotheses x 7 000 beats: spread over CTAs instead of one per track.
+__global__ void __launch_bounds__(256) comb_kernel(const TrackDev* tr, float* fa, const int32_t* __restrict__ ia, DevCfg cfg) {
+    const TrackDev& T = tr[blockIdx.y];
+    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (T.status != 0 || T.n_on_final < 2 || b >= cfg.n_comb) return;
+    fa[T.lg_comb + b] = comb_score(ia + T.on_final, T.n_on_final, T.sr, cfg.bpm_tab[b]);
+}
+
+template <bool FINE>  // FINE: more than AC_CAP hypotheses, scored beforehand by comb_kernel
 __global__ void __launch_bounds__(256) legacy_kernel(TrackDev* tr, float* fa, const int32_t* __restrict__ ia, DevCfg cfg) {
     __shared__ float sred[32];
+    __shared__ float top_val[8];
+    __shared__ int top_w[8], top_idx[LG_COMB_TOP];
     __shared__ LgCand ac[LG_MAX_ACF];
     __shared__ LgCand comb[AC_CAP];
     __shared__ float craw[AC_CAP], cbpm[AC_CAP];
@@ -341,69 +387,68 @@ __global__ void __launch_bounds__(256) legacy_kernel(TrackDev* tr, float* fa, co
         }
     }
     __syncthreads();
-    // ---- comb filterbank: one thread per BPM hypothesis ----
-    int nb = 0;
-    {
-        float b = cfg.min_bpm;
-        while (b <= cfg.max_bpm + 1e-10f && nb < AC_CAP) {
-            ++nb;
-            b = b + cfg.bpm_resolution;
-        }
-    }
-    float my_max = 0.0f;
-    for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) {
-        float bpm = cfg.min_bpm;
-        for (int q = 0; q < bi; ++q) bpm = bpm + cfg.bpm_resolution;
-        const float tol = clamp_rs(0.1f * (120.0f / bpm), 0.05f, 0.15f);
-        const float period = (60.0f * (float)sr) / bpm;
-        float score = 0.0f;
-        if (period >= 1.0f) {  // `period < 1` is a NumericalError in the reference; unreachable for sr >= 240 / 60
-            const float tol_s = period * tol;
-            const float last = (float)on[n_on - 1];
-            const uint32_t num_beats = as_u32(ceilf(last / period)) + 1;
-            uint32_t aligned = 0, cur = 0;
-            for (uint32_t k = 0; k < num_beats; ++k) {
-                const float eb = (float)k * period;
-                while (cur + 1 < n_on && (float)on[cur + 1] <= eb) ++cur;
-                const uint32_t lo = cur >= 3 ? cur - 3 : 0, hi = min(cur + 4, n_on);
-                uint32_t best_i = lo;
-                uint64_t best_k = ~0ull;
-                for (uint32_t i = lo; i < hi; ++i) {
-                    const uint64_t key = as_u64(fabsf((float)on[i] - eb));
-                    if (key < best_k) {
-                        best_k = key;
-                        best_i = i;
-                    }
-                }
-                const float d = fabsf((float)on[best_i] - eb);
-                if (d <= tol_s) ++aligned;
-            }
-            score = num_beats > 0 ? (float)aligned / (float)num_beats : 0.0f;
-        }
-        craw[bi] = score;
-        cbpm[bi] = bpm;
-        my_max = fmaxf(my_max, score);
-    }
-    const float max_score = block_max(my_max, sred);
-    __syncthreads();
-    for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) craw[bi] = max_score > 1e-10f ? craw[bi] / max_score : 0.0f;
-    __syncthreads();
     if (threadIdx.x == 0) s_ncomb = 0;
     __syncthreads();
-    // stable sort by confidence desc (rank counting), entries below 0.1 dropped (they sort last)
-    for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) {
-        const float x = craw[bi];
-        int r = 0;
-        for (int j = 0; j < nb; ++j) r += (craw[j] > x) || (craw[j] == x && j < bi);
-        comb[r] = LgCand{cbpm[bi], x};
-        if (x >= 0.1f) atomicAdd(&s_ncomb, 1);
+    float* raw = fa + T.lg_comb;  // raw scores in hypothesis order
+    if constexpr (!FINE) {
+        // ---- comb filterbank: one thread per BPM hypothesis ----
+        int nb = 0;
+        {
+            float b = cfg.min_bpm;
+            while (b <= cfg.max_bpm + 1e-10f && nb < AC_CAP) {
+                ++nb;
+                b = b + cfg.bpm_resolution;
+            }
+        }
+        float my_max = 0.0f;
+        for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) {
+            float bpm = cfg.min_bpm;
+            for (int q = 0; q < bi; ++q) bpm = bpm + cfg.bpm_resolution;
+            const float score = comb_score(on, n_on, sr, bpm);
+            craw[bi] = score;
+            cbpm[bi] = bpm;
+            raw[bi] = score;
+            my_max = fmaxf(my_max, score);
+        }
+        const float max_score = block_max(my_max, sred);
+        __syncthreads();
+        for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) craw[bi] = max_score > 1e-10f ? craw[bi] / max_score : 0.0f;
+        __syncthreads();
+        // stable sort by confidence desc (rank counting), entries below 0.1 dropped (they sort last)
+        for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) {
+            const float x = craw[bi];
+            int r = 0;
+            for (int j = 0; j < nb; ++j) r += (craw[j] > x) || (craw[j] == x && j < bi);
+            comb[r] = LgCand{cbpm[bi], x};
+            if (x >= 0.1f) atomicAdd(&s_ncomb, 1);
+        }
+    } else {
+        // ---- fine grid: comb_kernel wrote the raw scores.  legacy_merge reads the first 10 entries of the confidence order and the
+        // count of entries >= 0.1, so the order is only needed that far: top 10 by (confidence desc, index asc) = the stable sort's
+        // head.  Selected on the normalised values, as the sort is (the division can tie different raw scores).
+        const int nb = (int)cfg.n_comb;
+        float my_max = 0.0f;
+        for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) my_max = fmaxf(my_max, raw[bi]);
+        const float max_score = block_max(my_max, sred);
+        auto conf = [&](int bi) { return max_score > 1e-10f ? raw[bi] / max_score : 0.0f; };
+        int n_keep = 0;
+        for (int bi = threadIdx.x; bi < nb; bi += blockDim.x) n_keep += conf(bi) >= 0.1f;
+        if (n_keep) atomicAdd(&s_ncomb, n_keep);
+        const int k = block_topk<LG_COMB_TOP>(conf, 0, nb - 1, top_idx, top_val, top_w);
+        if ((int)threadIdx.x < k) comb[threadIdx.x] = LgCand{cfg.bpm_tab[top_idx[threadIdx.x]], conf(top_idx[threadIdx.x])};
     }
     __syncthreads();
     if (threadIdx.x == 0) legacy_merge(ac, s_nac, comb, s_ncomb, est, cfg, &T.legacy);
 }
 
 void launch_legacy_bpm(const WaveCtx& c) {
-    legacy_kernel<<<c.n_tracks, 256, 0, c.stream>>>(c.tracks, c.fa, c.ia, c.cfg);
+    if (fine_bpm_grid(c.cfg)) {
+        comb_kernel<<<dim3((c.cfg.n_comb + 255) / 256, c.n_tracks), 256, 0, c.stream>>>(c.tracks, c.fa, c.ia, c.cfg);
+        count_launch("legacy_bpm");
+        legacy_kernel<true><<<c.n_tracks, 256, 0, c.stream>>>(c.tracks, c.fa, c.ia, c.cfg);
+    } else {
+        legacy_kernel<false><<<c.n_tracks, 256, 0, c.stream>>>(c.tracks, c.fa, c.ia, c.cfg);
+    }
     count_launch("legacy_bpm");
 }
 

@@ -187,6 +187,26 @@ __device__ __forceinline__ int ac_count(const DevCfg& cfg) {
 // keep the loads ahead of the adds.
 constexpr uint32_t TGAC_SMEM_FLOATS = 40 * 1024;  // 160 KB: covers hop-256 curves of 6-minute tracks
 
+// Strength of one lag: sum(nov[i] * nov[i + lag]) / (n - lag), one ordered f32 add chain (tempogram_autocorr.rs:141-150).
+__device__ __forceinline__ float ac_strength(const float* nov, uint32_t n, uint32_t lag) {
+    float sum = 0.0f;
+    uint32_t cnt = 0;
+    if (lag < n) {
+        cnt = n - lag;
+        const float* q = nov + lag;
+        uint32_t i = 0;
+        for (; i + 8 <= cnt; i += 8) {
+            float pr[8];
+#pragma unroll
+            for (int u = 0; u < 8; ++u) pr[u] = __fmul_rn(nov[i + u], q[i + u]);
+#pragma unroll
+            for (int u = 0; u < 8; ++u) sum = __fadd_rn(sum, pr[u]);
+        }
+        for (; i < cnt; ++i) sum = __fadd_rn(sum, __fmul_rn(nov[i], q[i]));
+    }
+    return cnt > 0 ? __fdiv_rn(sum, (float)cnt) : 0.0f;
+}
+
 __global__ void __launch_bounds__(256) tgac_kernel(const TrackDev* tr, const int32_t* __restrict__ list, const SrTables* srtab, const int32_t* sr_index, int h,
                                                    float* fa, DevCfg cfg, uint32_t smem_floats) {
     extern __shared__ float snov[];
@@ -210,23 +230,74 @@ __global__ void __launch_bounds__(256) tgac_kernel(const TrackDev* tr, const int
     for (int b = threadIdx.x; b < nb; b += blockDim.x) {
         const float bpm = ac_bpm(cfg, b);
         const float fpb = __fdiv_rn(frame_rate, __fdiv_rn(bpm, 60.0f));
-        const uint32_t lag = as_u32(fpb);
-        float sum = 0.0f;
-        uint32_t cnt = 0;
-        if (lag < n) {
-            cnt = n - lag;
-            const float* q = nov + lag;
-            uint32_t i = 0;
-            for (; i + 8 <= cnt; i += 8) {
-                float pr[8];
-#pragma unroll
-                for (int u = 0; u < 8; ++u) pr[u] = __fmul_rn(nov[i + u], q[i + u]);
-#pragma unroll
-                for (int u = 0; u < 8; ++u) sum = __fadd_rn(sum, pr[u]);
-            }
-            for (; i < cnt; ++i) sum = __fadd_rn(sum, __fmul_rn(nov[i], q[i]));
+        ac[b] = ac_strength(nov, n, as_u32(fpb));
+    }
+}
+
+// ---- autocorrelation tempogram of a fine BPM grid: one add chain per distinct lag ----------------------------------------
+// A hypothesis enters the strength only through lag = trunc(frame_rate / (bpm / 60)), which does not increase along the grid, so
+// equal lags form contiguous runs: 40..240 BPM at hop 512 and 44.1 kHz has at most 109 of them whatever the resolution.  Pass 1
+// walks the grid 256 hypotheses at a time, compacts the run heads in order (block scan of the head flags) and computes one chain
+// per run, up to 256 runs at a time; run r's strength is stored at ac[r] (r <= the run's first index).  Pass 2 walks the grid
+// from the top down and copies ac[run(b)] to ac[b]: every ac[r] it reads still holds a run strength.  Each strength is the
+// chain tgac_kernel computes for the same lag, so the result is bit-identical to the per-hypothesis form.
+__global__ void __launch_bounds__(256) tgac_lag_kernel(const TrackDev* tr, const int32_t* __restrict__ list, const SrTables* srtab, const int32_t* sr_index,
+                                                       int h, float* fa, DevCfg cfg, uint32_t smem_floats) {
+    extern __shared__ float snov[];
+    __shared__ uint32_t pend[512];  // lags of the runs found and not computed yet (< 256 carried over + <= 256 new)
+    __shared__ uint32_t wsum[33];
+    const int t = list ? list[blockIdx.y] : blockIdx.y;
+    const int v = blockIdx.x;
+    const TrackDev& T = tr[t];
+    if (T.status != 0 || T.F[h] < 2) return;
+    if (!variant_on(srtab[sr_index[t]], v)) return;
+    const uint32_t n = T.F[h] - 1;
+    const HopLayout& HL = T.hop[h];
+    const float* gnov = fa + HL.nov + (uint64_t)v * HL.fmax;
+    const float* nov = gnov;
+    if (n <= smem_floats) {
+        for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) snov[i] = gnov[i];
+        nov = snov;
+    }
+    __syncthreads();
+    float* ac = fa + HL.tgac + (uint64_t)v * cfg.ac_stride;
+    const uint32_t nb = cfg.n_bpm, B = blockDim.x;
+    const float frame_rate = __fdiv_rn((float)T.sr, (float)HL.hop);
+    auto lag_of = [&](uint32_t b) { return as_u32(__fdiv_rn(frame_rate, __fdiv_rn(cfg.bpm_tab[b], 60.0f))); };
+    auto is_head = [&](uint32_t b) { return b < nb && (b == 0 || lag_of(b) != lag_of(b - 1)); };
+    uint32_t n_pend = 0, n_runs = 0;  // block-uniform
+    for (uint32_t c0 = 0; c0 < nb; c0 += B) {
+        const uint32_t b = c0 + threadIdx.x;
+        const bool head = is_head(b);
+        uint32_t tot;
+        const uint32_t pos = block_exclusive_scan(head ? 1u : 0u, &tot, wsum);
+        if (head) pend[n_pend + pos] = lag_of(b);
+        n_pend += tot;
+        __syncthreads();
+        const bool last = c0 + B >= nb;
+        while (n_pend >= B || (last && n_pend > 0)) {
+            const uint32_t m = min(n_pend, B);
+            if (threadIdx.x < m) ac[n_runs + threadIdx.x] = ac_strength(nov, n, pend[threadIdx.x]);
+            const bool carry = threadIdx.x + m < n_pend;  // n_pend - m < B
+            const uint32_t kept = carry ? pend[threadIdx.x + m] : 0u;
+            __syncthreads();
+            if (carry) pend[threadIdx.x] = kept;
+            __syncthreads();
+            n_runs += m;
+            n_pend -= m;
         }
-        ac[b] = cnt > 0 ? __fdiv_rn(sum, (float)cnt) : 0.0f;
+    }
+    uint32_t above = 0;  // run heads at or above the end of the current chunk
+    for (int64_t c0 = (int64_t)((nb - 1) / B) * B; c0 >= 0; c0 -= B) {
+        const uint32_t b = (uint32_t)c0 + threadIdx.x;
+        const bool head = is_head(b);
+        uint32_t tot;
+        const uint32_t before = block_exclusive_scan(head ? 1u : 0u, &tot, wsum);  // heads in [c0, b)
+        const float x = b < nb ? ac[n_runs - above - tot + before + (head ? 1u : 0u) - 1u] : 0.0f;
+        __syncthreads();
+        if (b < nb) ac[b] = x;
+        __syncthreads();
+        above += tot;
     }
 }
 
@@ -257,11 +328,30 @@ __device__ inline float lookup_fft(const FftList& l, float bpm, float tol) {
     }
     return best_v;
 }
+
+// lookup_nearest over the strength-sorted autocorrelation list (tempogram.rs:518-529), ties by strength.  acb[b] = bpm of entry b.
+// Coarse grids: entry b sits within +-3 steps of (bpm - min) / res.  Fine grids: the accumulated values drift from min + b * res (5 steps
+// at 0.01 BPM over 40..240), so the entry is found by value: the lower bound of bpm in the strictly increasing table and its left
+// neighbour are the two nearest entries.
+template <bool FINE>
 __device__ inline float lookup_ac(const float* ac, int nb, const DevCfg& cfg, const float* acb, float bpm, float tol) {
-    float bf = __fdiv_rn(__fsub_rn(bpm, cfg.min_bpm), cfg.bpm_resolution);
-    int bc = (int)bf;
+    int lo, hi;
+    if constexpr (FINE) {
+        int a = 0, e = nb;
+        while (a < e) {
+            const int mid = (a + e) >> 1;
+            if (acb[mid] < bpm) a = mid + 1;
+            else e = mid;
+        }
+        lo = max(a - 1, 0);
+        hi = min(a, nb - 1);
+    } else {
+        float bf = __fdiv_rn(__fsub_rn(bpm, cfg.min_bpm), cfg.bpm_resolution);
+        int bc = (int)bf;
+        lo = max(bc - 3, 0);
+        hi = min(bc + 3, nb - 1);
+    }
     float best_d = INFINITY, best_v = 0.0f;
-    int lo = max(bc - 3, 0), hi = min(bc + 3, nb - 1);
     for (int b = lo; b <= hi; ++b) {
         float d = fabsf(__fsub_rn(acb[b], bpm));
         if (!(d <= tol)) continue;
@@ -274,53 +364,7 @@ __device__ inline float lookup_ac(const float* ac, int nb, const DevCfg& cfg, co
     return best_v;
 }
 
-// top-8 by (value desc, index asc) of v[lo..hi]; all threads participate; result in out_idx[0..cnt)
-__device__ inline int block_top8(const float* v, int lo, int hi, int* out_idx, float* sval, int* sidx) {
-    int cnt = 0;
-    for (int r = 0; r < 8; ++r) {
-        float bv = -1.0f;
-        int bi = 0x7fffffff;
-        for (int i = lo + (int)threadIdx.x; i <= hi; i += blockDim.x) {
-            bool taken = false;
-            for (int q = 0; q < cnt; ++q) taken |= (out_idx[q] == i);
-            if (taken) continue;
-            float x = v[i];
-            if (x > bv || (x == bv && i < bi)) {
-                bv = x;
-                bi = i;
-            }
-        }
-        for (int o = 16; o > 0; o >>= 1) {
-            float ov = __shfl_xor_sync(0xffffffffu, bv, o);
-            int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-            if (ov > bv || (ov == bv && oi < bi)) {
-                bv = ov;
-                bi = oi;
-            }
-        }
-        if ((threadIdx.x & 31) == 0) {
-            sval[threadIdx.x >> 5] = bv;
-            sidx[threadIdx.x >> 5] = bi;
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            for (int w = 1; w < (int)(blockDim.x >> 5); ++w)
-                if (sval[w] > bv || (sval[w] == bv && sidx[w] < bi)) {
-                    bv = sval[w];
-                    bi = sidx[w];
-                }
-            if (bi != 0x7fffffff) out_idx[cnt] = bi;
-            sidx[0] = (bi != 0x7fffffff) ? 1 : 0;
-        }
-        __syncthreads();
-        int ok = sidx[0];
-        __syncthreads();
-        if (!ok) break;
-        ++cnt;
-    }
-    return cnt;
-}
-
+template <bool FINE>  // FINE: more than AC_CAP hypotheses, read from the device table cfg.bpm_tab
 __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t* __restrict__ list, const SrTables* srtab, const int32_t* sr_index, int h,
                                                     float* fa, DevCfg cfg, uint32_t top_n) {
     __shared__ float sval[8];
@@ -335,8 +379,10 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
     const int t = list ? list[blockIdx.x] : blockIdx.x;
     TrackDev& T = tr[t];
     if (threadIdx.x == 0) {
-        float bq = cfg.min_bpm;
-        for (int b = 0; b < AC_CAP; ++b) { acb[b] = bq; bq = __fadd_rn(bq, cfg.bpm_resolution); }
+        if constexpr (!FINE) {
+            float bq = cfg.min_bpm;
+            for (int b = 0; b < AC_CAP; ++b) { acb[b] = bq; bq = __fadd_rn(bq, cfg.bpm_resolution); }
+        }
         T.est[h].ok = 0;
         T.est[h].n_cands = 0;
     }
@@ -361,7 +407,9 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
         kmin = a;
         kmax = b;
     }
-    const int nb = ac_count(cfg);
+    const int nb = FINE ? (int)cfg.n_bpm : ac_count(cfg);
+    const float* bt = FINE ? cfg.bpm_tab : acb;
+    const uint64_t acs = FINE ? cfg.ac_stride : AC_CAP;
     for (int v = 0; v < MAX_VARIANTS; ++v) {
         fl[v].p = fa + HL.tgfft + (uint64_t)v * (HL.fft_cap / 2 + 1);
         fl[v].kmin = kmin;
@@ -374,13 +422,15 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
             if (threadIdx.x == 0) { ntop_fft[v] = 0; ntop_ac[v] = 0; }
             continue;
         }
-        int c1 = (kmin <= kmax) ? block_top8(fl[v].p, (int)kmin, (int)kmax, top_fft[v], sval, sidx) : 0;
-        int c2 = block_top8(fa + HL.tgac + (uint64_t)v * AC_CAP, 0, nb - 1, top_ac[v], sval, sidx);
+        const float* pf = fl[v].p;
+        const float* pa = fa + HL.tgac + (uint64_t)v * acs;
+        int c1 = (kmin <= kmax) ? block_topk<8>([&](int i) { return pf[i]; }, (int)kmin, (int)kmax, top_fft[v], sval, sidx) : 0;
+        int c2 = block_topk<8>([&](int i) { return pa[i]; }, 0, nb - 1, top_ac[v], sval, sidx);
         if (threadIdx.x == 0) { ntop_fft[v] = c1; ntop_ac[v] = c2; }
     }
     __syncthreads();
     const float fft_primary = ntop_fft[0] > 0 ? fft_bpm(fl[0], (uint32_t)top_fft[0][0]) : 0.0f;
-    const float ac_primary = ntop_ac[0] > 0 ? acb[top_ac[0][0]] : 0.0f;
+    const float ac_primary = ntop_ac[0] > 0 ? bt[top_ac[0][0]] : 0.0f;
     if (threadIdx.x == 0) {
         const float FACT[7] = {1.0f, 0.5f, 2.0f, 1.0f / 3.0f, 3.0f, 2.0f / 3.0f, 3.0f / 2.0f};
         int c = 0;
@@ -393,7 +443,7 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
         for (int v = 0; v < MAX_VARIANTS; ++v) {
             if (!variant_on(st, v)) continue;
             for (int i = 0; i < ntop_fft[v]; ++i) push(fft_bpm(fl[v], (uint32_t)top_fft[v][i]));
-            for (int i = 0; i < ntop_ac[v]; ++i) push(acb[top_ac[v][i]]);
+            for (int i = 0; i < ntop_ac[v]; ++i) push(bt[top_ac[v][i]]);
         }
         if (fft_primary > 0.0f) push(fft_primary);
         if (ac_primary > 0.0f) push(ac_primary);
@@ -431,7 +481,7 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
     for (int v = 0; v < n_score; ++v) {
         vmax_fft[v] = vmax_ac[v] = 1.0f;
         if (!variant_on(st, v)) continue;
-        const float* acv = fa + HL.tgac + (uint64_t)v * AC_CAP;
+        const float* acv = fa + HL.tgac + (uint64_t)v * acs;
         vmax_fft[v] = fmaxf(ntop_fft[v] > 0 ? fl[v].p[top_fft[v][0]] : 1.0f, 1e-12f);
         vmax_ac[v] = fmaxf(ntop_ac[v] > 0 ? acv[top_ac[v][0]] : 1.0f, 1e-12f);
         w_sum = __fadd_rn(w_sum, fmaxf(vw[v], 0.0f));
@@ -442,9 +492,9 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
         float fft_acc = 0.0f, ac_acc = 0.0f;
         for (int v = 0; v < n_score; ++v) {
             if (!variant_on(st, v) || !(vw[v] > 0.0f)) continue;
-            const float* acv = fa + HL.tgac + (uint64_t)v * AC_CAP;
+            const float* acv = fa + HL.tgac + (uint64_t)v * acs;
             float fv = lookup_fft(fl[v], bpm, 0.75f);
-            float av = lookup_ac(acv, nb, cfg, acb, bpm, ac_tol);
+            float av = lookup_ac<FINE>(acv, nb, cfg, bt, bpm, ac_tol);
             fft_acc = __fadd_rn(fft_acc, __fmul_rn(vw[v], clamp_rs(__fdiv_rn(fv, vmax_fft[v]), 0.0f, 1.0f)));
             ac_acc = __fadd_rn(ac_acc, __fmul_rn(vw[v], clamp_rs(__fdiv_rn(av, vmax_ac[v]), 0.0f, 1.0f)));
         }
@@ -455,11 +505,11 @@ __global__ void __launch_bounds__(256) score_kernel(TrackDev* tr, const int32_t*
             uint32_t support = 0;
             for (int v = 1; v < MAX_VARIANTS; ++v) {
                 if (!variant_on(st, v)) continue;
-                const float* acv = fa + HL.tgac + (uint64_t)v * AC_CAP;
+                const float* acv = fa + HL.tgac + (uint64_t)v * acs;
                 const float mf = fmaxf(ntop_fft[v] > 0 ? fl[v].p[top_fft[v][0]] : 1.0f, 1e-12f);
                 const float ma = fmaxf(ntop_ac[v] > 0 ? acv[top_ac[v][0]] : 1.0f, 1e-12f);
                 float sf = clamp_rs(__fdiv_rn(lookup_fft(fl[v], bpm, 0.75f), mf), 0.0f, 1.0f);
-                float sa = clamp_rs(__fdiv_rn(lookup_ac(acv, nb, cfg, acb, bpm, ac_tol), ma), 0.0f, 1.0f);
+                float sa = clamp_rs(__fdiv_rn(lookup_ac<FINE>(acv, nb, cfg, bt, bpm, ac_tol), ma), 0.0f, 1.0f);
                 if (fmaxf(sf, sa) >= support_thr) ++support;
             }
             if (support >= 2) score = __fmul_rn(score, __fadd_rn(1.0f, __fmul_rn(bonus, __fsub_rn((float)support, 1.0f))));
@@ -1001,21 +1051,24 @@ void launch_tempogram(const WaveCtx& c, int h, const int32_t* d_list, int n_list
     count_launch("tempogram");
     tgfft_kernel<<<g5, 512, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa);
     count_launch("tempogram");
+    const bool fine = fine_bpm_grid(c.cfg);
     {
-        static bool attr_dev[64] = {};  // function attributes are per device
+        static bool attr_dev[2][64] = {};  // function attributes are per device
         int dev = 0;
         cudaGetDevice(&dev);
-        if (!attr_dev[dev & 63]) {
-            cudaFuncSetAttribute(tgac_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TGAC_SMEM_FLOATS * sizeof(float));
-            attr_dev[dev & 63] = true;
+        if (!attr_dev[fine][dev & 63]) {
+            cudaFuncSetAttribute(fine ? tgac_lag_kernel : tgac_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TGAC_SMEM_FLOATS * sizeof(float));
+            attr_dev[fine][dev & 63] = true;
         }
         const uint32_t want = c.max_F[h];  // novelty length upper bound of the wave
         const uint32_t smem_floats = want <= TGAC_SMEM_FLOATS ? want : 0;  // curves that do not fit stay in global memory
-        tgac_kernel<<<g5, 256, smem_floats * sizeof(float), c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, smem_floats);
+        if (fine) tgac_lag_kernel<<<g5, 256, smem_floats * sizeof(float), c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, smem_floats);
+        else tgac_kernel<<<g5, 256, smem_floats * sizeof(float), c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, smem_floats);
     }
     count_launch("tempogram");
     const uint32_t top_n = (h == c.cfg.bs || h == SLOT_PERC) ? c.cfg.base_top_n : c.cfg.mr_aux_k;
-    score_kernel<<<n_list, 256, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, top_n);
+    if (fine) score_kernel<true><<<n_list, 256, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, top_n);
+    else score_kernel<false><<<n_list, 256, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg, top_n);
     count_launch("tempogram");
 }
 

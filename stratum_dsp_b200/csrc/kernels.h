@@ -7,6 +7,11 @@ namespace sb {
 // Values of StratumConfig that kernels read (copied by value into launches).
 struct DevCfg {
     float min_bpm, max_bpm, bpm_resolution;
+    // BPM hypothesis grid, built on the host with the reference's f32 accumulation (engine.cu: bpm_grid)
+    uint32_t n_bpm;               // autocorrelation tempogram: `bpm <= max_bpm` (tempogram_autocorr.rs:79-178)
+    uint32_t n_comb;              // comb filterbank: `bpm <= max_bpm + 1e-10` (comb_filter.rs:96-215)
+    uint32_t ac_stride;           // floats per variant of HopLayout::tgac: max(AC_CAP, n_bpm)
+    const float* bpm_tab;         // max(n_bpm, n_comb) hypothesis BPMs on the device; set only on the fine-grid path (either count > AC_CAP)
     float silence_thr_linear;     // 10^(min_amplitude_db/20), silence.rs:141
     uint32_t silence_min_ms;      // 500, lib.rs:134
     float energy_thr_mul;         // 10^(-20/20), energy_flux.rs:160
@@ -71,6 +76,9 @@ struct DevCfg {
     uint32_t khpss_step, khpss_tm, khpss_fm;
     float khpss_power;
 };
+
+// Grids of more than AC_CAP hypotheses take the fine-grid kernels (distinct-lag tempogram, table lookups, comb filterbank across CTAs).
+__host__ __device__ inline bool fine_bpm_grid(const DevCfg& d) { return d.bpm_tab != nullptr; }
 
 // Per-sample-rate tables (band edges, mel filterbank) — novelty.rs:72-190, tempogram.rs:364-372.
 struct SrTables {
