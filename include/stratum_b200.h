@@ -262,7 +262,7 @@ size_t stratum_b200_sizeof(int32_t which);
 /* ---- stage-level entry points (kernel parity tests and bench instrumentation) ------------------ */
 
 /* compute_stft (src/features/chroma/extractor.rs:301-359) on the device: `samples` host pointer,
- * out = frames x (frame_size/2+1) magnitudes on the host.  frame_size in {2048, 8192}. */
+ * out = frames x (frame_size/2+1) magnitudes on the host.  frame_size: a power of two from 64 to 16 384. */
 int64_t stratum_b200_stft(const float* samples, uint64_t n, uint32_t frame_size, uint32_t hop, float gain, float* out, uint64_t out_cap);
 
 /* Device-side synthetic generator (tests/synth.py, SURVEY §8d): fills d_out (device) with n_tracks

@@ -1,8 +1,8 @@
 // Host engine + C ABI (include/stratum_b200.h) of the B200 analysis path.
 //
 // Execution model: a batch is cut into WAVES of tracks whose work areas fit the device arena
-// (spectrograms are the bulk: 64 MB for the 2048/512 STFT and 254 MB for the 8192/512 key STFT of a
-// 3-minute track).  Every stage of the reference's analyze_audio (lib.rs:86-1635) is one or a few
+// (spectrograms are the bulk: 64 MB for the 2048/512 STFT — 254 MB at frame_size 8192 — and 254 MB for the 8192/512 key STFT
+// of a 3-minute track).  Every stage of the reference's analyze_audio (lib.rs:86-1635) is one or a few
 // kernels launched over the whole wave; per-track state lives in a TrackDev record on the device.
 // The only host round trip inside a wave is the escalation decision (lib.rs:412-459): the records
 // are read back, the tracks that need the multi-resolution pass are given arena slots for their
@@ -569,8 +569,8 @@ static int sr_slot(DeviceCtx& c, uint32_t sr, const StratumConfig& cfg, int* slo
     st.sr = sr;
     const uint32_t key_frame = cfg.enable_key_stft_override ? std::max<uint32_t>(cfg.key_stft_frame_size, 256) : cfg.frame_size;  // lib.rs:984-989
     const uint32_t key_bins = key_frame / 2 + 1;
-    const uint32_t n_bins = 1025;
-    const float freq_res = (float)sr / 2048.0f;
+    const uint32_t n_bins = cfg.frame_size / 2 + 1;  // tempo-path STFT bins (the novelty curves' spectrogram)
+    const float freq_res = (float)sr / (float)cfg.frame_size;
     uint32_t vm = 1u;  // full
     // band edges — period/tempogram.rs:356-372
     const uint32_t b0 = 1;
@@ -611,7 +611,7 @@ static int sr_slot(DeviceCtx& c, uint32_t sr, const StratumConfig& cfg, int* slo
             if (fmax < lo) fmax = lo;
             if (fmax > nyq) fmax = nyq;
         }
-        const float res = (float)sr / 2048.0f;
+        const float res = (float)sr / (float)cfg.frame_size;
         const float mmin = mel_of(fmin), mmax = mel_of(fmax);
         const float step = (mmax - mmin) / (float)(n_mels + 1);
         std::vector<uint32_t> pts(n_mels + 2);
@@ -944,7 +944,7 @@ static int config_validate(const StratumConfig& c) {
     }
     if ((c.enable_hpss_onsets || c.enable_tempogram_percussive_fallback) && c.hpss_margin > 10) return ni("hpss_margin > 10");
     if (c.emit_tempogram_candidates && c.tempogram_candidates_top_n > 200) return ni("tempogram_candidates_top_n > 200");
-    if (c.frame_size != 2048) return ni("frame_size other than 2048");
+    if (!tempo_frame_supported(c.frame_size)) return ni("frame_size other than 2048, 4096 or 8192");
     if (c.hop_size == 0) {
         set_error("Hop size must be > 0");
         return STRATUM_INVALID_INPUT;
@@ -1070,6 +1070,8 @@ static DevCfg make_devcfg(const StratumConfig& c) {
     d.hpcp_pow = c.key_hpcp_mag_power;
     d.hpcp_sigma = c.soft_mapping_sigma;
     d.hop = c.hop_size;
+    d.frame = c.frame_size;
+    d.bins = c.frame_size / 2 + 1;
     d.bs = c.hop_size == 512 ? 0 : SLOT_BASE_ALT;  // the base path shares slot 0 with the multi-resolution pass only at hop 512
     d.key_frame = c.enable_key_stft_override ? std::max<uint32_t>(c.key_stft_frame_size, 256) : c.frame_size;  // lib.rs:984-995
     d.key_hop = c.enable_key_stft_override ? std::max<uint32_t>(c.key_stft_hop_size, 1) : c.hop_size;
@@ -1114,8 +1116,6 @@ static DevCfg make_devcfg(const StratumConfig& c) {
 }
 
 // ---- arena planning -----------------------------------------------------------------------------------------
-static inline uint32_t frames_of(uint64_t n, uint32_t frame, uint32_t hop) { return n >= frame ? (uint32_t)((n - frame) / hop + 1) : 0; }
-
 struct Bump {
     uint64_t pos = 0;
     uint64_t take(uint64_t n, uint64_t al = 32) {
@@ -1126,16 +1126,16 @@ struct Bump {
     }
 };
 
-static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, uint32_t ac_stride, bool with_spec = true) {
+static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, const DevCfg& kd, bool with_spec = true) {
     H.fmax = fcap;
     H.hop = hop;
     H.fft_cap = std::max<uint32_t>(next_pow2_u32(fcap > 1 ? fcap - 1 : 1), 4);
-    H.spec = with_spec ? fa.take((uint64_t)fcap * 1025) : 0;
+    H.spec = with_spec ? fa.take((uint64_t)fcap * kd.bins) : 0;
     H.frame = fa.take((uint64_t)FRAME_Q * fcap);
     H.pair = fa.take((uint64_t)PAIR_Q * fcap);
     H.nov = fa.take((uint64_t)MAX_VARIANTS * fcap);
     H.tgfft = fa.take((uint64_t)MAX_VARIANTS * (H.fft_cap / 2 + 1));
-    H.tgac = fa.take((uint64_t)MAX_VARIANTS * ac_stride);
+    H.tgac = fa.take((uint64_t)MAX_VARIANTS * kd.ac_stride);
     H.tgwork = fa.take((uint64_t)MAX_VARIANTS * 2 * H.fft_cap);
     H.tgtw = nullptr;
     H.pad_ = 0;
@@ -1144,16 +1144,16 @@ static void plan_hop(Bump& fa, HopLayout& H, uint32_t fcap, uint32_t hop, uint32
 // Base (always needed) work areas of one track.
 static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumConfig& cfg, const DevCfg& kd) {
     const uint64_t n = T.n;
-    const uint32_t F512 = frames_of(n, 2048, 512), F256 = frames_of(n, 2048, 256), F1024 = frames_of(n, 2048, 1024);
+    const uint32_t F512 = frames_of(n, kd.frame, 512), F256 = frames_of(n, kd.frame, 256), F1024 = frames_of(n, kd.frame, 1024);
     const uint32_t Fk = frames_of(n, kd.key_frame, kd.key_hop);
-    const uint32_t Fsil = n >= 2048 ? frames_of(n, 2048, 1024) : 1;
-    const uint32_t Fb = frames_of(n, 2048, kd.hop);  // frames of the base path (= F512 at the default hop_size)
+    const uint32_t Fsil = n >= kd.frame ? frames_of(n, kd.frame, kd.frame / 2) : 1;
+    const uint32_t Fb = frames_of(n, kd.frame, kd.hop);  // frames of the base path (= F512 at the default hop_size)
     T.fall = std::max(std::max(std::max(F256, F512), std::max(F1024, 1u)), Fb);
     T.fkmax = Fk;
-    plan_hop(fa, T.hop[0], std::max(F512, 1u), 512, kd.ac_stride);
+    plan_hop(fa, T.hop[0], std::max(F512, 1u), 512, kd);
     T.cands[0] = fa.take((uint64_t)MAX_CANDS * 4);
     if (kd.bs != 0) {  // hop_size other than 512: the base path gets a slot of its own
-        plan_hop(fa, T.hop[SLOT_BASE_ALT], std::max(Fb, 1u), kd.hop, kd.ac_stride);
+        plan_hop(fa, T.hop[SLOT_BASE_ALT], std::max(Fb, 1u), kd.hop, kd);
         T.cands[SLOT_BASE_ALT] = fa.take((uint64_t)MAX_CANDS * 4);
     }
     T.sil_rms = fa.take(Fsil + 1);
@@ -1197,13 +1197,13 @@ static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumC
     T.on_merged = 0;
     T.on_hpss = 0;
     const bool hpss = cfg.enable_hpss_onsets || cfg.enable_tempogram_percussive_fallback;
-    if (hpss) {  // HPSS work areas (onset/hpss.rs): two ping-pong pairs of F x 1025 and the feature slot of the percussive part
+    if (hpss) {  // HPSS work areas (onset/hpss.rs): two ping-pong pairs of F x bins and the feature slot of the percussive part
         T.on_hpss = ia.take(on_cap);
         for (int q = 0; q < 2; ++q) {
-            T.hpss_h[q] = fa.take((uint64_t)std::max(Fb, 1u) * 1025);
-            T.hpss_p[q] = fa.take((uint64_t)std::max(Fb, 1u) * 1025);
+            T.hpss_h[q] = fa.take((uint64_t)std::max(Fb, 1u) * kd.bins);
+            T.hpss_p[q] = fa.take((uint64_t)std::max(Fb, 1u) * kd.bins);
         }
-        plan_hop(fa, T.hop[SLOT_PERC], std::max(Fb, 1u), kd.hop, kd.ac_stride, false);
+        plan_hop(fa, T.hop[SLOT_PERC], std::max(Fb, 1u), kd.hop, kd, false);
         T.cands[SLOT_PERC] = fa.take((uint64_t)MAX_CANDS * 4);
     }
     T.on_final = ia.take((uint64_t)(hpss ? 4 : 3) * on_cap);
@@ -1241,10 +1241,10 @@ static void plan_track(Bump& fa, Bump& oa, Bump& ia, TrackDev& T, const StratumC
     }
 }
 
-static void plan_escalation(Bump& fa, TrackDev& T, uint32_t ac_stride) {
-    plan_hop(fa, T.hop[1], std::max(frames_of(T.n, 2048, 256), 1u), 256, ac_stride);
+static void plan_escalation(Bump& fa, TrackDev& T, const DevCfg& kd) {
+    plan_hop(fa, T.hop[1], std::max(frames_of(T.n, kd.frame, 256), 1u), 256, kd);
     T.cands[1] = fa.take((uint64_t)MAX_CANDS * 4);
-    plan_hop(fa, T.hop[2], std::max(frames_of(T.n, 2048, 1024), 1u), 1024, ac_stride);
+    plan_hop(fa, T.hop[2], std::max(frames_of(T.n, kd.frame, 1024), 1u), 1024, kd);
     T.cands[2] = fa.take((uint64_t)MAX_CANDS * 4);
 }
 
@@ -1377,11 +1377,11 @@ static void debug_put_i(const char* name, const int32_t* d, size_t n, cudaStream
     g_debug_arrays[name] = std::move(f);
 }
 
-static uint64_t esc_floats(uint64_t n, uint32_t ac_stride) {
+static uint64_t esc_floats(uint64_t n, const DevCfg& kd) {
     TrackDev T{};
     T.n = n;
     Bump b;
-    plan_escalation(b, T, ac_stride);
+    plan_escalation(b, T, kd);
     return align_up(b.pos, 64);
 }
 
@@ -1460,6 +1460,13 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
             return STRATUM_PROCESSING_ERROR;
         }
     }
+    if (dcfg.frame == 4096) {  // the tempo-path STFT takes the generic kernel at this size (k_stft.cu: launch_stft_hop)
+        w.gen_tempo = get_gen_stft(c, dcfg.frame);
+        if (w.gen_tempo.n == 0) {
+            set_error("table allocation failed");
+            return STRATUM_PROCESSING_ERROR;
+        }
+    }
     bool kband_seen = false;
     const bool mr_on = dcfg.mr_enabled && !dcfg.force_legacy;
     for (int i = 0; i < nt; ++i) {
@@ -1501,7 +1508,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
         T.lg_tw = get_tw(c, T.lg_fft);
         if (mr_on) {  // escalation work areas, relative to the start of whichever arena slot escalation_compact_kernel assigns
             Bump b;
-            plan_escalation(b, T, dcfg.ac_stride);
+            plan_escalation(b, T, dcfg);
             T.hop[1].tgtw = get_tw(c, T.hop[1].fft_cap);
             T.hop[2].tgtw = get_tw(c, T.hop[2].fft_cap);
         }
@@ -1509,16 +1516,16 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
             set_error("twiddle table allocation failed");
             return STRATUM_PROCESSING_ERROR;
         }
-        const uint32_t Fsil = T.n >= 2048 ? frames_of(T.n, 2048, 1024) : (T.n > 0 ? 1 : 0);
+        const uint32_t Fsil = T.n >= dcfg.frame ? frames_of(T.n, dcfg.frame, dcfg.frame / 2) : (T.n > 0 ? 1 : 0);
         T.Fsil = Fsil;
         // provisional (untrimmed) frame counts; trim_kernel rewrites them
         T.m = T.n;
         T.trim_start = 0;
         T.trim_end = T.n;
-        w.max_F[0] = std::max(w.max_F[0], frames_of(T.n, 2048, 512));
-        w.max_F[1] = std::max(w.max_F[1], frames_of(T.n, 2048, 256));
-        w.max_F[2] = std::max(w.max_F[2], frames_of(T.n, 2048, 1024));
-        w.max_F[SLOT_BASE_ALT] = std::max(w.max_F[SLOT_BASE_ALT], frames_of(T.n, 2048, dcfg.hop));
+        w.max_F[0] = std::max(w.max_F[0], frames_of(T.n, dcfg.frame, 512));
+        w.max_F[1] = std::max(w.max_F[1], frames_of(T.n, dcfg.frame, 256));
+        w.max_F[2] = std::max(w.max_F[2], frames_of(T.n, dcfg.frame, 1024));
+        w.max_F[SLOT_BASE_ALT] = std::max(w.max_F[SLOT_BASE_ALT], frames_of(T.n, dcfg.frame, dcfg.hop));
         w.max_F[SLOT_PERC] = w.max_F[dcfg.bs];
         w.max_Fk = std::max(w.max_Fk, frames_of(T.n, dcfg.key_frame, dcfg.key_hop));
         w.max_Fsil = std::max(w.max_Fsil, Fsil);
@@ -1531,7 +1538,7 @@ static int wave_begin(DeviceCtx& c, const float* d_samples, const uint64_t* samp
     const uint64_t fa_base_end = align_up(fa.pos, 64);
     // escalation pool: whatever is left of the budget (at least one track's worth)
     uint64_t esc_each = 0;
-    for (int i = 0; i < nt; ++i) esc_each = std::max<uint64_t>(esc_each, esc_floats(tracks[i].n, dcfg.ac_stride));
+    for (int i = 0; i < nt; ++i) esc_each = std::max<uint64_t>(esc_each, esc_floats(tracks[i].n, dcfg));
     uint64_t esc_slots = 0;
     if (mr_on) {
         const uint64_t room = fa_budget > fa_base_end ? fa_budget - fa_base_end : 0;
@@ -1824,7 +1831,7 @@ static void debug_dump_wave(DeviceCtx& c, const WaveJob& job) {
     const uint32_t F = T.F[bs], L = F > 0 ? F - 1 : 0;
     const uint64_t fm = H.fmax;
     debug_put("gain", &c.d_tracks[0].gain, 1, s);
-    debug_put("spec512_head", c.fa + H.spec, (size_t)std::min<uint32_t>(F, 64) * 1025, s);
+    debug_put("spec512_head", c.fa + H.spec, (size_t)std::min<uint32_t>(F, 64) * dcfg.bins, s);
     debug_put("onset.spectral_flux", c.fa + H.pair + 0 * fm, L, s);
     debug_put("frame.hfc", c.fa + H.frame + 2 * fm, F, s);
     debug_put("frame.energy", c.fa + H.frame + 1 * fm, F, s);
@@ -1835,7 +1842,7 @@ static void debug_dump_wave(DeviceCtx& c, const WaveJob& job) {
     debug_put_i("onset.hfc", c.ia + T.on_hfc, T.n_on_hfc, s);
     if (dcfg.hpss_onsets) debug_put_i("onset.hpss", c.ia + T.on_hpss, T.n_on_hpss, s);
     if (T.hpss_ready) {
-        debug_put("hpss.perc_head", c.fa + T.hop[SLOT_PERC].spec, (size_t)std::min<uint32_t>(F, 64) * 1025, s);
+        debug_put("hpss.perc_head", c.fa + T.hop[SLOT_PERC].spec, (size_t)std::min<uint32_t>(F, 64) * dcfg.bins, s);
         float pe[4] = {T.est[SLOT_PERC].bpm, T.est[SLOT_PERC].confidence, (float)T.est[SLOT_PERC].agreement, (float)T.est[SLOT_PERC].ok};
         std::lock_guard<std::mutex> lk(g_debug_mu);
         g_debug_arrays["perc.est"] = std::vector<float>(pe, pe + 4);
@@ -1896,7 +1903,7 @@ static void pack_wave(uint32_t& i, uint32_t n_tracks, const uint64_t* lens, cons
     while (i < n_tracks && wp.idx.size() < std::min(L.wave_max, WAVE_MAX_TRACKS)) {
         if (!wp.idx.empty() && wave_samples + lens[i] / 2 > wave_target) break;
         const uint64_t need = track_floats(lens[i], srs[i], cfg, kd);
-        const uint64_t esc = esc_floats(lens[i], kd.ac_stride);
+        const uint64_t esc = esc_floats(lens[i], kd);
         const uint64_t esc_new = std::max(esc_max, esc);
         // keep room for escalating about a quarter of the wave at a time (at least one track)
         const uint64_t esc_room = esc_new * std::max<uint64_t>(1, (wp.idx.size() + 4) / 4);

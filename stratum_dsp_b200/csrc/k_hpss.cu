@@ -19,7 +19,6 @@ namespace sb {
 constexpr int HP_T = 32;       // tile: frames
 constexpr int HP_B = 32;       // tile: bins
 constexpr int HP_MAXM = 10;    // margin upper bound (21-wire network); larger margins are rejected by the ABI
-constexpr int HP_BINS = 1025;
 
 __device__ __forceinline__ float median21(float (&v)[21], int n) {
 #define CE(i, j)                    \
@@ -49,7 +48,8 @@ __device__ __forceinline__ bool hpss_converged_before(const TrackDev& T, int it)
     return false;
 }
 
-__global__ void __launch_bounds__(256) hpss_iter_kernel(TrackDev* tr, const int32_t* __restrict__ list, float* fa, int it, uint32_t margin, int bs) {
+// nb: bins per spectrogram row (frame_size / 2 + 1)
+__global__ void __launch_bounds__(256) hpss_iter_kernel(TrackDev* tr, const int32_t* __restrict__ list, float* fa, int it, uint32_t margin, int bs, int nb) {
     __shared__ float Ht[HP_T + 2 * HP_MAXM][HP_B + 1];
     __shared__ float Pt[HP_T][HP_B + 2 * HP_MAXM + 1];
     __shared__ float sred[8];
@@ -70,19 +70,19 @@ __global__ void __launch_bounds__(256) hpss_iter_kernel(TrackDev* tr, const int3
     for (int i = threadIdx.x; i < (HP_T + 2 * HP_MAXM) * HP_B; i += blockDim.x) {
         const int r = i / HP_B, c = i % HP_B;
         const int f = f0 - HP_MAXM + r, b = b0 + c;
-        Ht[r][c] = (f >= 0 && f < F && b < HP_BINS) ? Hs[(uint64_t)f * HP_BINS + b] : INF;
+        Ht[r][c] = (f >= 0 && f < F && b < nb) ? Hs[(uint64_t)f * nb + b] : INF;
     }
     for (int i = threadIdx.x; i < HP_T * (HP_B + 2 * HP_MAXM); i += blockDim.x) {
         const int r = i / (HP_B + 2 * HP_MAXM), c = i % (HP_B + 2 * HP_MAXM);
         const int f = f0 + r, b = b0 - HP_MAXM + c;
-        Pt[r][c] = (f < F && b >= 0 && b < HP_BINS) ? Ps[(uint64_t)f * HP_BINS + b] : INF;
+        Pt[r][c] = (f < F && b >= 0 && b < nb) ? Ps[(uint64_t)f * nb + b] : INF;
     }
     __syncthreads();
     float mx = 0.0f;
     for (int e = threadIdx.x; e < HP_T * HP_B; e += blockDim.x) {
         const int r = e / HP_B, c = e % HP_B;
         const int f = f0 + r, b = b0 + c;
-        if (f >= F || b >= HP_BINS) continue;
+        if (f >= F || b >= nb) continue;
         float v[21];
         // time window [f-m, f+m] clipped to [0, F)
         int n = 0;
@@ -98,12 +98,12 @@ __global__ void __launch_bounds__(256) hpss_iter_kernel(TrackDev* tr, const int3
 #pragma unroll
         for (int j = 0; j < 21; ++j) {
             const int d = j - HP_MAXM;
-            const bool in = d >= -m && d <= m && b + d >= 0 && b + d < HP_BINS;
+            const bool in = d >= -m && d <= m && b + d >= 0 && b + d < nb;
             v[j] = in ? Pt[r][c + HP_MAXM + d] : INF;
             n += in;
         }
         const float pf = median21(v, n);
-        const float original = S[(uint64_t)f * HP_BINS + b];
+        const float original = S[(uint64_t)f * nb + b];
         const float total = hf + pf;
         float hn, pn;
         if (total > 1e-10f) {
@@ -113,8 +113,8 @@ __global__ void __launch_bounds__(256) hpss_iter_kernel(TrackDev* tr, const int3
             hn = original * 0.5f;
             pn = original * 0.5f;
         }
-        Hd[(uint64_t)f * HP_BINS + b] = hn;
-        Pd[(uint64_t)f * HP_BINS + b] = pn;
+        Hd[(uint64_t)f * nb + b] = hn;
+        Pd[(uint64_t)f * nb + b] = pn;
         mx = fmaxf(mx, fmaxf(fabsf(hn - Ht[r + HP_MAXM][c]), fabsf(pn - Pt[r][c + HP_MAXM])));
     }
     for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
@@ -144,9 +144,9 @@ __global__ void hpss_finish_kernel(TrackDev* tr, const int32_t* __restrict__ lis
 
 void launch_hpss(const WaveCtx& c, const int32_t* d_list, int n_list) {
     if (n_list == 0 || c.max_F[c.cfg.bs] == 0) return;
-    const dim3 grid((HP_BINS + HP_B - 1) / HP_B, (c.max_F[c.cfg.bs] + HP_T - 1) / HP_T, n_list);
+    const dim3 grid((c.cfg.bins + HP_B - 1) / HP_B, (c.max_F[c.cfg.bs] + HP_T - 1) / HP_T, n_list);
     for (int it = 0; it < 10; ++it) {  // DEFAULT_ITERATIONS, hpss.rs:20
-        hpss_iter_kernel<<<grid, 256, 0, c.stream>>>(c.tracks, d_list, c.fa, it, c.cfg.hpss_margin, c.cfg.bs);
+        hpss_iter_kernel<<<grid, 256, 0, c.stream>>>(c.tracks, d_list, c.fa, it, c.cfg.hpss_margin, c.cfg.bs, (int)c.cfg.bins);
         count_launch("hpss");
     }
     hpss_finish_kernel<<<(n_list + 127) / 128, 128, 0, c.stream>>>(c.tracks, d_list, n_list, 10);

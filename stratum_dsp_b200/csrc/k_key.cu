@@ -1027,7 +1027,7 @@ __global__ void key_vote_kernel(TrackDev* tr, const float* fa, int n_tracks, Dev
         T.key_clarity = 0.0f;
         T.key_fallback = 0;
     }
-    if (T.status != 0 || T.kf == 0 || T.m < 2048) return;
+    if (T.status != 0 || T.kf == 0 || T.m < cfg.frame) return;  // so_key.cpp:790: shorter than frame_size
     uint32_t f0, nf;
     key_slice(T.kf, cfg, &f0, &nf);
     if (nf == 0) return;

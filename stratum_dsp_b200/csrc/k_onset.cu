@@ -22,22 +22,28 @@ constexpr int MEL_MAX = 40;
 // ---- energy flux onsets ------------------------------------------------------------------------
 constexpr int ERMS_SEG = 32;  // hop-blocks per segment of the streamed frame-RMS (framed.cuh)
 // hop_size other than 512: the tile form (one lane per frame, any hop), same per-frame sums in the same order
+template <int FRAME>
 __global__ void __launch_bounds__(128) energy_rms_any_kernel(const float* __restrict__ x, const TrackDev* tr, float* fa, uint32_t hop, int bs) {
     __shared__ float tiles[4][32][33];
     const TrackDev& T = tr[blockIdx.y];
     const uint32_t nf = T.F[bs];
     const uint32_t f0 = (blockIdx.x * 4 + (threadIdx.x >> 5)) * 32;
     if (f0 >= nf || T.status != 0) return;
-    framed_rms_warp<2048>(x + T.off + T.trim_start, T.m, T.gain, hop, f0, nf, tiles[threadIdx.x >> 5], fa + T.erms);
+    framed_rms_warp<FRAME>(x + T.off + T.trim_start, T.m, T.gain, hop, f0, nf, tiles[threadIdx.x >> 5], fa + T.erms);
 }
 
+// hop 512: FRAME / 512 lanes per segment (4 at 2048, 8 at 4096, 16 at 8192), ERMS_GPW segments per warp
+template <int FRAME>
+constexpr int ERMS_GPW = 32 / (FRAME / 512);
+template <int FRAME>
 __global__ void __launch_bounds__(128) energy_rms_kernel(const float* __restrict__ x, const TrackDev* tr, float* fa) {
-    __shared__ float tiles[4][2][8][33];
+    constexpr int GPW = ERMS_GPW<FRAME>;
+    __shared__ float tiles[4][2][GPW][33];
     const TrackDev& T = tr[blockIdx.y];
     const uint32_t nf = T.F[0];  // > 0 only when the trimmed track holds a full frame
-    const uint32_t seg_first = (blockIdx.x * 4 + (threadIdx.x >> 5)) * 8;  // 8 segments per warp (4 lanes each)
+    const uint32_t seg_first = (blockIdx.x * 4 + (threadIdx.x >> 5)) * GPW;
     if (seg_first * ERMS_SEG >= nf || T.status != 0) return;
-    framed_rms_stream_warp<2048, 512, ERMS_SEG>(x + T.off + T.trim_start, T.m, T.gain, nf, seg_first, tiles[threadIdx.x >> 5], fa + T.erms);
+    framed_rms_stream_warp<FRAME, 512, ERMS_SEG>(x + T.off + T.trim_start, T.m, T.gain, nf, seg_first, tiles[threadIdx.x >> 5], fa + T.erms);
 }
 
 // Shared peak rule of the three detectors (energy_flux.rs:176-217, spectral_flux.rs:183-210, hfc.rs:180-204).
@@ -126,11 +132,11 @@ __device__ __forceinline__ SpecRows spec_rows(const TrackDev& T, const float* fa
     return SpecRows{fa + T.hop[h].spec, fa + T.hop[0].spec, fa + T.hop[h].frame + (uint64_t)FQ_ROWMAX * T.hop[h].fmax,
                     fa + T.hop[0].frame + (uint64_t)FQ_ROWMAX * T.hop[0].fmax};
 }
-template <int MODE>
+template <int MODE, int NB>
 __device__ __forceinline__ const float* spec_row(const SpecRows& R, uint32_t f) {
-    if (MODE == 1) return (f & 1u) ? R.own + (uint64_t)f * 1025 : R.base + (uint64_t)(f >> 1) * 1025;
-    if (MODE == 2) return R.base + (uint64_t)(2 * f) * 1025;
-    return R.own + (uint64_t)f * 1025;
+    if (MODE == 1) return (f & 1u) ? R.own + (uint64_t)f * NB : R.base + (uint64_t)(f >> 1) * NB;
+    if (MODE == 2) return R.base + (uint64_t)(2 * f) * NB;
+    return R.own + (uint64_t)f * NB;
 }
 template <int MODE>
 __device__ __forceinline__ float spec_rowmax(const SpecRows& R, uint32_t f) {
@@ -142,7 +148,8 @@ __device__ __forceinline__ float spec_rowmax(const SpecRows& R, uint32_t f) {
 constexpr int FEAT_RUN = 32;
 constexpr int HALO = 8;  // superflux radius upper bound (the ABI rejects larger values)
 
-template <int MODE>
+// NB: bins per row (frame_size / 2 + 1)
+template <int MODE, int NB>
 __global__ void __launch_bounds__(128) seq_feat_kernel(const TrackDev* tr, const int32_t* __restrict__ list, int h, float* fa) {
     // A warp owns 32 consecutive frames f0 .. f0+31 and produces the flux of the 31 pairs inside them: the normalised value
     // x[f][k] / max[f] that frame f contributes as "current" is the same number frame f+1 needs as "previous", so every lane
@@ -180,18 +187,18 @@ __global__ void __launch_bounds__(128) seq_feat_kernel(const TrackDev* tr, const
         E = __fadd_rn(E, __fmul_rn(cur, cur));
         H = __fadd_rn(H, __fmul_rn(__fmul_rn((float)k, cur), cur));  // hfc.rs:137
     };
-    for (uint32_t jb = 0; jb < 32; ++jb) {
+    for (uint32_t jb = 0; jb < (NB - 1) / 32; ++jb) {
 #pragma unroll 4
         for (int r = 0; r < 32; ++r) {
             const uint32_t fr_ = f0 + r;
-            tile[r][lane] = fr_ < F ? spec_row<MODE>(R, fr_)[jb * 32 + lane] : 0.0f;
+            tile[r][lane] = fr_ < F ? spec_row<MODE, NB>(R, fr_)[jb * 32 + lane] : 0.0f;
         }
         __syncwarp();
 #pragma unroll 4
         for (int j = 0; j < 32; ++j) step(jb * 32 + j, tile[lane][j]);
         __syncwarp();
     }
-    step(1024, valid ? spec_row<MODE>(R, f)[1024] : 0.0f);  // all lanes: the shuffle inside is warp-wide
+    step(NB - 1, valid ? spec_row<MODE, NB>(R, f)[NB - 1] : 0.0f);  // all lanes: the shuffle inside is warp-wide
     if (valid) {
         fr[FQ_E * fm + f] = E;
         fr[FQ_H * fm + f] = H;
@@ -199,28 +206,41 @@ __global__ void __launch_bounds__(128) seq_feat_kernel(const TrackDev* tr, const
     }
 }
 
+template <int NB>
 struct ParSmem {
-    float L[2][1025 + 2 * HALO + 7];
+    float L[2][NB + 2 * HALO + 7];
     float mel[2][MEL_MAX];
     float part[64];  // partial sums of the mel fold's chunks
 };
+// Warps per CTA: 4 at 1025 bins (static shared memory, 35 KB); 4 at 2049 (66 KB) and 2 at 4097 (66 KB) in dynamic shared memory,
+// so that three CTAs fit an SM at every size.
+template <int NB>
+constexpr int PAR_WARPS = NB <= 2049 ? 4 : 2;
 
 // K4: the SuperFlux radius is the default 4 (config.rs:634) — the pair pass then gives every lane four CONSECUTIVE bins: the twelve
 // previous-frame values their windows cover come from three 16-byte shared loads and the four 9-tap maxima share the maximum of the
 // six values common to all windows (17 FMNMX for four bins instead of 36 loads + 36 FMNMX, and a quarter of the shared-memory
 // instructions: ncu had the L1/shared pipe at 73 % on the lane-strided version).  Sums are warp trees either way (tolerance-level
 // consumers), so only their association changes.
-template <bool K4, int MODE>
-__global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const int32_t* __restrict__ list, const SrTables* srtab,
-                                                       const int32_t* sr_index, int h, float* fa, DevCfg cfg) {
-    __shared__ __align__(16) ParSmem sm[4];
+template <bool K4, int MODE, int NB>
+__global__ void __launch_bounds__(32 * PAR_WARPS<NB>) par_feat_kernel(const TrackDev* tr, const int32_t* __restrict__ list, const SrTables* srtab,
+                                                                     const int32_t* sr_index, int h, float* fa, DevCfg cfg) {
+    constexpr int W = PAR_WARPS<NB>;
+    ParSmem<NB>* sm;
+    if constexpr (NB == 1025) {
+        __shared__ __align__(16) ParSmem<NB> sm_static[W];
+        sm = sm_static;
+    } else {
+        extern __shared__ __align__(16) unsigned char par_dyn[];
+        sm = reinterpret_cast<ParSmem<NB>*>(par_dyn);
+    }
     const int t = list ? list[blockIdx.y] : blockIdx.y;
     const TrackDev& T = tr[t];
     const uint32_t F = T.F[h];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t f0 = (blockIdx.x * 4 + w) * FEAT_RUN;
+    const uint32_t f0 = (blockIdx.x * W + w) * FEAT_RUN;
     if (f0 >= F || T.status != 0) return;
-    ParSmem& S = sm[w];
+    ParSmem<NB>& S = sm[w];
     const SrTables& st = srtab[sr_index[t]];
     const HopLayout& HL = T.hop[h];
     float* fr = fa + HL.frame;
@@ -231,7 +251,7 @@ __global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const
     const int MK = (int)max(cfg.mel_k, 1u);
     const int nm = (int)st.n_mels;
     const int e0 = (int)st.b0, e1 = (int)st.b_low, e2 = (int)st.b_mid, e3 = (int)st.b_hi;
-    for (int i = lane; i < 1025 + 2 * HALO + 7; i += 32) S.L[0][i] = S.L[1][i] = 0.0f;  // halos stay zero: ln(1+x) >= 0 and the reference's running max starts at 0
+    for (int i = lane; i < NB + 2 * HALO + 7; i += 32) S.L[0][i] = S.L[1][i] = 0.0f;  // halos stay zero: ln(1+x) >= 0 and the reference's running max starts at 0
     __syncwarp();
     int cur = 0;
     const uint32_t f_first = f0 > 0 ? f0 - 1 : 0;
@@ -239,7 +259,7 @@ __global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const
     for (uint32_t f = f_first; f < f_last; ++f, cur ^= 1) {
         float* Lc = S.L[cur] + HALO;
         const float* Lp = S.L[cur ^ 1] + HALO;
-        const float* row = spec_row<MODE>(R, f);
+        const float* row = spec_row<MODE, NB>(R, f);
         const bool emit = f >= f0;           // this warp owns the outputs of frame f
         const bool pair = emit && f >= 1;    // pair (f-1, f) -> index f-1
         // per-band accumulators are selected with predicates, never indexed: a run-time index would put the arrays in local
@@ -257,12 +277,12 @@ __global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const
 #pragma unroll
             for (int u = 0; u < PF; ++u) xq[u] = __ldg(row + 32 * u + lane);
 #pragma unroll PF
-            for (int b0 = 0; b0 < 1025; b0 += 32) {
+            for (int b0 = 0; b0 < NB; b0 += 32) {
                 const int b = b0 + lane;
-                const bool in = b < 1025;
+                const bool in = b < NB;
                 const int u = (b0 >> 5) & (PF - 1);
                 const float x = in ? xq[u] : 0.0f;
-                if (b + 32 * PF < 1025) xq[u] = __ldg(row + b + 32 * PF);
+                if (b + 32 * PF < NB) xq[u] = __ldg(row + b + 32 * PF);
                 if (in) Lc[b] = logf(1.0f + fmaxf(x, 0.0f));  // novelty.rs:354
                 if (emit && in && b >= e0 && b < e3) {
                     const float xx = x * x, kx = (float)b * x * x;
@@ -299,8 +319,8 @@ __global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const
         if (pair) {
             if (K4) {
 #pragma unroll 2
-                for (int g = 0; g < 8; ++g) {
-                    const int b0 = 4 * lane + 128 * g;  // bins b0 .. b0+3 (<= 1023); windows cover Lp[b0-4 .. b0+7]
+                for (int g = 0; g < (NB - 1) / 128; ++g) {
+                    const int b0 = 4 * lane + 128 * g;  // bins b0 .. b0+3 (<= NB - 2); windows cover Lp[b0-4 .. b0+7]
                     const float4 va = *reinterpret_cast<const float4*>(Lp + b0 - 4);
                     const float4 vb = *reinterpret_cast<const float4*>(Lp + b0);
                     const float4 vc = *reinterpret_cast<const float4*>(Lp + b0 + 4);
@@ -316,13 +336,13 @@ __global__ void __launch_bounds__(128) par_feat_kernel(const TrackDev* tr, const
                     pair_bin(b0 + 2, fmaxf(m2, 0.0f), lc4.z);
                     pair_bin(b0 + 3, fmaxf(m3, 0.0f), lc4.w);
                 }
-                if (lane == 0) {  // bin 1024
+                if (lane == 0) {  // the last bin, NB - 1
                     float pm = 0.0f;
-                    for (int j = -4; j <= 4; ++j) pm = fmaxf(pm, Lp[1024 + j]);
-                    pair_bin(1024, pm, Lc[1024]);
+                    for (int j = -4; j <= 4; ++j) pm = fmaxf(pm, Lp[NB - 1 + j]);
+                    pair_bin(NB - 1, pm, Lc[NB - 1]);
                 }
             } else {
-                for (int b = lane; b < 1025; b += 32) {
+                for (int b = lane; b < NB; b += 32) {
                     float pm = 0.0f;
                     for (int j = -K; j <= K; ++j) pm = fmaxf(pm, Lp[b + j]);
                     pair_bin(b, pm, Lc[b]);
@@ -591,8 +611,11 @@ __global__ void __launch_bounds__(256) consensus_kernel(TrackDev* tr, int32_t* i
 
 void launch_energy_onsets(const WaveCtx& c) {
     if (c.max_F[c.cfg.bs] > 0) {
-        if (c.cfg.bs == 0) energy_rms_kernel<<<dim3((c.max_F[0] + ERMS_SEG * 32 - 1) / (ERMS_SEG * 32), c.n_tracks), 128, 0, c.stream>>>(c.samples, c.tracks, c.fa);
-        else energy_rms_any_kernel<<<dim3((c.max_F[c.cfg.bs] + 127) / 128, c.n_tracks), 128, 0, c.stream>>>(c.samples, c.tracks, c.fa, c.cfg.hop, c.cfg.bs);
+        with_frame(c.cfg.frame, [&](auto fc) {
+            constexpr int FR = decltype(fc)::F, PER_CTA = ERMS_SEG * 4 * ERMS_GPW<FR>;  // frames per CTA of the streamed form
+            if (c.cfg.bs == 0) energy_rms_kernel<FR><<<dim3((c.max_F[0] + PER_CTA - 1) / PER_CTA, c.n_tracks), 128, 0, c.stream>>>(c.samples, c.tracks, c.fa);
+            else energy_rms_any_kernel<FR><<<dim3((c.max_F[c.cfg.bs] + 127) / 128, c.n_tracks), 128, 0, c.stream>>>(c.samples, c.tracks, c.fa, c.cfg.hop, c.cfg.bs);
+        });
         count_launch("onsets");
     }
     energy_onset_kernel<<<c.n_tracks, 256, 0, c.stream>>>(c.tracks, c.fa, c.ia, c.cfg);
@@ -608,9 +631,12 @@ void launch_hpss_onsets(const WaveCtx& c) {
 
 static void launch_seq(const WaveCtx& c, int h, const int32_t* d_list, int n_list) {
     const dim3 grid((c.max_F[h] + 123) / 124, n_list);  // 4 warps x 31 new frames
-    if (h == 1) seq_feat_kernel<1><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
-    else if (h == 2) seq_feat_kernel<2><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
-    else seq_feat_kernel<0><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
+    with_frame(c.cfg.frame, [&](auto fc) {
+        constexpr int NB = decltype(fc)::B;
+        if (h == 1) seq_feat_kernel<1, NB><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
+        else if (h == 2) seq_feat_kernel<2, NB><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
+        else seq_feat_kernel<0, NB><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, h, c.fa);
+    });
     count_launch("spec_features");
 }
 
@@ -619,12 +645,31 @@ void launch_seq_features(const WaveCtx& c, int h, const int32_t* d_list, int n_l
     launch_seq(c, h, d_list, n_list);
 }
 
+template <bool K4, int MODE, int NB>
+static void launch_par_mode(const WaveCtx& c, int h, const int32_t* d_list, int n_list) {
+    constexpr int W = PAR_WARPS<NB>;
+    constexpr size_t smem = NB == 1025 ? 0 : W * sizeof(ParSmem<NB>);
+    if (smem > 0) {
+        static bool attr_dev[64] = {};  // function attributes are per device
+        int dev = 0;
+        cudaGetDevice(&dev);
+        if (!attr_dev[dev & 63]) {
+            cudaFuncSetAttribute(par_feat_kernel<K4, MODE, NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            attr_dev[dev & 63] = true;
+        }
+    }
+    const dim3 grid((c.max_F[h] + W * FEAT_RUN - 1) / (W * FEAT_RUN), n_list);
+    par_feat_kernel<K4, MODE, NB><<<grid, 32 * W, smem, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg);
+}
+
 template <bool K4>
 static void launch_par(const WaveCtx& c, int h, const int32_t* d_list, int n_list) {
-    const dim3 grid((c.max_F[h] + 127) / 128, n_list);
-    if (h == 1) par_feat_kernel<K4, 1><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg);
-    else if (h == 2) par_feat_kernel<K4, 2><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg);
-    else par_feat_kernel<K4, 0><<<grid, 128, 0, c.stream>>>(c.tracks, d_list, c.srtab, c.sr_index, h, c.fa, c.cfg);
+    with_frame(c.cfg.frame, [&](auto fc) {
+        constexpr int NB = decltype(fc)::B;
+        if (h == 1) launch_par_mode<K4, 1, NB>(c, h, d_list, n_list);
+        else if (h == 2) launch_par_mode<K4, 2, NB>(c, h, d_list, n_list);
+        else launch_par_mode<K4, 0, NB>(c, h, d_list, n_list);
+    });
     count_launch("spec_features");
 }
 

@@ -227,18 +227,21 @@ __global__ void __launch_bounds__(32) lufs_scan_kernel(const TrackDev* __restric
 }
 
 constexpr int SRMS_SEG = 16;  // hop-blocks per segment of the streamed frame-RMS (framed.cuh)
+// Frames of FRAME samples at hop FRAME / 2 (silence.rs:144)
+template <int FRAME>
 __global__ void __launch_bounds__(128) silence_rms_kernel(const float* __restrict__ x, TrackDev* tr, float* fa) {
     __shared__ float tiles[4][2][16][33];
     const int t = blockIdx.y;
     const TrackDev& T = tr[t];
     const uint32_t nf = T.Fsil;
-    if (T.n < 2048) {  // one short frame (silence.rs:154-169 on a track shorter than the frame): the tile scheme with its length-aware divisor
-        if (blockIdx.x == 0 && threadIdx.x < 32 && nf > 0) framed_rms_warp<2048>(x + T.off, T.n, T.gain, 1024, 0, nf, reinterpret_cast<float(*)[33]>(&tiles[0][0][0][0]), fa + T.sil_rms);
+    if (T.n < FRAME) {  // one short frame (silence.rs:154-169 on a track shorter than the frame): the tile scheme with its length-aware divisor
+        if (blockIdx.x == 0 && threadIdx.x < 32 && nf > 0)
+            framed_rms_warp<FRAME>(x + T.off, T.n, T.gain, FRAME / 2, 0, nf, reinterpret_cast<float(*)[33]>(&tiles[0][0][0][0]), fa + T.sil_rms);
         return;
     }
     const uint32_t seg_first = (blockIdx.x * 4 + (threadIdx.x >> 5)) * 16;  // 16 segments per warp (2 lanes each)
     if (seg_first * SRMS_SEG >= nf) return;
-    framed_rms_stream_warp<2048, 1024, SRMS_SEG>(x + T.off, T.n, T.gain, nf, seg_first, tiles[threadIdx.x >> 5], fa + T.sil_rms);
+    framed_rms_stream_warp<FRAME, FRAME / 2, SRMS_SEG>(x + T.off, T.n, T.gain, nf, seg_first, tiles[threadIdx.x >> 5], fa + T.sil_rms);
 }
 
 // detect_and_trim region logic — silence.rs:171-256.  One CTA per track.
@@ -252,7 +255,7 @@ __global__ void __launch_bounds__(256) trim_kernel(TrackDev* tr, const float* fa
     TrackDev& T = tr[t];
     const uint64_t n = T.n;
     const uint32_t nf = T.Fsil;
-    const uint32_t hop = 1024;
+    const uint32_t hop = cfg.frame / 2;
     if (threadIdx.x == 0) {
         s_first = 0xffffffffu;  // first non-silent frame
         s_last = 0u;            // last non-silent frame + 1
@@ -293,10 +296,10 @@ __global__ void __launch_bounds__(256) trim_kernel(TrackDev* tr, const float* fa
     const uint64_t m = te - ts;
     T.m = m;
     const uint32_t hops[N_HOPS] = {512, 256, 1024};
-    for (int h = 0; h < N_HOPS; ++h) T.F[h] = m >= 2048 ? (uint32_t)((m - 2048) / hops[h] + 1) : 0;
-    T.F[SLOT_BASE_ALT] = m >= 2048 ? (uint32_t)((m - 2048) / cfg.hop + 1) : 0;
+    for (int h = 0; h < N_HOPS; ++h) T.F[h] = frames_of(m, cfg.frame, hops[h]);
+    T.F[SLOT_BASE_ALT] = frames_of(m, cfg.frame, cfg.hop);
     T.F[SLOT_PERC] = T.F[cfg.bs];
-    T.Fk = m >= cfg.key_frame ? (uint32_t)((m - cfg.key_frame) / cfg.key_hop + 1) : 0;
+    T.Fk = frames_of(m, cfg.key_frame, cfg.key_hop);
     if (m == 0 && T.status == 0) {
         T.status = STRATUM_PROCESSING_ERROR;
         T.err_code = 3;  // "Audio is entirely silent after trimming" (lib.rs:143-147)
@@ -333,7 +336,8 @@ void launch_gain(const WaveCtx& c, const float* d_lufs_gain) {
 
 void launch_silence_trim(const WaveCtx& c) {
     if (c.cfg.enable_trim && c.max_Fsil > 0) {
-        silence_rms_kernel<<<dim3((c.max_Fsil + SRMS_SEG * 64 - 1) / (SRMS_SEG * 64), c.n_tracks), 128, 0, c.stream>>>(c.samples, c.tracks, c.fa);
+        const dim3 grid((c.max_Fsil + SRMS_SEG * 64 - 1) / (SRMS_SEG * 64), c.n_tracks);
+        with_frame(c.cfg.frame, [&](auto fc) { silence_rms_kernel<decltype(fc)::F><<<grid, 128, 0, c.stream>>>(c.samples, c.tracks, c.fa); });
         count_launch("preprocess");
     }
     trim_kernel<<<c.n_tracks, 256, 0, c.stream>>>(c.tracks, c.fa, c.n_tracks, c.cfg);

@@ -23,7 +23,8 @@ struct DevCfg {
     float cons_w[4];
     int32_t hpss_onsets, perc_fallback, emit_cands;
     uint32_t hpss_margin;
-    uint32_t hop;                 // hop_size of the base path (config.rs: 512); frame_size is 2048
+    uint32_t hop;                 // hop_size of the base path (config.rs: 512)
+    uint32_t frame, bins;         // frame_size of the tempo path (2048, 4096 or 8192: tempo_frame_supported) and its bin count frame/2 + 1
     int32_t bs;                   // slot of the base path: 0 (hop 512, shared with the multi-resolution pass) or SLOT_BASE_ALT
     uint32_t sf_k, mel_k;
     float nov_ws, nov_we, nov_wh;
@@ -76,6 +77,25 @@ struct DevCfg {
     uint32_t khpss_step, khpss_tm, khpss_fm;
     float khpss_power;
 };
+
+// Frame sizes of the tempo path (silence detector, energy flux, STFT and its feature kernels).  2048 is the default; 4096 and 8192
+// buy bass resolution.  Kernels that depend on the frame size are instantiated for exactly these three and dispatched by with_frame.
+__host__ __device__ inline bool tempo_frame_supported(uint32_t frame) { return frame == 2048 || frame == 4096 || frame == 8192; }
+
+// Frames of `frame` samples at `hop` in n samples (compute_stft, extractor.rs:301-359): the one frame-count rule of host and device.
+__host__ __device__ inline uint32_t frames_of(uint64_t n, uint32_t frame, uint32_t hop) { return n >= frame ? (uint32_t)((n - frame) / hop + 1) : 0; }
+
+template <int N>
+struct FrameC {
+    static constexpr int F = N, B = N / 2 + 1;
+};
+// Calls fn(FrameC<F>{}) with the configuration's frame size as a compile-time constant.
+template <class Fn>
+inline void with_frame(uint32_t frame, Fn&& fn) {
+    if (frame == 8192) fn(FrameC<8192>{});
+    else if (frame == 4096) fn(FrameC<4096>{});
+    else fn(FrameC<2048>{});
+}
 
 // Grids of more than AC_CAP hypotheses take the fine-grid kernels (distinct-lag tempogram, table lookups, comb filterbank across CTAs).
 __host__ __device__ inline bool fine_bpm_grid(const DevCfg& d) { return d.bpm_tab != nullptr; }
@@ -139,6 +159,7 @@ struct WaveCtx {
     uint32_t max_lufs_nb;
     uint32_t max_key_peaks;  // HPCP peak slots a frame may need: (band bins + 1) / 2 over the wave's sample rates
     GenStft gen_key;         // key STFT frames other than 2048 / 8192 points (n = 0: unused)
+    GenStft gen_tempo;       // tempo-path STFT tables at frame_size 4096 (n = 0: unused)
     uint32_t kband_stride_common;  // row stride of the compact key band when every live track of the wave has the same one, else 0
 };
 
