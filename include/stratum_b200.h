@@ -225,6 +225,47 @@ int32_t stratum_b200_analyze_batch_pcm(const void* pcm, const uint64_t* byte_off
                                        const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const int32_t* device_ids, uint32_t n_devices,
                                        StratumResult* out);
 
+/* ITU-R BS.1770-4 / EBU R128 loudness of a batch of interleaved PCM tracks (beyond the reference, which has no such output).
+ * Track i: `frames` sample frames of C channels at sr Hz, converted to f32 exactly as stratum_b200_analyze_batch_pcm converts them
+ * (but never mixed down).  S = (sr + 5) / 10 frames (100 ms).
+ *  - Channel weights (libebur128's default map): 1 channel L; 4 channels L R Ls Rs; 5 channels L R C Ls Rs; any other count
+ *    0 L, 1 R, 2 C, 3 unused (LFE), 4 Ls, 5 Rs, 6 and up unused.  L, R, C weigh 1.0, Ls and Rs 1.41, unused channels 0.
+ *  - K-weighting: a high shelf (f0 1681.974450955533 Hz, G 3.999843853973347 dB, Q 0.7071752369554196) and a high-pass
+ *    (f0 38.13547087602444 Hz, Q 0.5003270373238773) per channel in cascade, zero state at frame 0, coefficients derived per
+ *    sample rate from the analog prototype (at 48 kHz they equal BS.1770-4's tables).
+ *  - Momentary block j covers frames [jS, jS + 4S), j < J = max(0, floor(frames / S) - 3); short-term window k covers
+ *    [kS, kS + 30S), k < K = max(0, floor(frames / S) - 29).  Power = sum over channels of G_c * mean of y_c^2 over the block;
+ *    loudness l = -0.691 + 10 log10(power) (power 0: -INFINITY).
+ *  - integrated_lufs: mean power of the blocks with l > -70 and l > the relative gate (the loudness of the mean power of the blocks
+ *    above -70, minus 10 LU).  momentary_max_lufs / short_term_max_lufs: ungated maxima.  All three -INFINITY when undefined.
+ *  - loudness_range_lu (EBU Tech 3342): short-term values above -70 LUFS and above the loudness of their mean power minus 20 LU,
+ *    sorted ascending; P(p) = v[floor((n - 1) p + 0.5)]; LRA = P(0.95) - P(0.10), 0 when fewer than two values remain.
+ *  - sample_peak: max |x| over channels and frames.  true_peak: max(sample_peak, max |u|) where u is each channel upsampled by
+ *    L = 4 (sr < 96 kHz), 2 (sr < 192 kHz) or 1 with the 49 taps c[j] = sinc((j - 24) / L) * 0.5 (1 - cos(2 pi j / 48)), samples
+ *    outside the track zero.  Both linear, full scale 1.0.
+ * Per-track failures (status/error, the batch carries on): 0 frames or sr = 0 -> STRATUM_INVALID_INPUT; sr outside 8000..384000 Hz
+ * -> STRATUM_NOT_IMPLEMENTED.  Calls with a null pointer, an unknown format, channels outside 1..64 or a partial frame are rejected
+ * whole (STRATUM_INVALID_INPUT).  Results are bit-identical whatever the batch, the upload chunks and the devices. */
+typedef struct StratumLoudness {
+    int32_t status; char error[128];
+    uint32_t sample_rate, channels; uint64_t frames;
+    double integrated_lufs, momentary_max_lufs, short_term_max_lufs;  /* -INFINITY when undefined (see above) */
+    double loudness_range_lu;
+    double sample_peak, true_peak;                                     /* linear full scale */
+    uint32_t n_momentary, n_short_term;                                /* J and K */
+} StratumLoudness;
+
+/* Host PCM (layout of stratum_b200_analyze_batch_pcm), sharded over `device_ids` and streamed through the double-buffered upload. */
+int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                        const uint32_t* formats, uint32_t n_tracks, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out);
+/* Same, with the PCM already resident in the memory of device `device_id`. */
+int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                               const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out);
+/* Host-side filters of the loudness measurement (no device work): kweight10 = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2 (either
+ * may be NULL), taps49 = the true-peak interpolator as the device uses it (f32).  Returns the oversampling factor L, or -1 for a
+ * sample rate outside 8000..384000 Hz. */
+int32_t stratum_b200_debug_loudness_filters(uint32_t sample_rate, double* kweight10, float* taps49);
+
 /* Same, with `samples` already resident in the memory of device `device_id` (single device). */
 int32_t stratum_b200_analyze_batch_device(const float* d_samples, const uint64_t* offsets, const uint32_t* sample_rates, uint32_t n_tracks,
                                           const StratumConfig* cfg, int32_t device_id, StratumResult* out);
@@ -255,7 +296,7 @@ int32_t stratum_b200_device_count(void);
 /* Frees the per-process device contexts. */
 void stratum_b200_shutdown(void);
 
-/* sizeof(StratumConfig) / sizeof(StratumResult) / sizeof(StratumConfidence) for which = 0 / 1 / 2:
+/* sizeof(StratumConfig) / sizeof(StratumResult) / sizeof(StratumConfidence) / sizeof(StratumLoudness) for which = 0 / 1 / 2 / 3:
  * lets an FFI binding assert that its mirror of the structs matches this build. */
 size_t stratum_b200_sizeof(int32_t which);
 

@@ -186,6 +186,74 @@ pub fn analyze_batch(tracks: &[&[f32]], sample_rates: &[u32], config: AnalysisCo
     Ok(out)
 }
 
+/// One track of undecoded interleaved PCM for `loudness_batch_pcm`: `data` holds whole sample frames, little-endian, 24-bit
+/// samples packed in 3 bytes; `format` is a `STRATUM_PCM_*` value (1 = u8 ... 6 = f64).
+pub struct PcmTrack<'a> {
+    pub data: &'a [u8],
+    pub format: u32,
+    pub channels: u32,
+    pub sample_rate: u32,
+}
+
+/// ITU-R BS.1770-4 / EBU R128 loudness of one track (`StratumLoudness` in `include/stratum_b200.h`): LUFS, LU and linear peaks;
+/// undefined loudness values are `f64::NEG_INFINITY`.
+#[derive(Clone, Copy, Debug, PartialEq)]
+pub struct Loudness {
+    pub integrated_lufs: f64,
+    pub momentary_max_lufs: f64,
+    pub short_term_max_lufs: f64,
+    pub loudness_range_lu: f64,
+    pub sample_peak: f64,
+    pub true_peak: f64,
+    pub n_momentary: u32,
+    pub n_short_term: u32,
+}
+
+/// Loudness of a batch of PCM tracks, measured on the device and sharded over `devices` (empty: the current device).  The outer
+/// error rejects the whole call (no device, malformed input); a track that fails on its own carries its error in its slot.
+pub fn loudness_batch_pcm(tracks: &[PcmTrack], devices: &[i32]) -> Result<Vec<Result<Loudness, AnalysisError>>, AnalysisError> {
+    let ok = unsafe { stratum_b200_sizeof(3) == std::mem::size_of::<StratumLoudness>() };
+    if !ok {
+        return Err(AnalysisError::ProcessingError("libstratum_b200.so does not match this binding (struct sizes differ)".to_string()));
+    }
+    let n = tracks.len();
+    let mut offsets = vec![0u64];
+    let mut flat: Vec<u8> = Vec::new();
+    for t in tracks {
+        flat.extend_from_slice(t.data);
+        offsets.push(flat.len() as u64);
+    }
+    let srs: Vec<u32> = tracks.iter().map(|t| t.sample_rate).collect();
+    let chans: Vec<u32> = tracks.iter().map(|t| t.channels).collect();
+    let fmts: Vec<u32> = tracks.iter().map(|t| t.format).collect();
+    let mut res: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
+    let st = unsafe {
+        stratum_b200_loudness_batch_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32,
+                                        if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32, res.as_mut_ptr())
+    };
+    if st != 0 {
+        return Err(to_error(st, last_error()));
+    }
+    Ok(res
+        .iter()
+        .map(|r| {
+            if r.status != 0 {
+                return Err(to_error(r.status, c_string(&r.error)));
+            }
+            Ok(Loudness {
+                integrated_lufs: r.integrated_lufs,
+                momentary_max_lufs: r.momentary_max_lufs,
+                short_term_max_lufs: r.short_term_max_lufs,
+                loudness_range_lu: r.loudness_range_lu,
+                sample_peak: r.sample_peak,
+                true_peak: r.true_peak,
+                n_momentary: r.n_momentary,
+                n_short_term: r.n_short_term,
+            })
+        })
+        .collect())
+}
+
 /// Decoder-side batch entry: interleaved 16-bit PCM uploaded as is and converted on the device with the arithmetic of
 /// `examples/analyze_batch.rs:96-113` (half the PCIe bytes of f32).
 pub fn analyze_batch_pcm16(tracks: &[&[i16]], sample_rates: &[u32], channels: &[u32], config: AnalysisConfig, devices: &[i32]) -> Result<Vec<Result<AnalysisResult, AnalysisError>>, AnalysisError> {

@@ -123,6 +123,15 @@ class StratumConfidence(C.Structure):
     _fields_ = [("bpm_confidence", _f), ("key_confidence", _f), ("grid_stability", _f), ("overall_confidence", _f), ("flags", _u)]
 
 
+class StratumLoudness(C.Structure):
+    _fields_ = [
+        ("status", _i), ("error", C.c_char * 128), ("sample_rate", _u), ("channels", _u), ("frames", C.c_uint64),
+        ("integrated_lufs", C.c_double), ("momentary_max_lufs", C.c_double), ("short_term_max_lufs", C.c_double),
+        ("loudness_range_lu", C.c_double), ("sample_peak", C.c_double), ("true_peak", C.c_double),
+        ("n_momentary", _u), ("n_short_term", _u),
+    ]
+
+
 _lib: C.CDLL | None = None
 
 
@@ -192,8 +201,15 @@ def lib() -> C.CDLL:
     L.stratum_b200_last_call_waves.restype = _u
     L.stratum_b200_transfer_bytes.argtypes = [u64p, u64p]
     L.stratum_b200_transfer_bytes.restype = None
+    loudp = C.POINTER(StratumLoudness)
+    L.stratum_b200_loudness_batch_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, i32p, _u, loudp]
+    L.stratum_b200_loudness_batch_pcm.restype = _i
+    L.stratum_b200_loudness_batch_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, _i, loudp]
+    L.stratum_b200_loudness_batch_pcm_device.restype = _i
+    L.stratum_b200_debug_loudness_filters.argtypes = [_u, C.POINTER(C.c_double), f32p]
+    L.stratum_b200_debug_loudness_filters.restype = _i
     if L.stratum_b200_sizeof(0) != C.sizeof(StratumConfig) or L.stratum_b200_sizeof(1) != C.sizeof(StratumResult) or \
-            L.stratum_b200_sizeof(2) != C.sizeof(StratumConfidence):
+            L.stratum_b200_sizeof(2) != C.sizeof(StratumConfidence) or L.stratum_b200_sizeof(3) != C.sizeof(StratumLoudness):
         raise RuntimeError("ctypes mirror of include/stratum_b200.h is out of date (struct size mismatch)")
     _lib = L
     return L
@@ -565,6 +581,90 @@ def analyze_batch_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None 
     if st != OK:
         _fail(st, res, n)
     return _collect(res, n)
+
+
+@dataclass
+class Loudness:
+    """ITU-R BS.1770-4 / EBU R128 loudness of one track (include/stratum_b200.h: StratumLoudness).  Loudness values are in LUFS,
+    the range in LU, peaks linear (full scale 1.0); undefined loudness values are ``float("-inf")``."""
+
+    integrated_lufs: float
+    momentary_max_lufs: float
+    short_term_max_lufs: float
+    loudness_range_lu: float
+    sample_peak: float
+    true_peak: float
+    n_momentary: int
+    n_short_term: int
+    sample_rate: int
+    channels: int
+    frames: int
+    error: AnalysisError | None = None  # set instead of raising for a track that failed on its own
+
+
+def _loudness(r: StratumLoudness) -> Loudness:
+    err = AnalysisError(r.status, r.error.decode(errors="replace")) if r.status != OK else None
+    return Loudness(r.integrated_lufs, r.momentary_max_lufs, r.short_term_max_lufs, r.loudness_range_lu, r.sample_peak, r.true_peak,
+                    int(r.n_momentary), int(r.n_short_term), int(r.sample_rate), int(r.channels), int(r.frames), err)
+
+
+def _pcm_tables(tracks: Sequence[PcmTrack]):
+    n = len(tracks)
+    offsets = np.zeros(n + 1, dtype=np.uint64)
+    offsets[1:] = np.cumsum([t.data.size for t in tracks], dtype=np.uint64)
+    srs = np.ascontiguousarray([t.sample_rate for t in tracks], dtype=np.uint32)
+    chans = np.ascontiguousarray([t.channels for t in tracks], dtype=np.uint32)
+    fmts = np.ascontiguousarray([t.fmt for t in tracks], dtype=np.uint32)
+    return offsets, srs, chans, fmts
+
+
+def loudness_batch_pcm(tracks: Sequence[PcmTrack], devices: Sequence[int] | None = None) -> list:
+    """stratum_b200_loudness_batch_pcm: integrated loudness, maxima, loudness range and peaks of undecoded PCM tracks, measured on
+    the device and sharded over ``devices`` (default: the current device).  A failed track carries ``.error``."""
+    n = len(tracks)
+    if n == 0:
+        return []
+    flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
+    cat = np.concatenate(flat) if n > 1 else flat[0]
+    offsets, srs, chans, fmts = _pcm_tables(tracks)
+    res = (StratumLoudness * n)()
+    dev = (C.c_int32 * len(devices))(*devices) if devices else None
+    st = lib().stratum_b200_loudness_batch_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                               srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
+                                               n, dev, len(devices) if devices else 0, res)
+    if st != OK:
+        _raise(st)
+    return [_loudness(res[i]) for i in range(n)]
+
+
+def loudness_batch_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
+                              device: int = -1) -> list:
+    """stratum_b200_loudness_batch_pcm_device: the same with the PCM already in device memory (``d_pcm_ptr`` = device address of the
+    concatenated track bytes, e.g. ``tensor.data_ptr()``; track i = bytes [byte_offsets[i], byte_offsets[i + 1]))."""
+    offsets = np.ascontiguousarray(byte_offsets, dtype=np.uint64)
+    n = offsets.size - 1
+    srs = np.ascontiguousarray(sample_rates, dtype=np.uint32)
+    chans = np.ascontiguousarray(channels, dtype=np.uint32)
+    fmts = np.ascontiguousarray(formats, dtype=np.uint32)
+    if not (srs.size == chans.size == fmts.size == n):
+        raise ValueError("one sample rate, channel count and format per track")
+    res = (StratumLoudness * max(n, 1))()
+    st = lib().stratum_b200_loudness_batch_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)), srs.ctypes.data_as(C.POINTER(_u)),
+                                                      chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)), n, device, res)
+    if st != OK:
+        _raise(st)
+    return [_loudness(res[i]) for i in range(n)]
+
+
+def loudness_filters(sample_rate: int) -> tuple:
+    """The host-side filters of the loudness measurement: (K-weighting coefficients [b0 b1 b2 a1 a2] x 2 stages in float64,
+    true-peak taps in float32, oversampling factor).  Raises for a sample rate outside 8000..384000 Hz."""
+    k = np.zeros(10, np.float64)
+    t = np.zeros(49, np.float32)
+    L = lib().stratum_b200_debug_loudness_filters(int(sample_rate), k.ctypes.data_as(C.POINTER(C.c_double)), t.ctypes.data_as(C.POINTER(_f)))
+    if L < 0:
+        raise AnalysisError(4, f"sample rate {sample_rate} Hz is outside 8000..384000 Hz")
+    return k, t, L
 
 
 def analyze_batch_device(d_samples_ptr: int, offsets: np.ndarray, sample_rates: Sequence[int], config: AnalysisConfig | None = None,

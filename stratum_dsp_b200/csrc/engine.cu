@@ -148,6 +148,18 @@ struct PinnedBuf {
     }
 };
 
+// Grow-only device buffer.
+template <class T>
+static bool grow_device(T*& p, size_t& cap, size_t need) {
+    if (need <= cap) return true;
+    if (p) cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    if (cudaMalloc((void**)&p, need) != cudaSuccess) return false;
+    cap = need;
+    return true;
+}
+
 // One long-lived helper thread per device (the sample uploads of host batches): tasks run in order.
 class Worker {
 public:
@@ -243,6 +255,10 @@ struct DeviceCtx {
     char* d_meta = nullptr;   // per-chunk offset / channel tables of the PCM16 path (two sets)
     size_t meta_cap = 0;
     PinnedBuf h_meta[2];      // their pinned host images
+    char* d_loud = nullptr;   // loudness work area of one chunk (track records, results, cascade states, energies, per-segment powers)
+    size_t loud_cap = 0;
+    PinnedBuf loud_rec[2], loud_out[2];  // pinned track records / results of two chunks (chunk k+1 is queued before chunk k is read)
+    cudaEvent_t loud_ev[2] = {nullptr, nullptr};
     int32_t* d_count = nullptr;  // escalated tracks of the wave being queued (escalation_compact_kernel)
     PinnedBuf h_count;
     cudaEvent_t ev_legacy = nullptr;  // legacy estimator finished on the key stream
@@ -2101,38 +2117,49 @@ static uint32_t pcm_bytes_per_sample(uint32_t fmt) {
     }
 }
 
-// boff: byte offsets of the tracks inside src (n_tracks + 1).  formats == nullptr: mono f32 samples analysed straight from the staging
-// buffer; otherwise interleaved PCM in the given per-track format and channel count, converted and mixed down on the device.
-static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const uint32_t* sample_rates, const uint32_t* channels, const uint32_t* formats,
-                                  uint32_t n_tracks, const StratumConfig* cfg, const int32_t* device_ids, uint32_t n_devices, StratumResult* out) {
-    const bool pcm = formats != nullptr;
-    if (!boff || !sample_rates || !out || (!src && n_tracks && boff[n_tracks] > 0) || (pcm && !channels)) {
-        set_error("null argument");
-        return STRATUM_INVALID_INPUT;
-    }
-    StratumConfig def;
-    config_default(&def);
-    const StratumConfig& c = cfg ? *cfg : def;
-    int st = config_validate(c);
-    if (st != STRATUM_OK) return st;
-    if (n_tracks == 0) return STRATUM_OK;
-    std::vector<uint32_t> bpf(n_tracks, 4);  // bytes per mono frame
-    if (pcm)
-        for (uint32_t i = 0; i < n_tracks; ++i) {
-            const uint32_t bps = pcm_bytes_per_sample(formats[i]);
-            if (bps == 0) {
-                set_error("unknown PCM sample format (STRATUM_PCM_*)");
-                return STRATUM_INVALID_INPUT;
-            }
-            if (channels[i] == 0 || channels[i] > 64 || (boff[i + 1] - boff[i]) % ((uint64_t)bps * channels[i]) != 0) {
-                set_error("PCM track length is not a whole number of frames (or channels outside 1..64)");
-                return STRATUM_INVALID_INPUT;
-            }
-            bpf[i] = bps * channels[i];
+// Bytes per frame of every PCM track into bpf; rejects the whole call on an unknown format, a channel count outside 1..64 or a
+// partial frame.
+static int pcm_frame_bytes(const uint64_t* boff, const uint32_t* channels, const uint32_t* formats, uint32_t n_tracks, std::vector<uint32_t>& bpf) {
+    for (uint32_t i = 0; i < n_tracks; ++i) {
+        const uint32_t bps = pcm_bytes_per_sample(formats[i]);
+        if (bps == 0) {
+            set_error("unknown PCM sample format (STRATUM_PCM_*)");
+            return STRATUM_INVALID_INPUT;
         }
+        if (channels[i] == 0 || channels[i] > 64 || (boff[i + 1] - boff[i]) % ((uint64_t)bps * channels[i]) != 0) {
+            set_error("PCM track length is not a whole number of frames (or channels outside 1..64)");
+            return STRATUM_INVALID_INPUT;
+        }
+        bpf[i] = bps * channels[i];
+    }
+    return STRATUM_OK;
+}
+
+// Chunk of a shard: tracks [i, j), `elems` bytes of host data, `frames` sample frames.
+struct HostChunk {
+    uint32_t i, j;
+    uint64_t elems, frames;
+};
+
+// The device work of one shard of a host batch, fed chunk by chunk by stream_host_batch.  Every method returns a StratumStatus and
+// leaves its message in g_last_error.
+struct ChunkSink {
+    virtual ~ChunkSink() = default;
+    virtual int open(const std::vector<HostChunk>& chunks) = 0;  // before the first upload; chunks are those of the shard
+    // Chunk k is staged at d_buf (byte 0 = the first byte of track ch.i).  after_prev must be called once, as soon as the device no
+    // longer reads the previous chunk's staging buffer: it starts the upload of chunk k + 1 into that buffer.
+    virtual int chunk(size_t k, const HostChunk& ch, const char* d_buf, const std::function<void()>& after_prev) = 0;
+    virtual int close() = 0;  // after the last chunk, and after a failure
+};
+
+// boff: byte offsets of the tracks inside src (n_tracks + 1); bpf: bytes per sample frame of every track.  The tracks are cut into
+// contiguous shards, one per device context (an id named twice, or -1 next to the current device's id, is one shard, not two), each
+// streamed by its own host thread through the context's staging buffers into the sink make_sink(ctx) returns.
+static int32_t stream_host_batch(const void* src, const uint64_t* boff, const std::vector<uint32_t>& bpf, uint32_t n_tracks, const int32_t* device_ids,
+                                 uint32_t n_devices, const std::function<std::unique_ptr<ChunkSink>(DeviceCtx*)>& make_sink) {
+    int st = STRATUM_OK;
     const uint64_t* offsets = boff;
     const size_t elt = 1;  // offsets are in bytes
-    // device contexts of the call; an id named twice (or -1 next to the current device's id) is one shard, not two
     std::vector<DeviceCtx*> ctxs;
     {
         std::vector<int32_t> devs;
@@ -2168,14 +2195,9 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
         uint64_t chunk_frames = (uint64_t)128 * 7938000;  // = the wave cap of a session: one full-size chunk is one wave
         if (const char* e = getenv("STRATUM_B200_STAGE_MB")) chunk_frames = std::max<uint64_t>((uint64_t)(atof(e) * 1024 * 1024 / 4), 1u << 16);
         static const bool no_ramp = getenv("STRATUM_B200_STAGE_NO_RAMP") != nullptr;
-        struct Chunk {
-            uint32_t i, j;
-            uint64_t elems, frames;
-        };
         auto frames_of_track = [&](uint32_t q) { return (offsets[q + 1] - offsets[q]) / bpf[q]; };
-        std::vector<Chunk> chunks;
-        uint64_t max_el = 0, max_fr = 0;
-        uint32_t max_cn = 0;
+        std::vector<HostChunk> chunks;
+        uint64_t max_el = 0;
         // ramp: "a,b" = first chunk a/8 of a full chunk, growth by b/8 of a full chunk per step (default 2,2: 1/4, 1/2, 3/4, 1 ...)
         static const char* ramp_env = getenv("STRATUM_B200_STAGE_RAMP");
         int ramp_first = 2, ramp_step = 2;
@@ -2191,10 +2213,8 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
                 ++j;
             }
             const uint64_t el = offsets[j] - offsets[i];
-            chunks.push_back(Chunk{i, j, el, fr});
+            chunks.push_back(HostChunk{i, j, el, fr});
             max_el = std::max(max_el, el);
-            max_fr = std::max(max_fr, fr);
-            max_cn = std::max(max_cn, j - i);
             i = j;
             cur_frames = std::min<uint64_t>(chunk_frames, cur_frames + chunk_frames * ramp_step / 8);
         }
@@ -2202,23 +2222,8 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
         {
             if (!ctx->copy_stream && cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking) != cudaSuccess)
                 return fail(STRATUM_PROCESSING_ERROR, "copy stream creation failed");
-            auto grow = [&](void** p, size_t* cap, size_t need) {
-                if (need <= *cap) return true;
-                if (*p) cudaFree(*p);
-                *p = nullptr;
-                *cap = 0;
-                if (cudaMalloc(p, need) != cudaSuccess) return false;
-                *cap = need;
-                return true;
-            };
-            bool okm = grow((void**)&ctx->d_stage, &ctx->stage_cap, 2 * buf_bytes);
-            if (okm && pcm) okm = grow((void**)&ctx->d_conv, &ctx->conv_cap, (max_fr + 16) * sizeof(float));
-            // per-chunk offset / channel tables of the PCM16 path, two sets (the conversion of chunk k+1 is queued while chunk k runs)
-            const size_t meta_each = (size_t)align_up((size_t)(max_cn + 1) * 16 + (size_t)max_cn * 8 + 64, 256);
-            if (okm && pcm) okm = grow((void**)&ctx->d_meta, &ctx->meta_cap, 2 * meta_each);
-            if (!okm) return fail(STRATUM_PROCESSING_ERROR, "staging buffer allocation failed");
+            if (!grow_device(ctx->d_stage, ctx->stage_cap, 2 * buf_bytes)) return fail(STRATUM_PROCESSING_ERROR, "staging buffer allocation failed");
         }
-        const size_t meta_each = (size_t)align_up((size_t)(max_cn + 1) * 16 + (size_t)max_cn * 8 + 64, 256);
         char* bufs[2] = {reinterpret_cast<char*>(ctx->d_stage), reinterpret_cast<char*>(ctx->d_stage) + buf_bytes};
         if (!ctx->uploader) ctx->uploader.reset(new Worker());
         // Uploads run on the device's uploader thread, in pieces of 128 MB with a stream synchronisation after each piece: the
@@ -2226,7 +2231,7 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
         // queue behind a multi-gigabyte transfer on the copy engine and stall the wave until the next chunk has landed (measured:
         // no overlap at all with 2 GB transfers enqueued in one piece).
         auto upload = [&, ctx](size_t k) -> bool {
-            const Chunk& ch = chunks[k];
+            const HostChunk& ch = chunks[k];
             if (cudaSetDevice(ctx->device) != cudaSuccess) return false;
             g_h2d_bytes.fetch_add(ch.elems * elt);
             const char* hsrc = static_cast<const char*>(src) + offsets[ch.i] * elt;
@@ -2237,8 +2242,8 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
             }
             return true;
         };
-        Session S(*ctx, c);
-        int s2 = S.open();
+        std::unique_ptr<ChunkSink> sink = make_sink(ctx);
+        int s2 = sink->open(chunks);
         if (s2 != STRATUM_OK) return fail(s2, g_last_error);
         std::future<bool> up = ctx->uploader->post([&] { return upload(0); });
         bool ok = true;
@@ -2251,47 +2256,8 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
                 fail(STRATUM_PROCESSING_ERROR, "host to device copy failed");
                 break;
             }
-            const Chunk& ch = chunks[k];
-            const uint32_t cn = ch.j - ch.i;
-            std::vector<uint64_t> rel(cn + 1, 0), lens(cn);  // per-track offsets in mono frames inside the chunk
-            for (uint32_t q = 0; q < cn; ++q) {
-                lens[q] = frames_of_track(ch.i + q);
-                rel[q + 1] = rel[q] + lens[q];
-            }
-            const float* d_mono = reinterpret_cast<const float*>(bufs[k & 1]);
-            if (pcm) {
-                // decoder arithmetic on the device: interleaved PCM -> mono f32 (examples/analyze_batch.rs:70-165).  Queued on
-                // the analysis stream, so it runs after the previous chunk's waves have finished with the conversion buffer.
-                char* hm = static_cast<char*>(ctx->h_meta[k & 1].need(meta_each));
-                if (!hm) {
-                    fail(STRATUM_PROCESSING_ERROR, "pinned host allocation failed");
-                    break;
-                }
-                uint64_t* h_poff = reinterpret_cast<uint64_t*>(hm);
-                uint64_t* h_ooff = h_poff + (cn + 1);
-                uint32_t* h_ch = reinterpret_cast<uint32_t*>(h_ooff + (cn + 1));
-                uint32_t* h_fmt = h_ch + cn;
-                uint64_t max_frames = 0;
-                for (uint32_t q = 0; q <= cn; ++q) {
-                    h_poff[q] = offsets[ch.i + q] - offsets[ch.i];
-                    h_ooff[q] = rel[q];
-                }
-                for (uint32_t q = 0; q < cn; ++q) {
-                    h_ch[q] = channels[ch.i + q];
-                    h_fmt[q] = formats[ch.i + q];
-                    max_frames = std::max(max_frames, lens[q]);
-                }
-                char* dm = ctx->d_meta + (k & 1) * meta_each;
-                uint64_t* d_poff = reinterpret_cast<uint64_t*>(dm);
-                uint64_t* d_ooff = d_poff + (cn + 1);
-                uint32_t* d_ch = reinterpret_cast<uint32_t*>(d_ooff + (cn + 1));
-                uint32_t* d_fmt = d_ch + cn;
-                cudaMemcpyAsync(dm, hm, (size_t)(cn + 1) * 16 + (size_t)cn * 8, cudaMemcpyHostToDevice, ctx->stream);
-                launch_pcm_to_mono(ctx->stream, bufs[k & 1], ctx->d_conv, d_poff, d_ooff, d_ch, d_fmt, cn, max_frames);
-                d_mono = ctx->d_conv;
-            }
             bool posted = false;
-            auto after_prev = [&] {  // the previous chunk's waves are gathered: its staging buffer takes chunk k+1
+            auto after_prev = [&] {  // the previous chunk's work is done: its staging buffer takes chunk k+1
                 if (k + 1 < chunks.size()) {
                     up = ctx->uploader->post([&, k] { return upload(k + 1); });
                     posted = true;
@@ -2299,7 +2265,7 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
             };
             {
                 HostSpan span_an("host_chunk_submit");  // wall time of queueing the chunk (includes gathering the previous one)
-                s2 = S.submit(d_mono, rel.data(), lens.data(), sample_rates + ch.i, cn, out + ch.i, after_prev);
+                s2 = sink->chunk(k, chunks[k], bufs[k & 1], after_prev);
             }
             if (s2 != STRATUM_OK) {
                 fail(s2, g_last_error);
@@ -2308,9 +2274,8 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
                 break;
             }
         }
-        s2 = S.drain();
+        s2 = sink->close();
         if (s2 != STRATUM_OK) fail(s2, g_last_error);
-        S.close();
         cudaStreamSynchronize(ctx->copy_stream);
     };
     if (nd == 1) {
@@ -2326,6 +2291,428 @@ static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const u
             return status[d];
         }
     return STRATUM_OK;
+}
+
+// The analysis of the staged chunks: mono f32 samples straight from the staging buffer, or interleaved PCM (formats != nullptr)
+// converted and mixed down on the device into the conversion buffer first.  The waves run one ahead of the gather (Session).
+struct AnalysisSink final : ChunkSink {
+    DeviceCtx* ctx;
+    Session S;
+    const uint64_t* offsets;
+    const std::vector<uint32_t>& bpf;
+    const uint32_t *sample_rates, *channels, *formats;
+    StratumResult* out;
+    size_t meta_each = 0;
+    AnalysisSink(DeviceCtx* c, const StratumConfig& cfg, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans,
+                 const uint32_t* fmts, StratumResult* o)
+        : ctx(c), S(*c, cfg), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o) {}
+    uint64_t frames_of_track(uint32_t q) const { return (offsets[q + 1] - offsets[q]) / bpf[q]; }
+
+    int open(const std::vector<HostChunk>& chunks) override {
+        if (formats) {
+            uint64_t max_fr = 0;
+            uint32_t max_cn = 0;
+            for (const HostChunk& ch : chunks) {
+                max_fr = std::max(max_fr, ch.frames);
+                max_cn = std::max(max_cn, ch.j - ch.i);
+            }
+            // per-chunk offset / channel tables of the PCM path, two sets (the conversion of chunk k+1 is queued while chunk k runs)
+            meta_each = (size_t)align_up((size_t)(max_cn + 1) * 16 + (size_t)max_cn * 8 + 64, 256);
+            if (!grow_device(ctx->d_conv, ctx->conv_cap, (max_fr + 16) * sizeof(float)) || !grow_device(ctx->d_meta, ctx->meta_cap, 2 * meta_each)) {
+                set_error("staging buffer allocation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
+        }
+        return S.open();
+    }
+
+    int chunk(size_t k, const HostChunk& ch, const char* d_buf, const std::function<void()>& after_prev) override {
+        const uint32_t cn = ch.j - ch.i;
+        std::vector<uint64_t> rel(cn + 1, 0), lens(cn);  // per-track offsets in mono frames inside the chunk
+        for (uint32_t q = 0; q < cn; ++q) {
+            lens[q] = frames_of_track(ch.i + q);
+            rel[q + 1] = rel[q] + lens[q];
+        }
+        const float* d_mono = reinterpret_cast<const float*>(d_buf);
+        if (formats) {
+            // decoder arithmetic on the device: interleaved PCM -> mono f32 (examples/analyze_batch.rs:70-165).  Queued on
+            // the analysis stream, so it runs after the previous chunk's waves have finished with the conversion buffer.
+            char* hm = static_cast<char*>(ctx->h_meta[k & 1].need(meta_each));
+            if (!hm) {
+                set_error("pinned host allocation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
+            uint64_t* h_poff = reinterpret_cast<uint64_t*>(hm);
+            uint64_t* h_ooff = h_poff + (cn + 1);
+            uint32_t* h_ch = reinterpret_cast<uint32_t*>(h_ooff + (cn + 1));
+            uint32_t* h_fmt = h_ch + cn;
+            uint64_t max_frames = 0;
+            for (uint32_t q = 0; q <= cn; ++q) {
+                h_poff[q] = offsets[ch.i + q] - offsets[ch.i];
+                h_ooff[q] = rel[q];
+            }
+            for (uint32_t q = 0; q < cn; ++q) {
+                h_ch[q] = channels[ch.i + q];
+                h_fmt[q] = formats[ch.i + q];
+                max_frames = std::max(max_frames, lens[q]);
+            }
+            char* dm = ctx->d_meta + (k & 1) * meta_each;
+            uint64_t* d_poff = reinterpret_cast<uint64_t*>(dm);
+            uint64_t* d_ooff = d_poff + (cn + 1);
+            uint32_t* d_ch = reinterpret_cast<uint32_t*>(d_ooff + (cn + 1));
+            uint32_t* d_fmt = d_ch + cn;
+            cudaMemcpyAsync(dm, hm, (size_t)(cn + 1) * 16 + (size_t)cn * 8, cudaMemcpyHostToDevice, ctx->stream);
+            launch_pcm_to_mono(ctx->stream, d_buf, ctx->d_conv, d_poff, d_ooff, d_ch, d_fmt, cn, max_frames);
+            d_mono = ctx->d_conv;
+        }
+        return S.submit(d_mono, rel.data(), lens.data(), sample_rates + ch.i, cn, out + ch.i, after_prev);
+    }
+
+    int close() override {
+        const int st = S.drain();
+        S.close();
+        return st;
+    }
+};
+
+// boff: byte offsets of the tracks inside src (n_tracks + 1).  formats == nullptr: mono f32 samples analysed straight from the staging
+// buffer; otherwise interleaved PCM in the given per-track format and channel count, converted and mixed down on the device.
+static int32_t analyze_host_batch(const void* src, const uint64_t* boff, const uint32_t* sample_rates, const uint32_t* channels, const uint32_t* formats,
+                                  uint32_t n_tracks, const StratumConfig* cfg, const int32_t* device_ids, uint32_t n_devices, StratumResult* out) {
+    const bool pcm = formats != nullptr;
+    if (!boff || !sample_rates || !out || (!src && n_tracks && boff[n_tracks] > 0) || (pcm && !channels)) {
+        set_error("null argument");
+        return STRATUM_INVALID_INPUT;
+    }
+    StratumConfig def;
+    config_default(&def);
+    const StratumConfig& c = cfg ? *cfg : def;
+    int st = config_validate(c);
+    if (st != STRATUM_OK) return st;
+    if (n_tracks == 0) return STRATUM_OK;
+    std::vector<uint32_t> bpf(n_tracks, 4);  // bytes per mono frame
+    if (pcm && (st = pcm_frame_bytes(boff, channels, formats, n_tracks, bpf)) != STRATUM_OK) return st;
+    return stream_host_batch(src, boff, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
+        return std::unique_ptr<ChunkSink>(new AnalysisSink(ctx, c, boff, bpf, sample_rates, channels, formats, out));
+    });
+}
+
+// ---- loudness (BS.1770-4 / EBU R128; include/stratum_b200.h: StratumLoudness) --------------------------------------------------------
+// K-weighting coefficients at sample rate sr from the analog prototype (libebur128's derivation), in double:
+// k = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2.
+static void kweight_coeffs(uint32_t sr, double* k) {
+    const double fs = (double)sr;
+    {
+        const double f0 = 1681.974450955533, G = 3.999843853973347, Q = 0.7071752369554196;
+        const double K = tan(M_PI * f0 / fs), Vh = pow(10.0, G / 20.0), Vb = pow(Vh, 0.4996667741545416);
+        const double a0 = 1.0 + K / Q + K * K;
+        k[0] = (Vh + Vb * K / Q + K * K) / a0;
+        k[1] = 2.0 * (K * K - Vh) / a0;
+        k[2] = (Vh - Vb * K / Q + K * K) / a0;
+        k[3] = 2.0 * (K * K - 1.0) / a0;
+        k[4] = (1.0 - K / Q + K * K) / a0;
+    }
+    {
+        const double f0 = 38.13547087602444, Q = 0.5003270373238773;
+        const double K = tan(M_PI * f0 / fs), d = 1.0 + K / Q + K * K;
+        k[5] = 1.0;
+        k[6] = -2.0;
+        k[7] = 1.0;
+        k[8] = 2.0 * (K * K - 1.0) / d;
+        k[9] = (1.0 - K / Q + K * K) / d;
+    }
+}
+
+static uint32_t true_peak_factor(uint32_t sr) { return sr < 96000 ? 4 : (sr < 192000 ? 2 : 1); }
+
+// c[j] = sinc((j - 24) / L) * Hann(j / 48); the phase-0 taps are exactly 1 (j = 24) and 0, so the filter interpolates.
+static void true_peak_taps(uint32_t L, float* c) {
+    for (int j = 0; j <= 48; ++j) {
+        const int d = j - 24;
+        double v;
+        if (d % (int)L == 0) v = d == 0 ? 1.0 : 0.0;
+        else {
+            const double t = M_PI * (double)d / (double)L;
+            v = sin(t) / t * 0.5 * (1.0 - cos(2.0 * M_PI * (double)j / 48.0));
+        }
+        c[j] = (float)v;
+    }
+}
+
+// M = A^S: A is the zero-input map of one sample on the state (z1, z2 of stage 1, z1, z2 of stage 2) of k_loudness.cu's cascade.
+static void kweight_power(const double* k, uint32_t S, double* M) {
+    double A[16], R[16], T[16];
+    for (int j = 0; j < 4; ++j) {
+        double s[4] = {0.0, 0.0, 0.0, 0.0};
+        s[j] = 1.0;
+        const double y1 = s[0];
+        const double z1a = -k[3] * y1 + s[1], z2a = -k[4] * y1;
+        const double y2 = k[5] * y1 + s[2];
+        const double z1b = k[6] * y1 - k[8] * y2 + s[3], z2b = k[7] * y1 - k[9] * y2;
+        const double col[4] = {z1a, z2a, z1b, z2b};
+        for (int i = 0; i < 4; ++i) A[4 * i + j] = col[i];
+    }
+    auto mul = [&](const double* X, const double* Y, double* out) {
+        for (int i = 0; i < 4; ++i)
+            for (int j = 0; j < 4; ++j) {
+                double acc = 0.0;
+                for (int q = 0; q < 4; ++q) acc += X[4 * i + q] * Y[4 * q + j];
+                T[4 * i + j] = acc;
+            }
+        memcpy(out, T, sizeof T);
+    };
+    for (int i = 0; i < 16; ++i) R[i] = (i % 5 == 0) ? 1.0 : 0.0;
+    for (uint32_t e = S; e; e >>= 1) {
+        if (e & 1) mul(A, R, R);
+        mul(A, A, A);
+    }
+    memcpy(M, R, sizeof R);
+}
+
+// Per-track failure of the loudness measurement (0 = measured).
+static int loud_track_status(uint32_t sr, uint64_t frames, char* msg, size_t cap) {
+    if (frames == 0 || sr == 0) {
+        snprintf(msg, cap, "%s", frames == 0 ? "empty track: no sample frames" : "sample rate 0");
+        return STRATUM_INVALID_INPUT;
+    }
+    if (sr < 8000 || sr > 384000) {
+        snprintf(msg, cap, "sample rate %u Hz is outside the 8000..384000 Hz range of the loudness measurement", sr);
+        return STRATUM_NOT_IMPLEMENTED;
+    }
+    return STRATUM_OK;
+}
+
+// The loudness of the staged chunks: one launch of each kernel per chunk over all its tracks, straight from the staged PCM.  Chunk
+// k's results are read back while chunk k+1 runs.
+struct LoudnessSink final : ChunkSink {
+    DeviceCtx* ctx;
+    const uint64_t* offsets;
+    const std::vector<uint32_t>& bpf;
+    const uint32_t *sample_rates, *channels, *formats;
+    StratumLoudness* out;
+    struct Slot {
+        uint32_t i = 0, j = 0;
+        bool queued = false;
+        std::vector<PendingStage> stages;
+    } slot[2];
+    size_t rec_bytes = 0, out_bytes = 0;
+    LoudnessSink(DeviceCtx* c, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans, const uint32_t* fmts,
+                 StratumLoudness* o)
+        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o) {}
+
+    // Records of tracks [i, j) (byte offsets relative to track i) into rec (may be null); returns the work items and segments.
+    void plan(uint32_t i, uint32_t j, LoudTrack* rec, uint64_t* n_work, uint64_t* n_seg, uint32_t* max_c) const {
+        uint64_t w = 0, sg = 0;
+        uint32_t mc = 1;
+        char msg[128];
+        for (uint32_t q = i; q < j; ++q) {
+            const uint32_t sr = sample_rates[q], C = channels[q];
+            const uint64_t frames = (offsets[q + 1] - offsets[q]) / bpf[q];
+            const bool ok = loud_track_status(sr, frames, msg, sizeof msg) == STRATUM_OK;
+            const uint32_t S = ok ? (sr + 5) / 10 : 1;
+            const uint32_t nseg = ok ? (uint32_t)((frames + S - 1) / S) : 0, nfull = ok ? (uint32_t)(frames / S) : 0;
+            if (rec) {
+                LoudTrack& T = rec[q - i];
+                memset(&T, 0, sizeof T);
+                T.byte_off = offsets[q] - offsets[i];
+                T.frames = frames;
+                T.work = w;
+                T.seg0 = sg;
+                T.C = C;
+                T.fmt = formats[q];
+                T.S = S;
+                T.nseg = nseg;
+                T.nfull = nfull;
+                T.J = nfull > 3 ? nfull - 3 : 0;
+                T.K = nfull > 29 ? nfull - 29 : 0;
+                if (ok) {
+                    T.L = true_peak_factor(sr);
+                    kweight_coeffs(sr, T.kw);
+                    kweight_power(T.kw, S, T.M);
+                    true_peak_taps(T.L, T.taps);
+                }
+            }
+            w += (uint64_t)nseg * C;
+            sg += nseg;
+            if (ok) mc = std::max(mc, C);
+        }
+        *n_work = w;
+        *n_seg = sg;
+        *max_c = mc;
+    }
+
+    size_t ws_bytes(uint64_t n_tracks, uint64_t n_work, uint64_t n_seg) const {
+        return align_up(n_tracks * sizeof(LoudTrack), 256) + align_up(n_tracks * sizeof(LoudOut), 256) + align_up(5 * n_work * sizeof(double), 256) +
+               align_up(4 * n_seg * sizeof(double), 256);
+    }
+
+    int open(const std::vector<HostChunk>& chunks) override {
+        size_t need = 0, max_n = 0;
+        for (const HostChunk& ch : chunks) {
+            uint64_t w, sg;
+            uint32_t mc;
+            plan(ch.i, ch.j, nullptr, &w, &sg, &mc);
+            need = std::max(need, ws_bytes(ch.j - ch.i, w, sg));
+            max_n = std::max<size_t>(max_n, ch.j - ch.i);
+        }
+        rec_bytes = max_n * sizeof(LoudTrack);
+        out_bytes = max_n * sizeof(LoudOut);
+        for (int b = 0; b < 2; ++b)
+            if (!ctx->loud_rec[b].need(rec_bytes) || !ctx->loud_out[b].need(out_bytes)) {
+                set_error("pinned host allocation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
+        if (!grow_device(ctx->d_loud, ctx->loud_cap, need)) {
+            set_error("loudness work area allocation failed");
+            return STRATUM_PROCESSING_ERROR;
+        }
+        for (cudaEvent_t& e : ctx->loud_ev)
+            if (!e && cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) {
+                set_error("event creation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
+        return STRATUM_OK;
+    }
+
+    int chunk(size_t k, const HostChunk& ch, const char* d_buf, const std::function<void()>& after_prev) override {
+        const uint32_t n = ch.j - ch.i;
+        LoudTrack* h_tr = static_cast<LoudTrack*>(ctx->loud_rec[k & 1].p);
+        LoudOut* h_out = static_cast<LoudOut*>(ctx->loud_out[k & 1].p);
+        uint64_t n_work, n_seg;
+        uint32_t max_c;
+        plan(ch.i, ch.j, h_tr, &n_work, &n_seg, &max_c);
+        char* d = ctx->d_loud;
+        LoudTrack* d_tr = reinterpret_cast<LoudTrack*>(d);
+        d += align_up((uint64_t)n * sizeof(LoudTrack), 256);
+        LoudOut* d_out = reinterpret_cast<LoudOut*>(d);
+        d += align_up((uint64_t)n * sizeof(LoudOut), 256);
+        double* d_st = reinterpret_cast<double*>(d);
+        double* d_en = d_st + 4 * n_work;
+        d += align_up(5 * n_work * sizeof(double), 256);
+        double* d_ws = reinterpret_cast<double*>(d);
+        cudaStream_t s = ctx->stream;
+        CUDA_OK(cudaMemcpyAsync(d_tr, h_tr, (size_t)n * sizeof(LoudTrack), cudaMemcpyHostToDevice, s));
+        CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(LoudOut), s));
+        g_h2d_bytes.fetch_add((uint64_t)n * sizeof(LoudTrack));
+        {
+            StageTimer tm(s, "loudness_pass1");
+            launch_loud_pass1(s, d_buf, d_tr, n, n_work, d_st);
+        }
+        {
+            StageTimer tm(s, "loudness_scan");
+            launch_loud_scan(s, d_tr, n, max_c, d_st);
+        }
+        {
+            StageTimer tm(s, "loudness_pass2");
+            launch_loud_pass2(s, d_buf, d_tr, n, n_work, d_st, d_en, d_out);
+        }
+        {
+            StageTimer tm(s, "loudness_gate");
+            launch_loud_gate(s, d_tr, n, d_en, d_ws, n_seg, d_out);
+        }
+        CUDA_OK(cudaGetLastError());
+        CUDA_OK(cudaMemcpyAsync(h_out, d_out, (size_t)n * sizeof(LoudOut), cudaMemcpyDeviceToHost, s));
+        g_d2h_bytes.fetch_add((uint64_t)n * sizeof(LoudOut));
+        CUDA_OK(cudaEventRecord(ctx->loud_ev[k & 1], s));
+        Slot& cur = slot[k & 1];
+        cur.i = ch.i;
+        cur.j = ch.j;
+        cur.queued = true;
+        cur.stages.swap(g_pending);
+        g_pending.clear();
+        const int st = gather((k + 1) & 1);  // the previous chunk: its staging buffer is free once it has finished
+        after_prev();
+        return st;
+    }
+
+    int gather(int b) {
+        Slot& sl = slot[b];
+        if (!sl.queued) return STRATUM_OK;
+        sl.queued = false;
+        CUDA_OK(cudaEventSynchronize(ctx->loud_ev[b]));
+        resolve_stage_times(sl.stages);
+        const LoudTrack* h_tr = static_cast<const LoudTrack*>(ctx->loud_rec[b].p);
+        const LoudOut* h_out = static_cast<const LoudOut*>(ctx->loud_out[b].p);
+        for (uint32_t q = sl.i; q < sl.j; ++q) {
+            const LoudTrack& T = h_tr[q - sl.i];
+            const LoudOut& o = h_out[q - sl.i];
+            StratumLoudness& r = out[q];
+            memset(&r, 0, sizeof r);
+            r.sample_rate = sample_rates[q];
+            r.channels = channels[q];
+            r.frames = T.frames;
+            r.status = loud_track_status(r.sample_rate, r.frames, r.error, sizeof r.error);
+            if (r.status != STRATUM_OK) continue;
+            r.integrated_lufs = o.integrated;
+            r.momentary_max_lufs = o.momentary_max;
+            r.short_term_max_lufs = o.short_term_max;
+            r.loudness_range_lu = o.loudness_range;
+            float f;
+            memcpy(&f, &o.sample_peak_bits, sizeof f);
+            r.sample_peak = f;
+            memcpy(&f, &o.true_peak_bits, sizeof f);
+            r.true_peak = f;
+            r.n_momentary = T.J;
+            r.n_short_term = T.K;
+        }
+        return STRATUM_OK;
+    }
+
+    int close() override {
+        const int s1 = gather(0), s2 = gather(1);
+        return s1 != STRATUM_OK ? s1 : s2;
+    }
+};
+
+static int32_t loudness_validate(const uint64_t* boff, const uint32_t* sample_rates, const uint32_t* channels, const uint32_t* formats, uint32_t n_tracks,
+                                 StratumLoudness* out, bool have_pcm, std::vector<uint32_t>& bpf) {
+    if (!boff || !sample_rates || !channels || !formats || !out || (!have_pcm && n_tracks && boff[n_tracks] > boff[0])) {
+        set_error("null argument");
+        return STRATUM_INVALID_INPUT;
+    }
+    bpf.assign(n_tracks, 1);
+    return pcm_frame_bytes(boff, channels, formats, n_tracks, bpf);
+}
+
+int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                        const uint32_t* formats, uint32_t n_tracks, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out) {
+    std::vector<uint32_t> bpf;
+    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, pcm != nullptr, bpf);
+    if (st != STRATUM_OK || n_tracks == 0) return st;
+    return stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
+        return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out));
+    });
+}
+
+int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                               const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out) {
+    std::vector<uint32_t> bpf;
+    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, d_pcm != nullptr, bpf);
+    if (st != STRATUM_OK || n_tracks == 0) return st;
+    DeviceCtx* ctx = get_ctx(device_id, &st);
+    if (!ctx) return st;
+    std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+    if (cudaSetDevice(ctx->device) != cudaSuccess) {
+        set_error("cudaSetDevice failed");
+        return STRATUM_PROCESSING_ERROR;
+    }
+    // the whole batch is one chunk: one launch of each kernel
+    const std::vector<HostChunk> one{HostChunk{0, n_tracks, byte_offsets[n_tracks] - byte_offsets[0], 0}};
+    LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out);
+    st = sink.open(one);
+    if (st != STRATUM_OK) return st;
+    const int s1 = sink.chunk(0, one[0], static_cast<const char*>(d_pcm) + byte_offsets[0], [] {});
+    const int s2 = sink.close();
+    return s1 != STRATUM_OK ? s1 : s2;
+}
+
+int32_t stratum_b200_debug_loudness_filters(uint32_t sample_rate, double* kweight10, float* taps49) {
+    char msg[128];
+    if (loud_track_status(sample_rate, 1, msg, sizeof msg) != STRATUM_OK) return -1;
+    const uint32_t L = true_peak_factor(sample_rate);
+    if (kweight10) kweight_coeffs(sample_rate, kweight10);
+    if (taps49) true_peak_taps(L, taps49);
+    return (int32_t)L;
 }
 
 void stratum_b200_debug_mel_schedule(const int32_t* mel_off, uint32_t n_mels, int32_t* schedule256) {
@@ -2543,6 +2930,7 @@ void stratum_b200_shutdown(void) {
             cudaFree(c->d_stage);
             cudaFree(c->d_conv);
             cudaFree(c->d_meta);
+            cudaFree(c->d_loud);
             cudaFree(c->d_count);
             c->uploader.reset();
             for (WaveJob& j : c->jobs) {
@@ -2555,6 +2943,11 @@ void stratum_b200_shutdown(void) {
             }
             c->h_meta[0].release();
             c->h_meta[1].release();
+            for (int b = 0; b < 2; ++b) {
+                c->loud_rec[b].release();
+                c->loud_out[b].release();
+                if (c->loud_ev[b]) cudaEventDestroy(c->loud_ev[b]);
+            }
             c->h_count.release();
             if (c->ev_legacy) cudaEventDestroy(c->ev_legacy);
             if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
@@ -2571,6 +2964,7 @@ size_t stratum_b200_sizeof(int32_t which) {
         case 0: return sizeof(StratumConfig);
         case 1: return sizeof(StratumResult);
         case 2: return sizeof(StratumConfidence);
+        case 3: return sizeof(StratumLoudness);
         default: return 0;
     }
 }

@@ -182,16 +182,34 @@ __device__ inline int block_topk(F val, int lo, int hi, int* out_idx, float* sva
     return cnt;
 }
 
-// Exact k-th smallest (0-based) of n non-negative floats: 4-pass MSB radix select on the bit
-// patterns (order-preserving for x >= 0).  All threads of the block call it; result broadcast.
-__device__ inline float block_select_kth(const float* __restrict__ v, uint32_t n, uint32_t k, uint32_t* hist /* 256 */, uint32_t* bcast /* 2 */) {
-    uint32_t prefix = 0, mask = 0;
-    for (int shift = 24; shift >= 0; shift -= 8) {
+template <class T>
+struct SelectBits;
+template <>
+struct SelectBits<float> {
+    using U = uint32_t;
+    static __device__ __forceinline__ U bits(float x) { return __float_as_uint(x); }
+    static __device__ __forceinline__ float value(U b) { return __uint_as_float(b); }
+};
+template <>
+struct SelectBits<double> {
+    using U = unsigned long long;
+    static __device__ __forceinline__ U bits(double x) { return (U)__double_as_longlong(x); }
+    static __device__ __forceinline__ double value(U b) { return __longlong_as_double((long long)b); }
+};
+
+// Exact k-th smallest (0-based) of n non-negative floats or doubles: MSB radix select on the bit patterns, 8 bits per
+// pass (order-preserving for x >= 0).  All threads of the block call it; result broadcast.
+template <class T>
+__device__ inline T block_select_kth(const T* __restrict__ v, uint32_t n, uint32_t k, uint32_t* hist /* 256 */, uint32_t* bcast /* 2 */) {
+    using B = SelectBits<T>;
+    using U = typename B::U;
+    U prefix = 0, mask = 0;
+    for (int shift = 8 * (int)sizeof(U) - 8; shift >= 0; shift -= 8) {
         for (uint32_t i = threadIdx.x; i < 256; i += blockDim.x) hist[i] = 0;
         __syncthreads();
         for (uint32_t i = threadIdx.x; i < n; i += blockDim.x) {
-            uint32_t b = __float_as_uint(v[i]);
-            if ((b & mask) == prefix) atomicAdd(&hist[(b >> shift) & 255u], 1u);
+            const U b = B::bits(v[i]);
+            if ((b & mask) == prefix) atomicAdd(&hist[(uint32_t)(b >> shift) & 255u], 1u);
         }
         __syncthreads();
         if (threadIdx.x == 0) {
@@ -204,12 +222,12 @@ __device__ inline float block_select_kth(const float* __restrict__ v, uint32_t n
             bcast[1] = k - acc;
         }
         __syncthreads();
-        prefix |= bcast[0] << shift;
-        mask |= 255u << shift;
+        prefix |= (U)bcast[0] << shift;
+        mask |= (U)255u << shift;
         k = bcast[1];
         __syncthreads();
     }
-    return __uint_as_float(prefix);
+    return B::value(prefix);
 }
 
 }  // namespace sb

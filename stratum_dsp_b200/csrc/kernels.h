@@ -202,6 +202,39 @@ void launch_key_hpcp(const WaveCtx& c);
 void launch_key_vote(const WaveCtx& c);
 void launch_key_variants_pre(const WaveCtx& c);  // k_keyvar.cu: median-HPSS mask, tuning estimate, whitening, per-track fold tables
 void launch_key_chroma_variants(const WaveCtx& c);  // k_keyvar.cu: log-frequency chroma, beat-synchronous chroma
+// k_loudness.cu: BS.1770-4 / EBU R128 loudness of interleaved PCM (stratum_b200_loudness_batch_pcm).
+// One record per track of a launch, built on the host (engine.cu: loud_track).
+struct LoudTrack {
+    uint64_t byte_off;     // first byte of the track in the launch's PCM buffer
+    uint64_t frames;
+    uint64_t work;         // first work item (segment-major (segment, channel) pairs of the earlier tracks)
+    uint64_t seg0;         // first entry in the per-segment work areas (segments of the earlier tracks)
+    uint32_t C, fmt;       // channels, STRATUM_PCM_*
+    uint32_t S, L;         // sub-block frames (sr + 5) / 10, true-peak oversampling factor
+    uint32_t nseg, nfull;  // segments covering the track (0: the track failed and is skipped), whole sub-blocks floor(frames / S)
+    uint32_t J, K;         // momentary blocks max(0, nfull - 3), short-term windows max(0, nfull - 29)
+    double kw[10];         // K-weighting: stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2
+    double M[16];          // A^S, row-major: maps the cascade state (z1, z2 of stage 1, z1, z2 of stage 2) across one silent sub-block
+    float taps[49];        // true-peak interpolator
+};
+struct LoudOut {
+    double integrated, momentary_max, short_term_max, loudness_range;
+    uint32_t sample_peak_bits, true_peak_bits;  // non-negative floats, reduced by atomicMax on the bits
+};
+// libebur128's default channel map: 1 channel L; 4 channels L R Ls Rs; 5 channels L R C Ls Rs; otherwise L R C LFE Ls Rs and unused
+// channels from 6 on.  L, R, C weigh 1, Ls and Rs 1.41, LFE and unused channels 0.
+__host__ __device__ inline double loud_channel_weight(uint32_t C, uint32_t c) {
+    if (C == 4) return c < 2 ? 1.0 : 1.41;
+    if (C == 5) return c < 3 ? 1.0 : 1.41;
+    if (c < 3) return 1.0;
+    return (c == 4 || c == 5) ? 1.41 : 0.0;
+}
+void launch_loud_pass1(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, double* d_st);
+void launch_loud_scan(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, uint32_t max_channels, double* d_st);
+void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, const double* d_st, double* d_en,
+                       LoudOut* d_out);
+// d_ws: 4 x n_seg doubles (sub-block, momentary and short-term powers, the compacted short-term powers of the loudness range)
+void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_en, double* d_ws, uint64_t n_seg, LoudOut* d_out);
 // k_synth.cu
 void launch_pcm_to_mono(cudaStream_t s, const void* d_pcm, float* d_out, const uint64_t* d_byte_off, const uint64_t* d_out_off, const uint32_t* d_channels,
                         const uint32_t* d_formats, uint32_t n_tracks, uint64_t max_frames);
