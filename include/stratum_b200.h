@@ -261,6 +261,34 @@ int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_of
 /* Same, with the PCM already resident in the memory of device `device_id`. */
 int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out);
+
+/* Album loudness (ReplayGain 2.0 / R128 album values): track i belongs to album album_of_track[i] < n_albums, or to none
+ * (STRATUM_NO_ALBUM).  An album's pooled momentary list is the concatenation of its members' momentary powers (the blocks defined
+ * above, each member at its own sample rate, channel count and format), members in ascending track index; its pooled short-term list
+ * likewise.
+ *  - integrated_lufs: the per-track rule on the pooled momentary list: absolute gate -70 LUFS, relative gate 10 LU below the
+ *    loudness of the mean power of the blocks above -70, loudness of the mean power of the blocks above both gates.  A quiet track
+ *    can fall under the album's relative gate although it passes its own.
+ *  - momentary_max_lufs / short_term_max_lufs: maxima over the pooled lists (-INFINITY for an empty list).
+ *  - loudness_range_lu: the per-track range rule on the pooled short-term list.
+ *  - sample_peak / true_peak: maxima over the members.  n_momentary / n_short_term: the pooled counts.  frames: the sum over the
+ *    members.  sample_rate, channels: 0.
+ * An album of one track has that track's values bit for bit, and album values depend only on the members' samples: not on the
+ * other tracks, the order of the albums, the upload chunks, the devices or the entry.
+ * Album status: STRATUM_OK when every member is measured; otherwise the status of the lowest-index failed member, the error
+ * "track <i>: <member's message>" and no values (no album value over a partial album).  An id no track names: STRATUM_INVALID_INPUT,
+ * "album has no tracks".  Neither case touches other albums or any track result.
+ * Rejected whole (STRATUM_INVALID_INPUT, before any device work), besides what the per-track entries reject: an id at or above
+ * n_albums other than STRATUM_NO_ALBUM; a NULL album_of_track or album_out while n_albums > 0.  album_of_track may be NULL when
+ * n_albums = 0, which is stratum_b200_loudness_batch_pcm.  out[i] is the per-track result of stratum_b200_loudness_batch_pcm. */
+#define STRATUM_NO_ALBUM 0xFFFFFFFFu
+int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out, StratumLoudness* album_out);
+/* Same, with the PCM already resident in the memory of device `device_id`. */
+int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                int32_t device_id, StratumLoudness* out, StratumLoudness* album_out);
 /* Host-side filters of the loudness measurement (no device work): kweight10 = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2 (either
  * may be NULL), taps49 = the true-peak interpolator as the device uses it (f32).  Returns the oversampling factor L, or -1 for a
  * sample rate outside 8000..384000 Hz. */

@@ -212,11 +212,29 @@ pub struct Loudness {
 /// Loudness of a batch of PCM tracks, measured on the device and sharded over `devices` (empty: the current device).  The outer
 /// error rejects the whole call (no device, malformed input); a track that fails on its own carries its error in its slot.
 pub fn loudness_batch_pcm(tracks: &[PcmTrack], devices: &[i32]) -> Result<Vec<Result<Loudness, AnalysisError>>, AnalysisError> {
+    loudness_albums_pcm(tracks, &vec![None; tracks.len()], devices).map(|(per_track, _)| per_track)
+}
+
+/// Per-track loudness plus the loudness of albums (ReplayGain / R128 album values): `albums[i]` is the album of track i (`None`: no
+/// album), ids from 0; there are max id + 1 albums.  Each album is measured over the pooled 400 ms blocks and 3 s windows of its
+/// members, so its integrated loudness and range are not functions of the track values.  An album with a failed member, or an id no
+/// track names, carries its error in its slot.
+pub fn loudness_albums_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], devices: &[i32])
+    -> Result<(Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>), AnalysisError> {
     let ok = unsafe { stratum_b200_sizeof(3) == std::mem::size_of::<StratumLoudness>() };
     if !ok {
         return Err(AnalysisError::ProcessingError("libstratum_b200.so does not match this binding (struct sizes differ)".to_string()));
     }
+    if albums.len() != tracks.len() {
+        return Err(AnalysisError::InvalidInput("one album id (or None) per track".to_string()));
+    }
     let n = tracks.len();
+    let ids: Vec<u32> = albums.iter().map(|a| a.unwrap_or(STRATUM_NO_ALBUM)).collect();
+    let n_albums = albums.iter().flatten().map(|a| *a as u64 + 1).max().unwrap_or(0);
+    if n_albums > u32::MAX as u64 {
+        return Err(AnalysisError::InvalidInput("album id STRATUM_NO_ALBUM is reserved for None".to_string()));
+    }
+    let n_albums = n_albums as usize;
     let mut offsets = vec![0u64];
     let mut flat: Vec<u8> = Vec::new();
     for t in tracks {
@@ -227,31 +245,31 @@ pub fn loudness_batch_pcm(tracks: &[PcmTrack], devices: &[i32]) -> Result<Vec<Re
     let chans: Vec<u32> = tracks.iter().map(|t| t.channels).collect();
     let fmts: Vec<u32> = tracks.iter().map(|t| t.format).collect();
     let mut res: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
+    let mut alb: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n_albums];
     let st = unsafe {
-        stratum_b200_loudness_batch_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32,
-                                        if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32, res.as_mut_ptr())
+        stratum_b200_loudness_albums_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, ids.as_ptr(),
+                                         n_albums as u32, if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
+                                         res.as_mut_ptr(), alb.as_mut_ptr())
     };
     if st != 0 {
         return Err(to_error(st, last_error()));
     }
-    Ok(res
-        .iter()
-        .map(|r| {
-            if r.status != 0 {
-                return Err(to_error(r.status, c_string(&r.error)));
-            }
-            Ok(Loudness {
-                integrated_lufs: r.integrated_lufs,
-                momentary_max_lufs: r.momentary_max_lufs,
-                short_term_max_lufs: r.short_term_max_lufs,
-                loudness_range_lu: r.loudness_range_lu,
-                sample_peak: r.sample_peak,
-                true_peak: r.true_peak,
-                n_momentary: r.n_momentary,
-                n_short_term: r.n_short_term,
-            })
+    let convert = |r: &StratumLoudness| {
+        if r.status != 0 {
+            return Err(to_error(r.status, c_string(&r.error)));
+        }
+        Ok(Loudness {
+            integrated_lufs: r.integrated_lufs,
+            momentary_max_lufs: r.momentary_max_lufs,
+            short_term_max_lufs: r.short_term_max_lufs,
+            loudness_range_lu: r.loudness_range_lu,
+            sample_peak: r.sample_peak,
+            true_peak: r.true_peak,
+            n_momentary: r.n_momentary,
+            n_short_term: r.n_short_term,
         })
-        .collect())
+    };
+    Ok((res.iter().map(convert).collect(), alb.iter().map(convert).collect()))
 }
 
 /// Decoder-side batch entry: interleaved 16-bit PCM uploaded as is and converted on the device with the arithmetic of

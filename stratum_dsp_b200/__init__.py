@@ -206,6 +206,10 @@ def lib() -> C.CDLL:
     L.stratum_b200_loudness_batch_pcm.restype = _i
     L.stratum_b200_loudness_batch_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, _i, loudp]
     L.stratum_b200_loudness_batch_pcm_device.restype = _i
+    L.stratum_b200_loudness_albums_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, i32p, _u, loudp, loudp]
+    L.stratum_b200_loudness_albums_pcm.restype = _i
+    L.stratum_b200_loudness_albums_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, _i, loudp, loudp]
+    L.stratum_b200_loudness_albums_pcm_device.restype = _i
     L.stratum_b200_debug_loudness_filters.argtypes = [_u, C.POINTER(C.c_double), f32p]
     L.stratum_b200_debug_loudness_filters.restype = _i
     if L.stratum_b200_sizeof(0) != C.sizeof(StratumConfig) or L.stratum_b200_sizeof(1) != C.sizeof(StratumResult) or \
@@ -585,7 +589,7 @@ def analyze_batch_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None 
 
 @dataclass
 class Loudness:
-    """ITU-R BS.1770-4 / EBU R128 loudness of one track (include/stratum_b200.h: StratumLoudness).  Loudness values are in LUFS,
+    """ITU-R BS.1770-4 / EBU R128 loudness of one track or album (include/stratum_b200.h: StratumLoudness).  Loudness values are in LUFS,
     the range in LU, peaks linear (full scale 1.0); undefined loudness values are ``float("-inf")``."""
 
     integrated_lufs: float
@@ -654,6 +658,64 @@ def loudness_batch_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_r
     if st != OK:
         _raise(st)
     return [_loudness(res[i]) for i in range(n)]
+
+
+NO_ALBUM = 0xFFFFFFFF  # STRATUM_NO_ALBUM
+
+
+def _album_ids(albums: Sequence[int | None], n_tracks: int, n_albums: int | None):
+    if len(albums) != n_tracks:
+        raise ValueError("one album id (or None) per track")
+    if any(a is not None and (int(a) < 0 or int(a) >= NO_ALBUM) for a in albums):
+        raise ValueError("album ids are non-negative integers below 0xFFFFFFFF, or None")
+    ids = np.ascontiguousarray([NO_ALBUM if a is None else int(a) for a in albums], dtype=np.uint32).reshape(-1)
+    if n_albums is None:
+        n_albums = max((int(a) + 1 for a in albums if a is not None), default=0)
+    return ids, int(n_albums)
+
+
+def loudness_albums_pcm(tracks: Sequence[PcmTrack], albums: Sequence[int | None], n_albums: int | None = None,
+                        devices: Sequence[int] | None = None) -> tuple:
+    """stratum_b200_loudness_albums_pcm: the per-track results of ``loudness_batch_pcm`` and the loudness of albums (ReplayGain /
+    R128 album values), each measured over the pooled 400 ms blocks and 3 s windows of its members.  ``albums[i]`` is the album id of
+    track i (``None``: no album); ``n_albums`` defaults to the largest id + 1.  Returns ``(tracks, albums)``, two lists of
+    ``Loudness``; an album with a failed member, or one that no track names, carries ``.error``."""
+    n = len(tracks)
+    ids, na = _album_ids(albums, n, n_albums)
+    flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
+    cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
+    offsets, srs, chans, fmts = _pcm_tables(tracks)
+    res = (StratumLoudness * max(n, 1))()
+    alb = (StratumLoudness * max(na, 1))()
+    dev = (C.c_int32 * len(devices))(*devices) if devices else None
+    st = lib().stratum_b200_loudness_albums_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
+                                                n, ids.ctypes.data_as(C.POINTER(_u)), na, dev, len(devices) if devices else 0, res, alb)
+    if st != OK:
+        _raise(st)
+    return [_loudness(res[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
+
+
+def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
+                               albums: Sequence[int | None], n_albums: int | None = None, device: int = -1) -> tuple:
+    """stratum_b200_loudness_albums_pcm_device: ``loudness_albums_pcm`` with the PCM already in device memory (arguments as
+    ``loudness_batch_pcm_device``)."""
+    offsets = np.ascontiguousarray(byte_offsets, dtype=np.uint64)
+    n = offsets.size - 1
+    srs = np.ascontiguousarray(sample_rates, dtype=np.uint32)
+    chans = np.ascontiguousarray(channels, dtype=np.uint32)
+    fmts = np.ascontiguousarray(formats, dtype=np.uint32)
+    if not (srs.size == chans.size == fmts.size == n):
+        raise ValueError("one sample rate, channel count and format per track")
+    ids, na = _album_ids(albums, n, n_albums)
+    res = (StratumLoudness * max(n, 1))()
+    alb = (StratumLoudness * max(na, 1))()
+    st = lib().stratum_b200_loudness_albums_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                       srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)),
+                                                       fmts.ctypes.data_as(C.POINTER(_u)), n, ids.ctypes.data_as(C.POINTER(_u)), na, device, res, alb)
+    if st != OK:
+        _raise(st)
+    return [_loudness(res[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_filters(sample_rate: int) -> tuple:

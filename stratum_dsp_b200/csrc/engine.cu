@@ -258,6 +258,9 @@ struct DeviceCtx {
     char* d_loud = nullptr;   // loudness work area of one chunk (track records, results, cascade states, energies, per-segment powers)
     size_t loud_cap = 0;
     PinnedBuf loud_rec[2], loud_out[2];  // pinned track records / results of two chunks (chunk k+1 is queued before chunk k is read)
+    PinnedBuf loud_blk[2];    // momentary and short-term powers of the same two chunks (calls with albums only)
+    char* d_album = nullptr;  // album phase: album records, pooled powers, selection scratch, results
+    size_t album_cap = 0;
     cudaEvent_t loud_ev[2] = {nullptr, nullptr};
     int32_t* d_count = nullptr;  // escalated tracks of the wave being queued (escalation_compact_kernel)
     PinnedBuf h_count;
@@ -2482,6 +2485,76 @@ static int loud_track_status(uint32_t sr, uint64_t frames, char* msg, size_t cap
     return STRATUM_OK;
 }
 
+// Sub-block frames S, segments covering the track, whole sub-blocks, momentary blocks J and short-term windows K of one track
+// (all counts 0 for a track that fails).
+struct LoudGeom {
+    bool ok;
+    uint32_t S, nseg, nfull, J, K;
+};
+static LoudGeom loud_geom(uint32_t sr, uint64_t frames) {
+    char msg[128];
+    LoudGeom g;
+    g.ok = loud_track_status(sr, frames, msg, sizeof msg) == STRATUM_OK;
+    g.S = g.ok ? (sr + 5) / 10 : 1;
+    g.nseg = g.ok ? (uint32_t)((frames + g.S - 1) / g.S) : 0;
+    g.nfull = g.ok ? (uint32_t)(frames / g.S) : 0;
+    g.J = g.nfull > 3 ? g.nfull - 3 : 0;
+    g.K = g.nfull > 29 ? g.nfull - 29 : 0;
+    return g;
+}
+
+// The host pools of the albums of one call: one buffer holding the album records, then every album's momentary powers, then every
+// album's short-term powers; albums one after the other, members in ascending track index.  Member q's powers go to
+// buf[m_at[q] ..) and buf[q_at[q] ..); the shards of a host batch fill disjoint ranges.
+struct AlbumPools {
+    const uint32_t* album_of = nullptr;
+    uint32_t n_albums = 0;
+    std::vector<uint64_t> m_at, q_at;
+    uint64_t mom0 = 0, sht0 = 0, n_mom = 0, n_sht = 0;  // buf offsets of the two pools and their lengths, in doubles
+    std::vector<double> buf;
+    LoudAlbum* albums() { return reinterpret_cast<LoudAlbum*>(buf.data()); }
+    bool member(uint32_t q) const { return album_of && album_of[q] < n_albums; }
+};
+
+static void album_layout(const uint32_t* album_of, uint32_t n_albums, const uint64_t* offsets, const std::vector<uint32_t>& bpf,
+                         const uint32_t* sample_rates, uint32_t n_tracks, AlbumPools& P) {
+    P.album_of = album_of;
+    P.n_albums = n_albums;
+    if (n_albums == 0) return;
+    std::vector<LoudAlbum> al(n_albums, LoudAlbum{0, 0, 0, 0});
+    std::vector<LoudGeom> g(n_tracks);
+    for (uint32_t q = 0; q < n_tracks; ++q) {
+        if (!P.member(q)) continue;
+        g[q] = loud_geom(sample_rates[q], (offsets[q + 1] - offsets[q]) / bpf[q]);
+        al[album_of[q]].J += g[q].J;
+        al[album_of[q]].K += g[q].K;
+    }
+    for (LoudAlbum& a : al) {
+        a.m0 = P.n_mom;
+        a.q0 = P.n_sht;
+        P.n_mom += a.J;
+        P.n_sht += a.K;
+    }
+    P.mom0 = (n_albums * sizeof(LoudAlbum) + sizeof(double) - 1) / sizeof(double);
+    P.sht0 = P.mom0 + P.n_mom;
+    P.buf.assign(P.sht0 + P.n_sht, 0.0);
+    memcpy(P.buf.data(), al.data(), n_albums * sizeof(LoudAlbum));
+    P.m_at.assign(n_tracks, 0);
+    P.q_at.assign(n_tracks, 0);
+    std::vector<uint64_t> mf(n_albums), qf(n_albums);
+    for (uint32_t a = 0; a < n_albums; ++a) {
+        mf[a] = P.mom0 + al[a].m0;
+        qf[a] = P.sht0 + al[a].q0;
+    }
+    for (uint32_t q = 0; q < n_tracks; ++q) {
+        if (!P.member(q)) continue;
+        P.m_at[q] = mf[album_of[q]];
+        P.q_at[q] = qf[album_of[q]];
+        mf[album_of[q]] += g[q].J;
+        qf[album_of[q]] += g[q].K;
+    }
+}
+
 // The loudness of the staged chunks: one launch of each kernel per chunk over all its tracks, straight from the staged PCM.  Chunk
 // k's results are read back while chunk k+1 runs.
 struct LoudnessSink final : ChunkSink {
@@ -2490,27 +2563,33 @@ struct LoudnessSink final : ChunkSink {
     const std::vector<uint32_t>& bpf;
     const uint32_t *sample_rates, *channels, *formats;
     StratumLoudness* out;
+    AlbumPools* pools;  // null without albums
     struct Slot {
         uint32_t i = 0, j = 0;
-        bool queued = false;
+        bool queued = false, blocks = false;  // blocks: the chunk's momentary / short-term powers were read back
+        uint64_t n_seg = 0;
         std::vector<PendingStage> stages;
     } slot[2];
     size_t rec_bytes = 0, out_bytes = 0;
     LoudnessSink(DeviceCtx* c, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans, const uint32_t* fmts,
-                 StratumLoudness* o)
-        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o) {}
+                 StratumLoudness* o, AlbumPools* p)
+        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p) {}
+    bool has_member(uint32_t i, uint32_t j) const {
+        for (uint32_t q = i; pools && q < j; ++q)
+            if (pools->member(q)) return true;
+        return false;
+    }
 
     // Records of tracks [i, j) (byte offsets relative to track i) into rec (may be null); returns the work items and segments.
     void plan(uint32_t i, uint32_t j, LoudTrack* rec, uint64_t* n_work, uint64_t* n_seg, uint32_t* max_c) const {
         uint64_t w = 0, sg = 0;
         uint32_t mc = 1;
-        char msg[128];
         for (uint32_t q = i; q < j; ++q) {
             const uint32_t sr = sample_rates[q], C = channels[q];
             const uint64_t frames = (offsets[q + 1] - offsets[q]) / bpf[q];
-            const bool ok = loud_track_status(sr, frames, msg, sizeof msg) == STRATUM_OK;
-            const uint32_t S = ok ? (sr + 5) / 10 : 1;
-            const uint32_t nseg = ok ? (uint32_t)((frames + S - 1) / S) : 0, nfull = ok ? (uint32_t)(frames / S) : 0;
+            const LoudGeom g = loud_geom(sr, frames);
+            const bool ok = g.ok;
+            const uint32_t S = g.S, nseg = g.nseg, nfull = g.nfull;
             if (rec) {
                 LoudTrack& T = rec[q - i];
                 memset(&T, 0, sizeof T);
@@ -2523,8 +2602,8 @@ struct LoudnessSink final : ChunkSink {
                 T.S = S;
                 T.nseg = nseg;
                 T.nfull = nfull;
-                T.J = nfull > 3 ? nfull - 3 : 0;
-                T.K = nfull > 29 ? nfull - 29 : 0;
+                T.J = g.J;
+                T.K = g.K;
                 if (ok) {
                     T.L = true_peak_factor(sr);
                     kweight_coeffs(sr, T.kw);
@@ -2547,14 +2626,20 @@ struct LoudnessSink final : ChunkSink {
     }
 
     int open(const std::vector<HostChunk>& chunks) override {
-        size_t need = 0, max_n = 0;
+        size_t need = 0, max_n = 0, blk_bytes = 0;
         for (const HostChunk& ch : chunks) {
             uint64_t w, sg;
             uint32_t mc;
             plan(ch.i, ch.j, nullptr, &w, &sg, &mc);
             need = std::max(need, ws_bytes(ch.j - ch.i, w, sg));
             max_n = std::max<size_t>(max_n, ch.j - ch.i);
+            if (has_member(ch.i, ch.j)) blk_bytes = std::max<size_t>(blk_bytes, 2 * sg * sizeof(double));
         }
+        for (int b = 0; b < 2 && blk_bytes; ++b)
+            if (!ctx->loud_blk[b].need(blk_bytes)) {
+                set_error("pinned host allocation failed");
+                return STRATUM_PROCESSING_ERROR;
+            }
         rec_bytes = max_n * sizeof(LoudTrack);
         out_bytes = max_n * sizeof(LoudOut);
         for (int b = 0; b < 2; ++b)
@@ -2613,11 +2698,18 @@ struct LoudnessSink final : ChunkSink {
         CUDA_OK(cudaGetLastError());
         CUDA_OK(cudaMemcpyAsync(h_out, d_out, (size_t)n * sizeof(LoudOut), cudaMemcpyDeviceToHost, s));
         g_d2h_bytes.fetch_add((uint64_t)n * sizeof(LoudOut));
+        const bool blocks = has_member(ch.i, ch.j);
+        if (blocks) {  // the momentary and short-term regions of the work area are adjacent: one copy for both
+            CUDA_OK(cudaMemcpyAsync(ctx->loud_blk[k & 1].p, d_ws + n_seg, 2 * n_seg * sizeof(double), cudaMemcpyDeviceToHost, s));
+            g_d2h_bytes.fetch_add(2 * n_seg * sizeof(double));
+        }
         CUDA_OK(cudaEventRecord(ctx->loud_ev[k & 1], s));
         Slot& cur = slot[k & 1];
         cur.i = ch.i;
         cur.j = ch.j;
         cur.queued = true;
+        cur.blocks = blocks;
+        cur.n_seg = n_seg;
         cur.stages.swap(g_pending);
         g_pending.clear();
         const int st = gather((k + 1) & 1);  // the previous chunk: its staging buffer is free once it has finished
@@ -2654,6 +2746,11 @@ struct LoudnessSink final : ChunkSink {
             r.true_peak = f;
             r.n_momentary = T.J;
             r.n_short_term = T.K;
+            if (sl.blocks && pools->member(q)) {
+                const double* blk = static_cast<const double*>(ctx->loud_blk[b].p);
+                memcpy(pools->buf.data() + pools->m_at[q], blk + T.seg0, (size_t)T.J * sizeof(double));
+                memcpy(pools->buf.data() + pools->q_at[q], blk + sl.n_seg + T.seg0, (size_t)T.K * sizeof(double));
+            }
         }
         return STRATUM_OK;
     }
@@ -2674,36 +2771,154 @@ static int32_t loudness_validate(const uint64_t* boff, const uint32_t* sample_ra
     return pcm_frame_bytes(boff, channels, formats, n_tracks, bpf);
 }
 
-int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
-                                        const uint32_t* formats, uint32_t n_tracks, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out) {
-    std::vector<uint32_t> bpf;
-    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, pcm != nullptr, bpf);
-    if (st != STRATUM_OK || n_tracks == 0) return st;
-    return stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
-        return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out));
-    });
+// Album ids: each below n_albums or STRATUM_NO_ALBUM.
+static int32_t albums_validate(const uint32_t* album_of, uint32_t n_tracks, uint32_t n_albums, const StratumLoudness* album_out) {
+    if (n_albums == 0 && !album_of) return STRATUM_OK;
+    if (n_albums > 0 && (!album_of || !album_out)) {
+        set_error("null argument");
+        return STRATUM_INVALID_INPUT;
+    }
+    for (uint32_t q = 0; q < n_tracks; ++q)
+        if (album_of[q] >= n_albums && album_of[q] != STRATUM_NO_ALBUM) {
+            set_error("track " + std::to_string(q) + ": album id " + std::to_string(album_of[q]) + " is not below n_albums = " + std::to_string(n_albums) +
+                      " (STRATUM_NO_ALBUM for a track of no album)");
+            return STRATUM_INVALID_INPUT;
+        }
+    return STRATUM_OK;
 }
 
-int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
-                                               const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out) {
-    std::vector<uint32_t> bpf;
-    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, d_pcm != nullptr, bpf);
-    if (st != STRATUM_OK || n_tracks == 0) return st;
-    DeviceCtx* ctx = get_ctx(device_id, &st);
+// The album results once every member is measured: status, frames and peaks from the member results on the host; the gates, maxima
+// and range of the albums with all members measured from one launch of loud_album_gate_kernel over the pools, on device `device`.
+static int32_t album_phase(int32_t device, AlbumPools& P, uint32_t n_tracks, const StratumLoudness* out, StratumLoudness* album_out) {
+    const uint32_t na = P.n_albums;
+    std::vector<uint32_t> members(na, 0);
+    for (uint32_t a = 0; a < na; ++a) memset(&album_out[a], 0, sizeof album_out[a]);
+    for (uint32_t q = 0; q < n_tracks; ++q) {
+        if (!P.member(q)) continue;
+        StratumLoudness& r = album_out[P.album_of[q]];
+        ++members[P.album_of[q]];
+        if (r.status != STRATUM_OK) continue;
+        if (out[q].status != STRATUM_OK) {  // no values over a partial album
+            r.status = out[q].status;
+            snprintf(r.error, sizeof r.error, "track %u: %.100s", q, out[q].error);
+            r.frames = 0;
+            r.sample_peak = r.true_peak = 0.0;
+            continue;
+        }
+        r.frames += out[q].frames;
+        r.sample_peak = std::max(r.sample_peak, out[q].sample_peak);
+        r.true_peak = std::max(r.true_peak, out[q].true_peak);
+    }
+    uint32_t n_ok = 0;
+    for (uint32_t a = 0; a < na; ++a) {
+        StratumLoudness& r = album_out[a];
+        if (members[a] == 0) {
+            r.status = STRATUM_INVALID_INPUT;
+            snprintf(r.error, sizeof r.error, "album has no tracks");
+        }
+        if (r.status == STRATUM_OK) ++n_ok;
+    }
+    if (n_ok == 0) return STRATUM_OK;
+    int st = STRATUM_OK;
+    DeviceCtx* ctx = get_ctx(device, &st);
     if (!ctx) return st;
     std::lock_guard<std::recursive_mutex> lk(ctx->mu);
     if (cudaSetDevice(ctx->device) != cudaSuccess) {
         set_error("cudaSetDevice failed");
         return STRATUM_PROCESSING_ERROR;
     }
-    // the whole batch is one chunk: one launch of each kernel
-    const std::vector<HostChunk> one{HostChunk{0, n_tracks, byte_offsets[n_tracks] - byte_offsets[0], 0}};
-    LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out);
-    st = sink.open(one);
+    // device: the host buffer as is (records, momentary pool, short-term pool), the selection scratch, the results
+    const size_t buf_bytes = P.buf.size() * sizeof(double), keep_bytes = P.n_sht * sizeof(double);
+    if (!grow_device(ctx->d_album, ctx->album_cap, buf_bytes + keep_bytes + na * sizeof(LoudOut))) {
+        set_error("album work area allocation failed");
+        return STRATUM_PROCESSING_ERROR;
+    }
+    double* d = reinterpret_cast<double*>(ctx->d_album);
+    LoudOut* d_out = reinterpret_cast<LoudOut*>(d + P.buf.size() + P.n_sht);
+    std::vector<LoudOut> h_out(na);
+    cudaStream_t s = ctx->stream;
+    CUDA_OK(cudaMemcpyAsync(d, P.buf.data(), buf_bytes, cudaMemcpyHostToDevice, s));
+    g_h2d_bytes.fetch_add(buf_bytes);
+    {
+        StageTimer tm(s, "loudness_album_gate");
+        launch_loud_album_gate(s, reinterpret_cast<const LoudAlbum*>(d), na, d + P.mom0, d + P.sht0, d + P.buf.size(), d_out);
+    }
+    CUDA_OK(cudaGetLastError());
+    CUDA_OK(cudaMemcpyAsync(h_out.data(), d_out, na * sizeof(LoudOut), cudaMemcpyDeviceToHost, s));
+    g_d2h_bytes.fetch_add(na * sizeof(LoudOut));
+    std::vector<PendingStage> stages;
+    stages.swap(g_pending);
+    CUDA_OK(cudaStreamSynchronize(s));
+    resolve_stage_times(stages);
+    for (uint32_t a = 0; a < na; ++a) {
+        StratumLoudness& r = album_out[a];
+        if (r.status != STRATUM_OK) continue;
+        r.integrated_lufs = h_out[a].integrated;
+        r.momentary_max_lufs = h_out[a].momentary_max;
+        r.short_term_max_lufs = h_out[a].short_term_max;
+        r.loudness_range_lu = h_out[a].loudness_range;
+        r.n_momentary = P.albums()[a].J;
+        r.n_short_term = P.albums()[a].K;
+    }
+    return STRATUM_OK;
+}
+
+int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out, StratumLoudness* album_out) {
+    std::vector<uint32_t> bpf;
+    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, pcm != nullptr, bpf);
+    if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
     if (st != STRATUM_OK) return st;
-    const int s1 = sink.chunk(0, one[0], static_cast<const char*>(d_pcm) + byte_offsets[0], [] {});
-    const int s2 = sink.close();
-    return s1 != STRATUM_OK ? s1 : s2;
+    AlbumPools pools;
+    album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    AlbumPools* pp = n_albums ? &pools : nullptr;
+    if (n_tracks)
+        st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
+            return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, pp));
+        });
+    if (st != STRATUM_OK || n_albums == 0) return st;
+    return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, out, album_out);
+}
+
+int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                int32_t device_id, StratumLoudness* out, StratumLoudness* album_out) {
+    std::vector<uint32_t> bpf;
+    int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, d_pcm != nullptr, bpf);
+    if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
+    if (st != STRATUM_OK) return st;
+    AlbumPools pools;
+    album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    if (n_tracks) {
+        DeviceCtx* ctx = get_ctx(device_id, &st);
+        if (!ctx) return st;
+        std::lock_guard<std::recursive_mutex> lk(ctx->mu);
+        if (cudaSetDevice(ctx->device) != cudaSuccess) {
+            set_error("cudaSetDevice failed");
+            return STRATUM_PROCESSING_ERROR;
+        }
+        // the whole batch is one chunk: one launch of each kernel
+        const std::vector<HostChunk> one{HostChunk{0, n_tracks, byte_offsets[n_tracks] - byte_offsets[0], 0}};
+        LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, n_albums ? &pools : nullptr);
+        st = sink.open(one);
+        if (st != STRATUM_OK) return st;
+        const int s1 = sink.chunk(0, one[0], static_cast<const char*>(d_pcm) + byte_offsets[0], [] {});
+        const int s2 = sink.close();
+        st = s1 != STRATUM_OK ? s1 : s2;
+    }
+    if (st != STRATUM_OK || n_albums == 0) return st;
+    return album_phase(device_id, pools, n_tracks, out, album_out);
+}
+
+int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                        const uint32_t* formats, uint32_t n_tracks, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out) {
+    return stratum_b200_loudness_albums_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, device_ids, n_devices, out, nullptr);
+}
+
+int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                               const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out) {
+    return stratum_b200_loudness_albums_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, device_id, out, nullptr);
 }
 
 int32_t stratum_b200_debug_loudness_filters(uint32_t sample_rate, double* kweight10, float* taps49) {
@@ -2931,6 +3146,7 @@ void stratum_b200_shutdown(void) {
             cudaFree(c->d_conv);
             cudaFree(c->d_meta);
             cudaFree(c->d_loud);
+            cudaFree(c->d_album);
             cudaFree(c->d_count);
             c->uploader.reset();
             for (WaveJob& j : c->jobs) {
@@ -2946,6 +3162,7 @@ void stratum_b200_shutdown(void) {
             for (int b = 0; b < 2; ++b) {
                 c->loud_rec[b].release();
                 c->loud_out[b].release();
+                c->loud_blk[b].release();
                 if (c->loud_ev[b]) cudaEventDestroy(c->loud_ev[b]);
             }
             c->h_count.release();

@@ -9,7 +9,9 @@
 //           sample peak and the 4x / 2x oversampled true peak (49-tap interpolator, 12 / 24 frames of context), reduced per track
 //           by atomicMax on the bit pattern;
 //   gate    one CTA per track: channel-weighted sub-block energies, momentary / short-term powers as in-order sums of 4 / 30
-//           sub-blocks, the absolute and relative gates, the maxima and the loudness range (exact order statistics).
+//           sub-blocks, the absolute and relative gates, the maxima and the loudness range (exact order statistics);
+//   album   one CTA per album: the same gates, maxima and range over the members' momentary / short-term powers, pooled on the
+//           host in ascending track order (stratum_b200_loudness_albums_pcm).
 // The recurrence runs in f64: at 192 kHz the high-pass pole of stage 2 lies 1.2e-3 from the unit circle, and f32 coefficients
 // and state move the 38 Hz corner by about 2 %.  The true-peak FIR runs in f32 with explicit FMAs.  No float atomics on sums:
 // every result depends only on the track's own samples.
@@ -277,33 +279,14 @@ __device__ __forceinline__ double gated_mean(const double* __restrict__ pw, uint
     return *cnt > 0.0 ? s / *cnt : 0.0;
 }
 
-__global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const LoudTrack* __restrict__ tr, const double* __restrict__ en, double* __restrict__ zs,
-                                                                      double* __restrict__ mom, double* __restrict__ sht, double* __restrict__ keep,
-                                                                      LoudOut* __restrict__ out) {
-    const LoudTrack& T = tr[blockIdx.x];
-    if (T.nseg == 0) return;
+// The gates, maxima and loudness range of the momentary powers m[0..J) and short-term powers q[0..K) into o's loudness fields
+// (keep: K doubles of scratch).  The per-track and the album kernel both run it on a CTA of LOUD_GATE_THREADS: the result depends
+// only on the two lists, so an album of one track reproduces the track's bits.
+__device__ __forceinline__ void loud_gate_lists(const double* __restrict__ m, uint32_t J, const double* __restrict__ q, uint32_t K,
+                                                double* __restrict__ kp, LoudOut* __restrict__ o) {
     __shared__ double sm[LOUD_GATE_THREADS];
     __shared__ uint32_t hist[256], bcast[2], wsum[33];
     const double ninf = -CUDART_INF;
-    const uint32_t C = T.C, nfull = T.nfull, J = T.J, K = T.K;
-    double* z = zs + T.seg0;
-    double* m = mom + T.seg0;
-    double* q = sht + T.seg0;
-    double* kp = keep + T.seg0;
-    for (uint32_t i = threadIdx.x; i < nfull; i += LOUD_GATE_THREADS) {
-        double acc = 0.0;
-        for (uint32_t c = 0; c < C; ++c) acc = acc + loud_channel_weight(C, c) * en[T.work + (uint64_t)i * C + c];
-        z[i] = acc;
-    }
-    __syncthreads();
-    const double dm = 4.0 * T.S, ds = 30.0 * T.S;
-    for (uint32_t j = threadIdx.x; j < J; j += LOUD_GATE_THREADS) m[j] = (((z[j] + z[j + 1]) + z[j + 2]) + z[j + 3]) / dm;
-    for (uint32_t j = threadIdx.x; j < K; j += LOUD_GATE_THREADS) {
-        double acc = 0.0;
-        for (int i = 0; i < 30; ++i) acc = acc + z[j + i];
-        q[j] = acc / ds;
-    }
-    __syncthreads();
     // integrated loudness: absolute gate, then the relative gate 10 LU below the absolute-gated mean
     double cnt;
     const double abs_mean = gated_mean(m, J, ninf, sm, &cnt);
@@ -348,12 +331,45 @@ __global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const Loud
         }
     }
     if (threadIdx.x == 0) {
-        LoudOut& o = out[blockIdx.x];
-        o.integrated = integrated;
-        o.momentary_max = J > 0 ? lufs_of(mx) : ninf;
-        o.short_term_max = K > 0 ? lufs_of(sx) : ninf;
-        o.loudness_range = lra;
+        o->integrated = integrated;
+        o->momentary_max = J > 0 ? lufs_of(mx) : ninf;
+        o->short_term_max = K > 0 ? lufs_of(sx) : ninf;
+        o->loudness_range = lra;
     }
+}
+
+__global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const LoudTrack* __restrict__ tr, const double* __restrict__ en, double* __restrict__ zs,
+                                                                      double* __restrict__ mom, double* __restrict__ sht, double* __restrict__ keep,
+                                                                      LoudOut* __restrict__ out) {
+    const LoudTrack& T = tr[blockIdx.x];
+    if (T.nseg == 0) return;
+    const uint32_t C = T.C, nfull = T.nfull, J = T.J, K = T.K;
+    double* z = zs + T.seg0;
+    double* m = mom + T.seg0;
+    double* q = sht + T.seg0;
+    for (uint32_t i = threadIdx.x; i < nfull; i += LOUD_GATE_THREADS) {
+        double acc = 0.0;
+        for (uint32_t c = 0; c < C; ++c) acc = acc + loud_channel_weight(C, c) * en[T.work + (uint64_t)i * C + c];
+        z[i] = acc;
+    }
+    __syncthreads();
+    const double dm = 4.0 * T.S, ds = 30.0 * T.S;
+    for (uint32_t j = threadIdx.x; j < J; j += LOUD_GATE_THREADS) m[j] = (((z[j] + z[j + 1]) + z[j + 2]) + z[j + 3]) / dm;
+    for (uint32_t j = threadIdx.x; j < K; j += LOUD_GATE_THREADS) {
+        double acc = 0.0;
+        for (int i = 0; i < 30; ++i) acc = acc + z[j + i];
+        q[j] = acc / ds;
+    }
+    __syncthreads();
+    loud_gate_lists(m, J, q, K, keep + T.seg0, out + blockIdx.x);
+}
+
+// One CTA per album over its pooled lists.
+__global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_album_gate_kernel(const LoudAlbum* __restrict__ al, const double* __restrict__ mom,
+                                                                            const double* __restrict__ sht, double* __restrict__ keep,
+                                                                            LoudOut* __restrict__ out) {
+    const LoudAlbum& A = al[blockIdx.x];
+    loud_gate_lists(mom + A.m0, A.J, sht + A.q0, A.K, keep + A.q0, out + blockIdx.x);
 }
 
 void launch_loud_pass1(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, double* d_st) {
@@ -378,6 +394,13 @@ void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr,
 void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_en, double* d_ws, uint64_t n_seg, LoudOut* d_out) {
     if (n_tracks == 0) return;
     loud_gate_kernel<<<n_tracks, LOUD_GATE_THREADS, 0, s>>>(d_tr, d_en, d_ws, d_ws + n_seg, d_ws + 2 * n_seg, d_ws + 3 * n_seg, d_out);
+    count_launch("loudness");
+}
+
+void launch_loud_album_gate(cudaStream_t s, const LoudAlbum* d_al, uint32_t n_albums, const double* d_mom, const double* d_sht, double* d_keep,
+                            LoudOut* d_out) {
+    if (n_albums == 0) return;
+    loud_album_gate_kernel<<<n_albums, LOUD_GATE_THREADS, 0, s>>>(d_al, d_mom, d_sht, d_keep, d_out);
     count_launch("loudness");
 }
 

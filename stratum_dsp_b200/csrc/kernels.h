@@ -235,6 +235,14 @@ void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr,
                        LoudOut* d_out);
 // d_ws: 4 x n_seg doubles (sub-block, momentary and short-term powers, the compacted short-term powers of the loudness range)
 void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_en, double* d_ws, uint64_t n_seg, LoudOut* d_out);
+// One record per album: its pooled momentary powers are mom[m0 .. m0 + J), its short-term powers sht[q0 .. q0 + K) (engine.cu:
+// AlbumPools).  d_keep has the size of d_sht; only the loudness fields of d_out are written.
+struct LoudAlbum {
+    uint64_t m0, q0;
+    uint32_t J, K;
+};
+void launch_loud_album_gate(cudaStream_t s, const LoudAlbum* d_al, uint32_t n_albums, const double* d_mom, const double* d_sht, double* d_keep,
+                            LoudOut* d_out);
 // k_synth.cu
 void launch_pcm_to_mono(cudaStream_t s, const void* d_pcm, float* d_out, const uint64_t* d_byte_off, const uint64_t* d_out_off, const uint32_t* d_channels,
                         const uint32_t* d_formats, uint32_t n_tracks, uint64_t max_frames);

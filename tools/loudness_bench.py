@@ -1,16 +1,19 @@
 #!/usr/bin/env python3
 """Throughput of the loudness measurement (stratum_b200_loudness_batch_pcm) on one GPU.
 
-    python tools/loudness_bench.py [--tracks N] [--rounds R] [--warmup W] [--out FILE]
+    python tools/loudness_bench.py [--tracks N] [--rounds R] [--warmup W] [--albums [M]] [--out FILE]
 
 Workload: N (default 1024) stereo three-minute 44.1 kHz PCM16 tracks, each channel a C2 track of tests/synth.py (channel 0 from
-seed i, channel 1 from seed i + 1000), generated on the device and quantised there.  Two legs, timed in alternation after W
-untimed calls of each:
+seed i, channel 1 from seed i + 1000), generated on the device and quantised there.  Two legs (three with --albums), timed in
+alternation after W untimed calls of each:
   device  the PCM already in device memory (stratum_b200_loudness_batch_pcm_device);
-  host    the same bytes in pinned host memory (stratum_b200_loudness_batch_pcm: upload included).
+  host    the same bytes in pinned host memory (stratum_b200_loudness_batch_pcm: upload included);
+  albums  with --albums M (default 12): the host leg as albums of M consecutive tracks (stratum_b200_loudness_albums_pcm), which
+          adds the read-back of the momentary / short-term powers and the album gate.
 Reports the median over R rounds of tracks/s and wall time per leg, the median kernel times of the device leg (pass 1, the scan,
-pass 2 with the true-peak FIR, the gate), the host-to-device rate of a plain 4 GB pinned copy measured in the same run, and the
-card's name and power limit.  Prints one JSON document."""
+pass 2 with the true-peak FIR, the gate), the album gate's kernel time and the device-to-host bytes the album leg adds to the host
+leg (stratum_b200_transfer_bytes), the host-to-device rate of a plain 4 GB pinned copy measured in the same run, and the card's name
+and power limit.  Prints one JSON document."""
 from __future__ import annotations
 
 import argparse
@@ -73,6 +76,7 @@ def main() -> None:
     ap.add_argument("--tracks", type=int, default=1024)
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--warmup", type=int, default=1)
+    ap.add_argument("--albums", type=int, nargs="?", const=12, default=None, metavar="M", help="add the album leg, M tracks per album")
     ap.add_argument("--out", default=None, help="also write the JSON document to this file")
     a = ap.parse_args()
     import torch
@@ -101,25 +105,36 @@ def main() -> None:
     def host_leg():
         return L.stratum_b200_loudness_batch_pcm(C.c_void_p(h_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, None, 0, res)
 
+    n_albums = (n + a.albums - 1) // a.albums if a.albums else 0
+    album_of = np.arange(n, dtype=np.uint32) // np.uint32(a.albums or 1)
+    alb = (S.StratumLoudness * max(n_albums, 1))()
+
+    def album_leg():
+        return L.stratum_b200_loudness_albums_pcm(C.c_void_p(h_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, u32(album_of), n_albums, None, 0,
+                                                  res, alb)
+
     def timed(fn):
         S.stage_times(reset=True)
+        d2h0 = S.transfer_bytes()[1]
         t0 = time.perf_counter()
         st = fn()
         wall = time.perf_counter() - t0
         if st != S.OK:
             raise SystemExit(f"loudness call failed: {S.last_error()}")
         ok = sum(1 for i in range(n) if res[i].status == 0)
-        return wall, S.stage_times(), ok
+        return wall, S.stage_times(), ok, S.transfer_bytes()[1] - d2h0
 
+    legs = [device_leg, host_leg] + ([album_leg] if n_albums else [])
     for _ in range(a.warmup):
-        timed(device_leg)
-        timed(host_leg)
+        for fn in legs:
+            timed(fn)
     S.stage_timing(True)
-    dev, host = [], []
+    runs = {fn: [] for fn in legs}
     for _ in range(a.rounds):
-        dev.append(timed(device_leg))
-        host.append(timed(host_leg))
+        for fn in legs:
+            runs[fn].append(timed(fn))
     S.stage_timing(False)
+    dev, host = runs[device_leg], runs[host_leg]
     # plain pinned host-to-device copy of 4 GB in the same run
     probe = min(h_pcm.numel(), 2 << 30)
     dst = torch.empty(probe, dtype=torch.int16, device="cuda")
@@ -143,6 +158,14 @@ def main() -> None:
         "h2d_pinned_copy_gb_per_s": statistics.median(rates),
         "track0": {"integrated_lufs": sample.integrated_lufs, "loudness_range_lu": sample.loudness_range_lu, "true_peak": sample.true_peak},
     }
+    if n_albums:
+        al = runs[album_leg]
+        doc["host_albums"] = {"tracks_per_album": a.albums, "albums": n_albums, "tracks_per_s": n / statistics.median(r[0] for r in al),
+                              "wall_s": statistics.median(r[0] for r in al), "album_gate_ms": statistics.median(r[1].get("loudness_album_gate", 0.0) for r in al),
+                              "extra_d2h_bytes": statistics.median(r[3] for r in al) - statistics.median(r[3] for r in host),
+                              "pcm_bytes": n * bytes_per_track, "ok_tracks": min(r[2] for r in al),
+                              "ok_albums": sum(1 for i in range(n_albums) if alb[i].status == 0),
+                              "album0": {"integrated_lufs": alb[0].integrated_lufs, "loudness_range_lu": alb[0].loudness_range_lu}}
     s = json.dumps(doc, indent=1)
     print(s)
     if a.out:
