@@ -289,6 +289,30 @@ int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_o
 int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                 const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
                                                 int32_t device_id, StratumLoudness* out, StratumLoudness* album_out);
+/* Analysis and loudness of one host PCM batch from a single upload (a library scan that wants BPM, key and beat grid next to the
+ * track and album gains moves each byte over the host link once instead of twice).  Arguments as stratum_b200_analyze_batch_pcm
+ * (pcm ... cfg, device_ids, n_devices, out) and stratum_b200_loudness_albums_pcm (album_of_track, n_albums, loudness_out = its out,
+ * album_out).
+ *  - out[i] is what stratum_b200_analyze_batch_pcm gives for the same arguments, every field bit for bit except processing_time_ms
+ *    (integer views, beat / onset / HMM arrays and tempogram candidates included); release it with stratum_b200_result_free.
+ *  - loudness_out[i] and album_out[a] are what stratum_b200_loudness_albums_pcm gives, bit for bit.
+ *  - A track's analysis status and its loudness status are independent: an all-zero track fails the analysis ("Audio is entirely
+ *    silent after trimming") and is still measured; a track at 7999 Hz fails the loudness (STRATUM_NOT_IMPLEMENTED) and is analysed
+ *    as stratum_b200_analyze_batch_pcm analyses it.
+ *  - Rejected whole, before any device work: whatever either entry rejects.  STRATUM_NOT_IMPLEMENTED for a configuration
+ *    stratum_b200_analyze_batch_pcm refuses; STRATUM_INVALID_INPUT for a NULL pointer (out and loudness_out included), an unknown
+ *    format, channels outside 1..64, a partial frame, an album id at or above n_albums other than STRATUM_NO_ALBUM, or a NULL
+ *    album_of_track / album_out while n_albums > 0.  n_albums = 0 with album_of_track = NULL: no albums.  Checked in the order of
+ *    stratum_b200_analyze_batch_pcm (NULL pointers, the configuration, the PCM layout), then the album ids: the first failure is
+ *    the one returned.
+ * Tracks are sharded over `device_ids` and streamed through the double-buffered upload as in the two entries; on each device the
+ * loudness passes are queued on a stream of their own, so they need not wait behind the analysis waves (where the analysis already
+ * keeps the device busy, they still add their own kernel time: DESIGN §2).  Album gates run on the first device once every shard
+ * is done. */
+int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                          const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                          uint32_t n_albums, const int32_t* device_ids, uint32_t n_devices, StratumResult* out,
+                                          StratumLoudness* loudness_out, StratumLoudness* album_out);
 /* Host-side filters of the loudness measurement (no device work): kweight10 = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2 (either
  * may be NULL), taps49 = the true-peak interpolator as the device uses it (f32).  Returns the oversampling factor L, or -1 for a
  * sample rate outside 8000..384000 Hz. */

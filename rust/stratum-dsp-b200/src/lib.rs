@@ -221,29 +221,10 @@ pub fn loudness_batch_pcm(tracks: &[PcmTrack], devices: &[i32]) -> Result<Vec<Re
 /// track names, carries its error in its slot.
 pub fn loudness_albums_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], devices: &[i32])
     -> Result<(Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>), AnalysisError> {
-    let ok = unsafe { stratum_b200_sizeof(3) == std::mem::size_of::<StratumLoudness>() };
-    if !ok {
-        return Err(AnalysisError::ProcessingError("libstratum_b200.so does not match this binding (struct sizes differ)".to_string()));
-    }
-    if albums.len() != tracks.len() {
-        return Err(AnalysisError::InvalidInput("one album id (or None) per track".to_string()));
-    }
+    check_loudness_abi()?;
+    let (ids, n_albums) = album_ids(albums, tracks.len())?;
     let n = tracks.len();
-    let ids: Vec<u32> = albums.iter().map(|a| a.unwrap_or(STRATUM_NO_ALBUM)).collect();
-    let n_albums = albums.iter().flatten().map(|a| *a as u64 + 1).max().unwrap_or(0);
-    if n_albums > u32::MAX as u64 {
-        return Err(AnalysisError::InvalidInput("album id STRATUM_NO_ALBUM is reserved for None".to_string()));
-    }
-    let n_albums = n_albums as usize;
-    let mut offsets = vec![0u64];
-    let mut flat: Vec<u8> = Vec::new();
-    for t in tracks {
-        flat.extend_from_slice(t.data);
-        offsets.push(flat.len() as u64);
-    }
-    let srs: Vec<u32> = tracks.iter().map(|t| t.sample_rate).collect();
-    let chans: Vec<u32> = tracks.iter().map(|t| t.channels).collect();
-    let fmts: Vec<u32> = tracks.iter().map(|t| t.format).collect();
+    let (flat, offsets, srs, chans, fmts) = pcm_tables(tracks);
     let mut res: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
     let mut alb: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n_albums];
     let st = unsafe {
@@ -254,22 +235,90 @@ pub fn loudness_albums_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], devices:
     if st != 0 {
         return Err(to_error(st, last_error()));
     }
-    let convert = |r: &StratumLoudness| {
-        if r.status != 0 {
-            return Err(to_error(r.status, c_string(&r.error)));
-        }
-        Ok(Loudness {
-            integrated_lufs: r.integrated_lufs,
-            momentary_max_lufs: r.momentary_max_lufs,
-            short_term_max_lufs: r.short_term_max_lufs,
-            loudness_range_lu: r.loudness_range_lu,
-            sample_peak: r.sample_peak,
-            true_peak: r.true_peak,
-            n_momentary: r.n_momentary,
-            n_short_term: r.n_short_term,
-        })
+    Ok((res.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect()))
+}
+
+/// Analysis (as `analyze_batch` gives it) and loudness (as `loudness_albums_pcm` gives it) of the same PCM tracks from one upload of
+/// each byte.  `albums`: as in `loudness_albums_pcm`, or `None` for no albums (the album list is then empty).  A track's analysis
+/// and its loudness fail or succeed independently.
+pub fn analyze_loudness_pcm(tracks: &[PcmTrack], albums: Option<&[Option<u32>]>, config: AnalysisConfig, devices: &[i32])
+    -> Result<(Vec<Result<AnalysisResult, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>), AnalysisError> {
+    check_abi()?;
+    check_loudness_abi()?;
+    let cfg = config_to_c(&config)?;
+    let n = tracks.len();
+    let (ids, n_albums) = match albums {
+        Some(a) => album_ids(a, n)?,
+        None => (Vec::new(), 0),
     };
-    Ok((res.iter().map(convert).collect(), alb.iter().map(convert).collect()))
+    let (flat, offsets, srs, chans, fmts) = pcm_tables(tracks);
+    let mut res: Vec<StratumResult> = vec![unsafe { std::mem::zeroed() }; n];
+    let mut loud: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
+    let mut alb: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n_albums];
+    let st = unsafe {
+        stratum_b200_analyze_loudness_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, &cfg,
+                                          if albums.is_some() { ids.as_ptr() } else { std::ptr::null() }, n_albums as u32,
+                                          if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
+                                          res.as_mut_ptr(), loud.as_mut_ptr(), alb.as_mut_ptr())
+    };
+    if st != 0 {
+        let e = to_error(st, last_error());
+        unsafe { stratum_b200_result_free(res.as_mut_ptr(), n as u32) }; // waves that completed before the error own heap arrays
+        return Err(e);
+    }
+    let out = res.iter().map(|r| if r.status == 0 { Ok(from_c(r, &config)) } else { Err(to_error(r.status, c_string(&r.error))) }).collect();
+    unsafe { stratum_b200_result_free(res.as_mut_ptr(), n as u32) };
+    Ok((out, loud.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect()))
+}
+
+fn check_loudness_abi() -> Result<(), AnalysisError> {
+    if unsafe { stratum_b200_sizeof(3) } != std::mem::size_of::<StratumLoudness>() {
+        return Err(AnalysisError::ProcessingError("libstratum_b200.so does not match this binding (struct sizes differ)".to_string()));
+    }
+    Ok(())
+}
+
+/// Album ids for the C call (`None` -> `STRATUM_NO_ALBUM`) and the album count, max id + 1.
+fn album_ids(albums: &[Option<u32>], n_tracks: usize) -> Result<(Vec<u32>, usize), AnalysisError> {
+    if albums.len() != n_tracks {
+        return Err(AnalysisError::InvalidInput("one album id (or None) per track".to_string()));
+    }
+    let ids: Vec<u32> = albums.iter().map(|a| a.unwrap_or(STRATUM_NO_ALBUM)).collect();
+    let n_albums = albums.iter().flatten().map(|a| *a as u64 + 1).max().unwrap_or(0);
+    if n_albums > u32::MAX as u64 {
+        return Err(AnalysisError::InvalidInput("album id STRATUM_NO_ALBUM is reserved for None".to_string()));
+    }
+    Ok((ids, n_albums as usize))
+}
+
+/// The tracks' bytes in one buffer, their byte offsets, sample rates, channel counts and formats.
+fn pcm_tables(tracks: &[PcmTrack]) -> (Vec<u8>, Vec<u64>, Vec<u32>, Vec<u32>, Vec<u32>) {
+    let mut offsets = vec![0u64];
+    let mut flat: Vec<u8> = Vec::new();
+    for t in tracks {
+        flat.extend_from_slice(t.data);
+        offsets.push(flat.len() as u64);
+    }
+    let srs: Vec<u32> = tracks.iter().map(|t| t.sample_rate).collect();
+    let chans: Vec<u32> = tracks.iter().map(|t| t.channels).collect();
+    let fmts: Vec<u32> = tracks.iter().map(|t| t.format).collect();
+    (flat, offsets, srs, chans, fmts)
+}
+
+fn loudness_from_c(r: &StratumLoudness) -> Result<Loudness, AnalysisError> {
+    if r.status != 0 {
+        return Err(to_error(r.status, c_string(&r.error)));
+    }
+    Ok(Loudness {
+        integrated_lufs: r.integrated_lufs,
+        momentary_max_lufs: r.momentary_max_lufs,
+        short_term_max_lufs: r.short_term_max_lufs,
+        loudness_range_lu: r.loudness_range_lu,
+        sample_peak: r.sample_peak,
+        true_peak: r.true_peak,
+        n_momentary: r.n_momentary,
+        n_short_term: r.n_short_term,
+    })
 }
 
 /// Decoder-side batch entry: interleaved 16-bit PCM uploaded as is and converted on the device with the arithmetic of

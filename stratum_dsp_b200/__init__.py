@@ -210,6 +210,9 @@ def lib() -> C.CDLL:
     L.stratum_b200_loudness_albums_pcm.restype = _i
     L.stratum_b200_loudness_albums_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, _i, loudp, loudp]
     L.stratum_b200_loudness_albums_pcm_device.restype = _i
+    L.stratum_b200_analyze_loudness_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, C.c_void_p, u32p, _u, i32p, _u, C.POINTER(StratumResult),
+                                                    loudp, loudp]
+    L.stratum_b200_analyze_loudness_pcm.restype = _i
     L.stratum_b200_debug_loudness_filters.argtypes = [_u, C.POINTER(C.c_double), f32p]
     L.stratum_b200_debug_loudness_filters.restype = _i
     if L.stratum_b200_sizeof(0) != C.sizeof(StratumConfig) or L.stratum_b200_sizeof(1) != C.sizeof(StratumResult) or \
@@ -716,6 +719,35 @@ def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_
     if st != OK:
         _raise(st)
     return [_loudness(res[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
+
+
+def analyze_loudness_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None = None, albums: Sequence[int | None] | None = None,
+                         n_albums: int | None = None, devices: Sequence[int] | None = None) -> tuple:
+    """stratum_b200_analyze_loudness_pcm: ``analyze_batch_pcm`` and ``loudness_albums_pcm`` of the same tracks from one upload.
+    Returns ``(results, loudness, album_loudness)``: the analysis results as ``analyze_batch_pcm`` returns them, one ``Loudness`` per
+    track and one per album (``[]`` without ``albums``).  A track's analysis and its loudness fail or succeed independently."""
+    n = len(tracks)
+    if albums is None:
+        if n_albums:
+            raise ValueError("n_albums without album ids")
+        ids, na = None, 0
+    else:
+        ids, na = _album_ids(albums, n, n_albums)
+    flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
+    cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
+    offsets, srs, chans, fmts = _pcm_tables(tracks)
+    res = (StratumResult * max(n, 1))()
+    loud = (StratumLoudness * max(n, 1))()
+    alb = (StratumLoudness * max(na, 1))()
+    dev = (C.c_int32 * len(devices))(*devices) if devices else None
+    cfgp = C.cast(C.byref(config._c), C.c_void_p) if config is not None else None
+    st = lib().stratum_b200_analyze_loudness_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                 srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
+                                                 n, cfgp, ids.ctypes.data_as(C.POINTER(_u)) if ids is not None else None, na, dev,
+                                                 len(devices) if devices else 0, res, loud, alb)
+    if st != OK:
+        _fail(st, res, n)
+    return _collect(res, n), [_loudness(loud[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_filters(sample_rate: int) -> tuple:

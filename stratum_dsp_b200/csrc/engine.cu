@@ -262,6 +262,7 @@ struct DeviceCtx {
     char* d_album = nullptr;  // album phase: album records, pooled powers, selection scratch, results
     size_t album_cap = 0;
     cudaEvent_t loud_ev[2] = {nullptr, nullptr};
+    cudaStream_t loud_stream = nullptr;  // loudness passes of stratum_b200_analyze_loudness_pcm, queued beside the analysis waves
     int32_t* d_count = nullptr;  // escalated tracks of the wave being queued (escalation_compact_kernel)
     PinnedBuf h_count;
     cudaEvent_t ev_legacy = nullptr;  // legacy estimator finished on the key stream
@@ -2564,6 +2565,7 @@ struct LoudnessSink final : ChunkSink {
     const uint32_t *sample_rates, *channels, *formats;
     StratumLoudness* out;
     AlbumPools* pools;  // null without albums
+    cudaStream_t stream;  // every launch and copy of the sink; ctx->stream unless set before open()
     struct Slot {
         uint32_t i = 0, j = 0;
         bool queued = false, blocks = false;  // blocks: the chunk's momentary / short-term powers were read back
@@ -2573,7 +2575,7 @@ struct LoudnessSink final : ChunkSink {
     size_t rec_bytes = 0, out_bytes = 0;
     LoudnessSink(DeviceCtx* c, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans, const uint32_t* fmts,
                  StratumLoudness* o, AlbumPools* p)
-        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p) {}
+        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p), stream(c->stream) {}
     bool has_member(uint32_t i, uint32_t j) const {
         for (uint32_t q = i; pools && q < j; ++q)
             if (pools->member(q)) return true;
@@ -2675,7 +2677,7 @@ struct LoudnessSink final : ChunkSink {
         double* d_en = d_st + 4 * n_work;
         d += align_up(5 * n_work * sizeof(double), 256);
         double* d_ws = reinterpret_cast<double*>(d);
-        cudaStream_t s = ctx->stream;
+        cudaStream_t s = stream;
         CUDA_OK(cudaMemcpyAsync(d_tr, h_tr, (size_t)n * sizeof(LoudTrack), cudaMemcpyHostToDevice, s));
         CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(LoudOut), s));
         g_h2d_bytes.fetch_add((uint64_t)n * sizeof(LoudTrack));
@@ -2921,6 +2923,74 @@ int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t
     return stratum_b200_loudness_albums_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, device_id, out, nullptr);
 }
 
+// Analysis and loudness of the same staged chunks: one upload feeds both.  The loudness passes of a chunk are queued first, on a
+// stream of their own, so they need not wait behind the analysis waves (where the waves keep the device busy they still add their
+// own kernel time: DESIGN §2).  The staged chunk is complete when chunk() is called (the uploads synchronise per piece), so that
+// stream needs no event to read it.  The previous chunk's staging buffer is released once both halves are done with it: the
+// loudness half after its gather, the analysis half once its mono conversion has run.
+struct AnalysisLoudnessSink final : ChunkSink {
+    AnalysisSink ana;
+    LoudnessSink loud;
+    AnalysisLoudnessSink(DeviceCtx* c, const StratumConfig& cfg, const uint64_t* offs, const std::vector<uint32_t>& bpf, const uint32_t* srs,
+                         const uint32_t* chans, const uint32_t* fmts, StratumResult* o, StratumLoudness* lo, AlbumPools* p)
+        : ana(c, cfg, offs, bpf, srs, chans, fmts, o), loud(c, offs, bpf, srs, chans, fmts, lo, p) {}
+
+    int open(const std::vector<HostChunk>& chunks) override {
+        DeviceCtx* ctx = ana.ctx;
+        if (!ctx->loud_stream && cudaStreamCreateWithFlags(&ctx->loud_stream, cudaStreamNonBlocking) != cudaSuccess) {
+            set_error("loudness stream creation failed");
+            return STRATUM_PROCESSING_ERROR;
+        }
+        loud.stream = ctx->loud_stream;
+        // the loudness buffers first: Session::open sizes the analysis arena from the device memory still free
+        const int st = loud.open(chunks);
+        return st != STRATUM_OK ? st : ana.open(chunks);
+    }
+
+    int chunk(size_t k, const HostChunk& ch, const char* d_buf, const std::function<void()>& after_prev) override {
+        int done = 0;
+        const std::function<void()> half_done = [&] {
+            if (++done == 2) after_prev();
+        };
+        const int st = loud.chunk(k, ch, d_buf, half_done);
+        return st != STRATUM_OK ? st : ana.chunk(k, ch, d_buf, half_done);
+    }
+
+    int close() override {
+        const int s1 = ana.close(), s2 = loud.close();
+        cudaStreamSynchronize(loud.stream);  // after a failure inside loud.chunk, launches without a recorded event may still read the staging buffer
+        return s1 != STRATUM_OK ? s1 : s2;
+    }
+};
+
+int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                          const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                          uint32_t n_albums, const int32_t* device_ids, uint32_t n_devices, StratumResult* out,
+                                          StratumLoudness* loudness_out, StratumLoudness* album_out) {
+    // the order of stratum_b200_analyze_batch_pcm: NULL pointers, the configuration, the PCM layout; then the album ids
+    if (!byte_offsets || !sample_rates || !channels || !formats || !out || !loudness_out || (!pcm && n_tracks && byte_offsets[n_tracks] > 0)) {
+        set_error("null argument");
+        return STRATUM_INVALID_INPUT;
+    }
+    StratumConfig def;
+    config_default(&def);
+    const StratumConfig& c = cfg ? *cfg : def;
+    std::vector<uint32_t> bpf;
+    int st = config_validate(c);
+    if (st == STRATUM_OK) st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, loudness_out, pcm != nullptr, bpf);
+    if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
+    if (st != STRATUM_OK) return st;
+    AlbumPools pools;
+    album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    AlbumPools* pp = n_albums ? &pools : nullptr;
+    if (n_tracks)
+        st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
+            return std::unique_ptr<ChunkSink>(new AnalysisLoudnessSink(ctx, c, byte_offsets, bpf, sample_rates, channels, formats, out, loudness_out, pp));
+        });
+    if (st != STRATUM_OK || n_albums == 0) return st;
+    return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, loudness_out, album_out);
+}
+
 int32_t stratum_b200_debug_loudness_filters(uint32_t sample_rate, double* kweight10, float* taps49) {
     char msg[128];
     if (loud_track_status(sample_rate, 1, msg, sizeof msg) != STRATUM_OK) return -1;
@@ -3133,6 +3203,7 @@ void stratum_b200_shutdown(void) {
         if (c->ready) {
             cudaSetDevice(c->device);
             cudaStreamSynchronize(c->stream);
+            if (c->loud_stream) cudaStreamSynchronize(c->loud_stream);
             for (void* p : c->owned) cudaFree(p);
             cudaFree(c->fa);
             cudaFree(c->oa);
@@ -3168,6 +3239,7 @@ void stratum_b200_shutdown(void) {
             c->h_count.release();
             if (c->ev_legacy) cudaEventDestroy(c->ev_legacy);
             if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
+            if (c->loud_stream) cudaStreamDestroy(c->loud_stream);
             cudaStreamDestroy(c->stream);
             if (c->key_stream) cudaStreamDestroy(c->key_stream);
         }
