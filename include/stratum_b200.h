@@ -229,7 +229,8 @@ int32_t stratum_b200_analyze_batch_pcm(const void* pcm, const uint64_t* byte_off
  * Track i: `frames` sample frames of C channels at sr Hz, converted to f32 exactly as stratum_b200_analyze_batch_pcm converts them
  * (but never mixed down).  S = (sr + 5) / 10 frames (100 ms).
  *  - Channel weights (libebur128's default map): 1 channel L; 4 channels L R Ls Rs; 5 channels L R C Ls Rs; any other count
- *    0 L, 1 R, 2 C, 3 unused (LFE), 4 Ls, 5 Rs, 6 and up unused.  L, R, C weigh 1.0, Ls and Rs 1.41, unused channels 0.
+ *    0 L, 1 R, 2 C, 3 unused (LFE), 4 Ls, 5 Rs, 6 and up unused.  L, R, C weigh 1.0, Ls and Rs 1.41, unused channels 0.  A caller
+ *    whose files state their layout passes a channel map instead (stratum_b200_loudness_mapped_pcm, StratumChannelClass).
  *  - K-weighting: a high shelf (f0 1681.974450955533 Hz, G 3.999843853973347 dB, Q 0.7071752369554196) and a high-pass
  *    (f0 38.13547087602444 Hz, Q 0.5003270373238773) per channel in cascade, zero state at frame 0, coefficients derived per
  *    sample rate from the analog prototype (at 48 kHz they equal BS.1770-4's tables).
@@ -313,6 +314,61 @@ int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_
                                           const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
                                           uint32_t n_albums, const int32_t* device_ids, uint32_t n_devices, StratumResult* out,
                                           StratumLoudness* loudness_out, StratumLoudness* album_out);
+
+/* Channel maps and per-channel results.  A channel map gives every channel of a track one class (one uint8_t per channel), and the
+ * class gives the channel's weight G_c in the power of the loudness definition above (BS.1770-4):
+ *   STRATUM_CH_UNUSED     weight 0     LFE, unassigned or ignored channels;
+ *   STRATUM_CH_FRONT      weight 1.0   L, R, C and every position with |azimuth| < 60 deg or > 120 deg, or elevation >= 30 deg;
+ *   STRATUM_CH_SURROUND   weight 1.41  |azimuth| 60..120 deg at elevation < 30 deg (5.1 Ls / Rs at +-110 deg, the 7.1 side pair at
+ *                                      +-90 deg);
+ *   STRATUM_CH_DUAL_MONO  weight 2.0   a mono channel played on two loudspeakers (+3.01 dB; libebur128's EBUR128_DUAL_MONO).
+ * The default map of each channel count is written in these classes by stratum_b200_loudness_channel_map(0, C, 0, map), and a map
+ * with the default classes gives results bit-identical to no map. */
+typedef enum StratumChannelClass {
+    STRATUM_CH_UNUSED = 0,
+    STRATUM_CH_FRONT = 1,
+    STRATUM_CH_SURROUND = 2,
+    STRATUM_CH_DUAL_MONO = 3
+} StratumChannelClass;
+/* stratum_b200_loudness_albums_pcm with two more arguments:
+ *  - channel_map: NULL, the default map for every track; otherwise sum of channels[i] classes, track i's from index
+ *    sum_{j<i} channels[j] on, in frame order.  The power stays sum over c of G_c * mean(y_c^2), summed in channel order.
+ *  - channel_out: NULL, no per-channel results; otherwise sum of channels[i] entries in the same layout.  Entry (i, c) is channel c of
+ *    track i measured alone as a one-channel programme of weight 1.0, whatever its class: every loudness value, both peaks,
+ *    n_momentary and n_short_term, channels = 1, the track's sample_rate and frames, and the track's status and error.  It equals,
+ *    bit for bit, the result of stratum_b200_loudness_batch_pcm for a one-channel track holding exactly that channel's samples in
+ *    the same format.
+ * out[i].sample_peak / true_peak stay the maxima over all channels, unused ones included (the maxima over channel_out's entries).
+ * Albums pool their members' momentary and short-term powers, weighted by the members' maps; there are no per-channel album values.
+ * Rejected whole (STRATUM_INVALID_INPUT, before any device work), after every check of stratum_b200_loudness_albums_pcm: a class
+ * code above STRATUM_CH_DUAL_MONO.  The four stratum_b200_loudness_*_pcm entries are this entry with channel_map = channel_out =
+ * NULL. */
+int32_t stratum_b200_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out,
+                                         StratumLoudness* album_out, StratumLoudness* channel_out);
+/* Same, with the PCM already resident in the memory of device `device_id`. */
+int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                const uint8_t* channel_map, int32_t device_id, StratumLoudness* out, StratumLoudness* album_out,
+                                                StratumLoudness* channel_out);
+/* stratum_b200_analyze_loudness_pcm with channel_map and channel_out as in stratum_b200_loudness_mapped_pcm.  The map weighs the
+ * loudness only: out[i] stays what stratum_b200_analyze_batch_pcm gives (its mixdown is the equal-weight average).  The map is
+ * checked after every other check; stratum_b200_analyze_loudness_pcm is this entry with channel_map = channel_out = NULL. */
+int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                 const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                                 uint32_t n_albums, const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices,
+                                                 StratumResult* out, StratumLoudness* loudness_out, StratumLoudness* album_out,
+                                                 StratumLoudness* channel_out);
+/* The classes of a track's `channels` channels (1..64) from a WAVE_FORMAT_EXTENSIBLE channel mask, into map[0 .. channels); no
+ * device work.  Mask 0: the default map of the channel count.  Otherwise channel c takes the c-th lowest set bit of the mask, and
+ * channels beyond the set bits are UNUSED.  SPEAKER_LOW_FREQUENCY (0x8) and the bits above SPEAKER_TOP_BACK_RIGHT (0x20000) are
+ * UNUSED; SIDE_LEFT / SIDE_RIGHT (0x200, 0x400) SURROUND; BACK_LEFT / BACK_RIGHT (0x10, 0x20) SURROUND when the mask has no side
+ * bit (quad, 5.1 with back surrounds: they sit at +-110 deg) and FRONT when it has one (7.1: the rear pair sits at +-135..150 deg);
+ * every other position (centre, back centre, front-of-centre, the top positions) FRONT.  dual_mono != 0 makes the class of a
+ * one-channel track DUAL_MONO unless it is UNUSED.  Returns STRATUM_OK, or STRATUM_INVALID_INPUT for a NULL map or channels
+ * outside 1..64. */
+int32_t stratum_b200_loudness_channel_map(uint32_t wave_mask, uint32_t channels, int32_t dual_mono, uint8_t* map);
 /* Host-side filters of the loudness measurement (no device work): kweight10 = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2 (either
  * may be NULL), taps49 = the true-peak interpolator as the device uses it (f32).  Returns the oversampling factor L, or -1 for a
  * sample rate outside 8000..384000 Hz. */

@@ -221,21 +221,47 @@ pub fn loudness_batch_pcm(tracks: &[PcmTrack], devices: &[i32]) -> Result<Vec<Re
 /// track names, carries its error in its slot.
 pub fn loudness_albums_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], devices: &[i32])
     -> Result<(Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>), AnalysisError> {
+    loudness_mapped_pcm(tracks, albums, None, false, devices).map(|(per_track, per_album, _)| (per_track, per_album))
+}
+
+/// Per-channel results of `loudness_mapped_pcm`: for each track, one `Loudness` per channel, each channel measured alone at weight
+/// 1.0 (empty without `per_channel`).
+pub type PerChannel = Vec<Vec<Result<Loudness, AnalysisError>>>;
+
+/// The BS.1770-4 channel classes (`STRATUM_CH_*`) of a track of `channels` channels from its WAVE_FORMAT_EXTENSIBLE channel mask
+/// (0: the default map of the channel count); `dual_mono` weighs a one-channel track as a mono signal on two loudspeakers.
+pub fn channel_map(wave_mask: u32, channels: u32, dual_mono: bool) -> Result<Vec<u8>, AnalysisError> {
+    let mut map = vec![0u8; channels.max(1) as usize];
+    let st = unsafe { stratum_b200_loudness_channel_map(wave_mask, channels, dual_mono as i32, map.as_mut_ptr()) };
+    if st != 0 {
+        return Err(to_error(st, last_error()));
+    }
+    Ok(map)
+}
+
+/// `loudness_albums_pcm` with channel maps and per-channel results: `channel_maps[i]` holds track i's channel classes (`None`: its
+/// default map; `channel_maps = None`: the default map for every track); with `per_channel` the third list holds each track's
+/// channels measured alone.  Albums pool their members' mapped powers.
+pub fn loudness_mapped_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], channel_maps: Option<&[Option<Vec<u8>>]>, per_channel: bool, devices: &[i32])
+    -> Result<(Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>, PerChannel), AnalysisError> {
     check_loudness_abi()?;
     let (ids, n_albums) = album_ids(albums, tracks.len())?;
     let n = tracks.len();
     let (flat, offsets, srs, chans, fmts) = pcm_tables(tracks);
+    let map = flat_channel_map(channel_maps, &chans)?;
     let mut res: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
     let mut alb: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n_albums];
+    let mut chout: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; if per_channel { chans.iter().map(|&c| c as usize).sum() } else { 0 }];
     let st = unsafe {
-        stratum_b200_loudness_albums_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, ids.as_ptr(),
-                                         n_albums as u32, if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
-                                         res.as_mut_ptr(), alb.as_mut_ptr())
+        stratum_b200_loudness_mapped_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, ids.as_ptr(),
+                                         n_albums as u32, map.as_ref().map_or(std::ptr::null(), |m| m.as_ptr()),
+                                         if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
+                                         res.as_mut_ptr(), alb.as_mut_ptr(), if per_channel { chout.as_mut_ptr() } else { std::ptr::null_mut() })
     };
     if st != 0 {
         return Err(to_error(st, last_error()));
     }
-    Ok((res.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect()))
+    Ok((res.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect(), split_channels(&chout, &chans, per_channel)))
 }
 
 /// Analysis (as `analyze_batch` gives it) and loudness (as `loudness_albums_pcm` gives it) of the same PCM tracks from one upload of
@@ -243,6 +269,16 @@ pub fn loudness_albums_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], devices:
 /// and its loudness fail or succeed independently.
 pub fn analyze_loudness_pcm(tracks: &[PcmTrack], albums: Option<&[Option<u32>]>, config: AnalysisConfig, devices: &[i32])
     -> Result<(Vec<Result<AnalysisResult, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>), AnalysisError> {
+    analyze_loudness_mapped_pcm(tracks, albums, None, false, config, devices).map(|(results, per_track, per_album, _)| (results, per_track, per_album))
+}
+
+/// `analyze_loudness_pcm` with `channel_maps` and `per_channel` as in `loudness_mapped_pcm`; the maps weigh the loudness only (the
+/// analysis mixdown stays the equal-weight average).
+#[allow(clippy::type_complexity)]
+pub fn analyze_loudness_mapped_pcm(tracks: &[PcmTrack], albums: Option<&[Option<u32>]>, channel_maps: Option<&[Option<Vec<u8>>]>, per_channel: bool,
+                                   config: AnalysisConfig, devices: &[i32])
+    -> Result<(Vec<Result<AnalysisResult, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>, Vec<Result<Loudness, AnalysisError>>, PerChannel),
+              AnalysisError> {
     check_abi()?;
     check_loudness_abi()?;
     let cfg = config_to_c(&config)?;
@@ -252,14 +288,18 @@ pub fn analyze_loudness_pcm(tracks: &[PcmTrack], albums: Option<&[Option<u32>]>,
         None => (Vec::new(), 0),
     };
     let (flat, offsets, srs, chans, fmts) = pcm_tables(tracks);
+    let map = flat_channel_map(channel_maps, &chans)?;
     let mut res: Vec<StratumResult> = vec![unsafe { std::mem::zeroed() }; n];
     let mut loud: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
     let mut alb: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n_albums];
+    let mut chout: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; if per_channel { chans.iter().map(|&c| c as usize).sum() } else { 0 }];
     let st = unsafe {
-        stratum_b200_analyze_loudness_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, &cfg,
-                                          if albums.is_some() { ids.as_ptr() } else { std::ptr::null() }, n_albums as u32,
-                                          if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
-                                          res.as_mut_ptr(), loud.as_mut_ptr(), alb.as_mut_ptr())
+        stratum_b200_analyze_loudness_mapped_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, &cfg,
+                                                 if albums.is_some() { ids.as_ptr() } else { std::ptr::null() }, n_albums as u32,
+                                                 map.as_ref().map_or(std::ptr::null(), |m| m.as_ptr()),
+                                                 if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
+                                                 res.as_mut_ptr(), loud.as_mut_ptr(), alb.as_mut_ptr(),
+                                                 if per_channel { chout.as_mut_ptr() } else { std::ptr::null_mut() })
     };
     if st != 0 {
         let e = to_error(st, last_error());
@@ -268,7 +308,39 @@ pub fn analyze_loudness_pcm(tracks: &[PcmTrack], albums: Option<&[Option<u32>]>,
     }
     let out = res.iter().map(|r| if r.status == 0 { Ok(from_c(r, &config)) } else { Err(to_error(r.status, c_string(&r.error))) }).collect();
     unsafe { stratum_b200_result_free(res.as_mut_ptr(), n as u32) };
-    Ok((out, loud.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect()))
+    Ok((out, loud.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect(), split_channels(&chout, &chans, per_channel)))
+}
+
+/// The maps of the tracks in one buffer for the C call (`None` entries filled with the default map), or `None` for no map.
+fn flat_channel_map(channel_maps: Option<&[Option<Vec<u8>>]>, chans: &[u32]) -> Result<Option<Vec<u8>>, AnalysisError> {
+    let Some(maps) = channel_maps else { return Ok(None) };
+    if maps.len() != chans.len() {
+        return Err(AnalysisError::InvalidInput("one channel map (or None) per track".to_string()));
+    }
+    let mut flat = Vec::new();
+    for (i, (m, &c)) in maps.iter().zip(chans).enumerate() {
+        let m = match m {
+            Some(m) => m.clone(),
+            None => channel_map(0, c, false)?,
+        };
+        if m.len() != c as usize {
+            return Err(AnalysisError::InvalidInput(format!("track {i}: {} channel classes for {c} channels", m.len())));
+        }
+        flat.extend_from_slice(&m);
+    }
+    Ok(Some(flat))
+}
+
+fn split_channels(chout: &[StratumLoudness], chans: &[u32], per_channel: bool) -> PerChannel {
+    if !per_channel {
+        return chans.iter().map(|_| Vec::new()).collect();
+    }
+    let mut at = 0usize;
+    chans.iter().map(|&c| {
+        let v = chout[at..at + c as usize].iter().map(loudness_from_c).collect();
+        at += c as usize;
+        v
+    }).collect()
 }
 
 fn check_loudness_abi() -> Result<(), AnalysisError> {

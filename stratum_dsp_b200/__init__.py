@@ -213,6 +213,16 @@ def lib() -> C.CDLL:
     L.stratum_b200_analyze_loudness_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, C.c_void_p, u32p, _u, i32p, _u, C.POINTER(StratumResult),
                                                     loudp, loudp]
     L.stratum_b200_analyze_loudness_pcm.restype = _i
+    u8p = C.POINTER(C.c_uint8)
+    L.stratum_b200_loudness_mapped_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, u8p, i32p, _u, loudp, loudp, loudp]
+    L.stratum_b200_loudness_mapped_pcm.restype = _i
+    L.stratum_b200_loudness_mapped_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, u8p, _i, loudp, loudp, loudp]
+    L.stratum_b200_loudness_mapped_pcm_device.restype = _i
+    L.stratum_b200_analyze_loudness_mapped_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, C.c_void_p, u32p, _u, u8p, i32p, _u,
+                                                           C.POINTER(StratumResult), loudp, loudp, loudp]
+    L.stratum_b200_analyze_loudness_mapped_pcm.restype = _i
+    L.stratum_b200_loudness_channel_map.argtypes = [_u, _u, _i, u8p]
+    L.stratum_b200_loudness_channel_map.restype = _i
     L.stratum_b200_debug_loudness_filters.argtypes = [_u, C.POINTER(C.c_double), f32p]
     L.stratum_b200_debug_loudness_filters.restype = _i
     if L.stratum_b200_sizeof(0) != C.sizeof(StratumConfig) or L.stratum_b200_sizeof(1) != C.sizeof(StratumResult) or \
@@ -515,6 +525,7 @@ class PcmTrack:
     fmt: int          # PCM_*
     channels: int
     sample_rate: int
+    channel_mask: int = 0  # WAVE_FORMAT_EXTENSIBLE dwChannelMask (0: not stated); read by channel_map, never implicitly
 
     @property
     def frames(self) -> int:
@@ -532,7 +543,7 @@ def read_wav(path) -> PcmTrack:
     hdr = bytes(raw[:12])
     if len(hdr) < 12 or hdr[:4] != b"RIFF" or hdr[8:12] != b"WAVE":
         raise ValueError("not a RIFF/WAVE file")
-    pos, fmt, data = 12, None, None
+    pos, fmt, data, mask = 12, None, None, 0
     while pos + 8 <= raw.size:
         cid = bytes(raw[pos:pos + 4])
         (size,) = struct.unpack("<I", bytes(raw[pos + 4:pos + 8]))
@@ -540,7 +551,8 @@ def read_wav(path) -> PcmTrack:
         if cid == b"fmt ":
             f = bytes(raw[body:body + min(size, 40)])
             tag, ch, sr, _br, _align, bits = struct.unpack("<HHIIHH", f[:16])
-            if tag == 0xFFFE and len(f) >= 40:  # WAVE_FORMAT_EXTENSIBLE: the sub-format GUID starts with the real tag
+            if tag == 0xFFFE and len(f) >= 40:  # WAVE_FORMAT_EXTENSIBLE: the channel mask, and the sub-format GUID starts with the real tag
+                (mask,) = struct.unpack("<I", f[20:24])
                 (tag,) = struct.unpack("<H", f[24:26])
             fmt = (tag, ch, sr, bits)
         elif cid == b"data":
@@ -562,7 +574,7 @@ def read_wav(path) -> PcmTrack:
     if ch == 0:
         raise ValueError("WAVE file with zero channels")
     frame = _PCM_BYTES[pf] * ch
-    return PcmTrack(np.ascontiguousarray(data[: data.size // frame * frame]), pf, ch, sr)
+    return PcmTrack(np.ascontiguousarray(data[: data.size // frame * frame]), pf, ch, sr, mask)
 
 
 def analyze_batch_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None = None, devices: Sequence[int] | None = None) -> list:
@@ -607,12 +619,67 @@ class Loudness:
     channels: int
     frames: int
     error: AnalysisError | None = None  # set instead of raising for a track that failed on its own
+    per_channel: list | None = None     # per_channel=True: one Loudness per channel, each measured alone at weight 1.0
 
 
 def _loudness(r: StratumLoudness) -> Loudness:
     err = AnalysisError(r.status, r.error.decode(errors="replace")) if r.status != OK else None
     return Loudness(r.integrated_lufs, r.momentary_max_lufs, r.short_term_max_lufs, r.loudness_range_lu, r.sample_peak, r.true_peak,
                     int(r.n_momentary), int(r.n_short_term), int(r.sample_rate), int(r.channels), int(r.frames), err)
+
+
+CH_UNUSED, CH_FRONT, CH_SURROUND, CH_DUAL_MONO = 0, 1, 2, 3  # StratumChannelClass: weights 0, 1.0, 1.41, 2.0
+
+
+def channel_map(track_or_mask, channels: int | None = None, dual_mono: bool = False) -> list:
+    """stratum_b200_loudness_channel_map: the BS.1770-4 channel classes (CH_*) of a track from its WAVE_FORMAT_EXTENSIBLE channel
+    mask.  ``track_or_mask`` is a ``PcmTrack`` (its ``channel_mask`` and ``channels``) or a mask with ``channels`` given; mask 0 gives
+    the default map of the channel count.  ``dual_mono`` weighs a one-channel track as a mono signal played on two loudspeakers."""
+    if isinstance(track_or_mask, PcmTrack):
+        mask, channels = track_or_mask.channel_mask, track_or_mask.channels if channels is None else channels
+    else:
+        mask = int(track_or_mask)
+        if channels is None:
+            raise ValueError("channels is required with a mask")
+    out = np.zeros(max(int(channels), 1), np.uint8)
+    st = lib().stratum_b200_loudness_channel_map(mask & 0xFFFFFFFF, int(channels), int(bool(dual_mono)), out.ctypes.data_as(C.POINTER(C.c_uint8)))
+    if st != OK:
+        _raise(st)
+    return [int(v) for v in out]
+
+
+def _channel_args(channel_maps, per_channel: bool, chans: np.ndarray):
+    """(flat uint8 map or None, per-channel result array or None) of the mapped entries."""
+    n = chans.size
+    cmap = None
+    if channel_maps is not None:
+        if len(channel_maps) != n:
+            raise ValueError("one channel map (or None) per track")
+        parts = []
+        for i, m in enumerate(channel_maps):
+            if m is None:
+                m = channel_map(0, int(chans[i]))
+            if len(m) != int(chans[i]):
+                raise ValueError(f"track {i}: {len(m)} channel classes for {int(chans[i])} channels")
+            if any(int(v) < 0 or int(v) > 255 for v in m):
+                raise ValueError(f"track {i}: channel classes are codes 0..3 (CH_*)")
+            parts.append(np.asarray([int(v) for v in m], np.uint8))
+        cmap = np.ascontiguousarray(np.concatenate(parts) if parts else np.zeros(0, np.uint8))
+    chout = (StratumLoudness * max(int(chans.sum()), 1))() if per_channel else None
+    return cmap, chout
+
+
+def _u8p(a):
+    return a.ctypes.data_as(C.POINTER(C.c_uint8)) if a is not None else None
+
+
+def _with_channels(loud: list, chout, chans: np.ndarray) -> list:
+    if chout is not None:
+        at = 0
+        for g, c in zip(loud, chans):
+            g.per_channel = [_loudness(chout[at + k]) for k in range(int(c))]
+            at += int(c)
+    return loud
 
 
 def _pcm_tables(tracks: Sequence[PcmTrack]):
@@ -625,42 +692,24 @@ def _pcm_tables(tracks: Sequence[PcmTrack]):
     return offsets, srs, chans, fmts
 
 
-def loudness_batch_pcm(tracks: Sequence[PcmTrack], devices: Sequence[int] | None = None) -> list:
+def loudness_batch_pcm(tracks: Sequence[PcmTrack], devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None,
+                       per_channel: bool = False) -> list:
     """stratum_b200_loudness_batch_pcm: integrated loudness, maxima, loudness range and peaks of undecoded PCM tracks, measured on
-    the device and sharded over ``devices`` (default: the current device).  A failed track carries ``.error``."""
-    n = len(tracks)
-    if n == 0:
+    the device and sharded over ``devices`` (default: the current device).  A failed track carries ``.error``.
+    ``channel_maps``: one list of channel classes (CH_*, e.g. from ``channel_map``) per track, ``None`` for a track's default map;
+    ``per_channel=True`` fills each track's ``.per_channel`` (stratum_b200_loudness_mapped_pcm)."""
+    if len(tracks) == 0:
         return []
-    flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
-    cat = np.concatenate(flat) if n > 1 else flat[0]
-    offsets, srs, chans, fmts = _pcm_tables(tracks)
-    res = (StratumLoudness * n)()
-    dev = (C.c_int32 * len(devices))(*devices) if devices else None
-    st = lib().stratum_b200_loudness_batch_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
-                                               srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
-                                               n, dev, len(devices) if devices else 0, res)
-    if st != OK:
-        _raise(st)
-    return [_loudness(res[i]) for i in range(n)]
+    return loudness_albums_pcm(tracks, [None] * len(tracks), 0, devices, channel_maps=channel_maps, per_channel=per_channel)[0]
 
 
 def loudness_batch_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
-                              device: int = -1) -> list:
+                              device: int = -1, *, channel_maps: Sequence | None = None, per_channel: bool = False) -> list:
     """stratum_b200_loudness_batch_pcm_device: the same with the PCM already in device memory (``d_pcm_ptr`` = device address of the
     concatenated track bytes, e.g. ``tensor.data_ptr()``; track i = bytes [byte_offsets[i], byte_offsets[i + 1]))."""
-    offsets = np.ascontiguousarray(byte_offsets, dtype=np.uint64)
-    n = offsets.size - 1
-    srs = np.ascontiguousarray(sample_rates, dtype=np.uint32)
-    chans = np.ascontiguousarray(channels, dtype=np.uint32)
-    fmts = np.ascontiguousarray(formats, dtype=np.uint32)
-    if not (srs.size == chans.size == fmts.size == n):
-        raise ValueError("one sample rate, channel count and format per track")
-    res = (StratumLoudness * max(n, 1))()
-    st = lib().stratum_b200_loudness_batch_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)), srs.ctypes.data_as(C.POINTER(_u)),
-                                                      chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)), n, device, res)
-    if st != OK:
-        _raise(st)
-    return [_loudness(res[i]) for i in range(n)]
+    n = np.asarray(byte_offsets).size - 1
+    return loudness_albums_pcm_device(d_pcm_ptr, byte_offsets, sample_rates, channels, formats, [None] * n, 0, device, channel_maps=channel_maps,
+                                      per_channel=per_channel)[0]
 
 
 NO_ALBUM = 0xFFFFFFFF  # STRATUM_NO_ALBUM
@@ -678,29 +727,32 @@ def _album_ids(albums: Sequence[int | None], n_tracks: int, n_albums: int | None
 
 
 def loudness_albums_pcm(tracks: Sequence[PcmTrack], albums: Sequence[int | None], n_albums: int | None = None,
-                        devices: Sequence[int] | None = None) -> tuple:
+                        devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None, per_channel: bool = False) -> tuple:
     """stratum_b200_loudness_albums_pcm: the per-track results of ``loudness_batch_pcm`` and the loudness of albums (ReplayGain /
     R128 album values), each measured over the pooled 400 ms blocks and 3 s windows of its members.  ``albums[i]`` is the album id of
     track i (``None``: no album); ``n_albums`` defaults to the largest id + 1.  Returns ``(tracks, albums)``, two lists of
-    ``Loudness``; an album with a failed member, or one that no track names, carries ``.error``."""
+    ``Loudness``; an album with a failed member, or one that no track names, carries ``.error``.  ``channel_maps`` and ``per_channel``
+    as in ``loudness_batch_pcm``; albums pool the members' mapped powers."""
     n = len(tracks)
     ids, na = _album_ids(albums, n, n_albums)
     flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
     cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
     offsets, srs, chans, fmts = _pcm_tables(tracks)
+    cmap, chout = _channel_args(channel_maps, per_channel, chans)
     res = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
     dev = (C.c_int32 * len(devices))(*devices) if devices else None
-    st = lib().stratum_b200_loudness_albums_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+    st = lib().stratum_b200_loudness_mapped_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
                                                 srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
-                                                n, ids.ctypes.data_as(C.POINTER(_u)), na, dev, len(devices) if devices else 0, res, alb)
+                                                n, ids.ctypes.data_as(C.POINTER(_u)), na, _u8p(cmap), dev, len(devices) if devices else 0, res, alb, chout)
     if st != OK:
         _raise(st)
-    return [_loudness(res[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
+    return _with_channels([_loudness(res[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
-                               albums: Sequence[int | None], n_albums: int | None = None, device: int = -1) -> tuple:
+                               albums: Sequence[int | None], n_albums: int | None = None, device: int = -1, *, channel_maps: Sequence | None = None,
+                               per_channel: bool = False) -> tuple:
     """stratum_b200_loudness_albums_pcm_device: ``loudness_albums_pcm`` with the PCM already in device memory (arguments as
     ``loudness_batch_pcm_device``)."""
     offsets = np.ascontiguousarray(byte_offsets, dtype=np.uint64)
@@ -711,21 +763,25 @@ def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_
     if not (srs.size == chans.size == fmts.size == n):
         raise ValueError("one sample rate, channel count and format per track")
     ids, na = _album_ids(albums, n, n_albums)
+    cmap, chout = _channel_args(channel_maps, per_channel, chans)
     res = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
-    st = lib().stratum_b200_loudness_albums_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+    st = lib().stratum_b200_loudness_mapped_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
                                                        srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)),
-                                                       fmts.ctypes.data_as(C.POINTER(_u)), n, ids.ctypes.data_as(C.POINTER(_u)), na, device, res, alb)
+                                                       fmts.ctypes.data_as(C.POINTER(_u)), n, ids.ctypes.data_as(C.POINTER(_u)), na, _u8p(cmap), device, res,
+                                                       alb, chout)
     if st != OK:
         _raise(st)
-    return [_loudness(res[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
+    return _with_channels([_loudness(res[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
 
 
 def analyze_loudness_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None = None, albums: Sequence[int | None] | None = None,
-                         n_albums: int | None = None, devices: Sequence[int] | None = None) -> tuple:
+                         n_albums: int | None = None, devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None,
+                         per_channel: bool = False) -> tuple:
     """stratum_b200_analyze_loudness_pcm: ``analyze_batch_pcm`` and ``loudness_albums_pcm`` of the same tracks from one upload.
     Returns ``(results, loudness, album_loudness)``: the analysis results as ``analyze_batch_pcm`` returns them, one ``Loudness`` per
-    track and one per album (``[]`` without ``albums``).  A track's analysis and its loudness fail or succeed independently."""
+    track and one per album (``[]`` without ``albums``).  A track's analysis and its loudness fail or succeed independently.
+    ``channel_maps`` and ``per_channel`` weigh and split the loudness only (stratum_b200_analyze_loudness_mapped_pcm)."""
     n = len(tracks)
     if albums is None:
         if n_albums:
@@ -736,18 +792,19 @@ def analyze_loudness_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | No
     flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
     cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
     offsets, srs, chans, fmts = _pcm_tables(tracks)
+    cmap, chout = _channel_args(channel_maps, per_channel, chans)
     res = (StratumResult * max(n, 1))()
     loud = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
     dev = (C.c_int32 * len(devices))(*devices) if devices else None
     cfgp = C.cast(C.byref(config._c), C.c_void_p) if config is not None else None
-    st = lib().stratum_b200_analyze_loudness_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
-                                                 srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
-                                                 n, cfgp, ids.ctypes.data_as(C.POINTER(_u)) if ids is not None else None, na, dev,
-                                                 len(devices) if devices else 0, res, loud, alb)
+    st = lib().stratum_b200_analyze_loudness_mapped_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                        srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)),
+                                                        fmts.ctypes.data_as(C.POINTER(_u)), n, cfgp, ids.ctypes.data_as(C.POINTER(_u)) if ids is not None else None,
+                                                        na, _u8p(cmap), dev, len(devices) if devices else 0, res, loud, alb, chout)
     if st != OK:
         _fail(st, res, n)
-    return _collect(res, n), [_loudness(loud[i]) for i in range(n)], [_loudness(alb[a]) for a in range(na)]
+    return _collect(res, n), _with_channels([_loudness(loud[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_filters(sample_rate: int) -> tuple:

@@ -2556,6 +2556,24 @@ static void album_layout(const uint32_t* album_of, uint32_t n_albums, const uint
     }
 }
 
+// The channel side of a loudness call: the caller's channel map (null: the default map of every track) and the per-channel results
+// (null: none).  Track q's entries of both start at at[q], the channels of the tracks before it.
+struct LoudChannels {
+    const uint8_t* map = nullptr;
+    StratumLoudness* out = nullptr;
+    std::vector<uint64_t> at;
+};
+
+// Weight of a channel class (include/stratum_b200.h: StratumChannelClass); codes are checked by channels_validate.
+static double loud_class_weight(uint8_t code) {
+    switch (code) {
+        case STRATUM_CH_FRONT: return 1.0;
+        case STRATUM_CH_SURROUND: return 1.41;
+        case STRATUM_CH_DUAL_MONO: return 2.0;
+        default: return 0.0;
+    }
+}
+
 // The loudness of the staged chunks: one launch of each kernel per chunk over all its tracks, straight from the staged PCM.  Chunk
 // k's results are read back while chunk k+1 runs.
 struct LoudnessSink final : ChunkSink {
@@ -2565,6 +2583,7 @@ struct LoudnessSink final : ChunkSink {
     const uint32_t *sample_rates, *channels, *formats;
     StratumLoudness* out;
     AlbumPools* pools;  // null without albums
+    const LoudChannels& chans_;  // channel map, per-channel results
     cudaStream_t stream;  // every launch and copy of the sink; ctx->stream unless set before open()
     struct Slot {
         uint32_t i = 0, j = 0;
@@ -2572,19 +2591,19 @@ struct LoudnessSink final : ChunkSink {
         uint64_t n_seg = 0;
         std::vector<PendingStage> stages;
     } slot[2];
-    size_t rec_bytes = 0, out_bytes = 0;
     LoudnessSink(DeviceCtx* c, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans, const uint32_t* fmts,
-                 StratumLoudness* o, AlbumPools* p)
-        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p), stream(c->stream) {}
+                 StratumLoudness* o, AlbumPools* p, const LoudChannels& lc)
+        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p), chans_(lc), stream(c->stream) {}
     bool has_member(uint32_t i, uint32_t j) const {
         for (uint32_t q = i; pools && q < j; ++q)
             if (pools->member(q)) return true;
         return false;
     }
 
-    // Records of tracks [i, j) (byte offsets relative to track i) into rec (may be null); returns the work items and segments.
-    void plan(uint32_t i, uint32_t j, LoudTrack* rec, uint64_t* n_work, uint64_t* n_seg, uint32_t* max_c) const {
-        uint64_t w = 0, sg = 0;
+    // Records of tracks [i, j) (byte offsets relative to track i) into rec and their channel weights into wt (both may be null);
+    // returns the work items, segments and channels.
+    void plan(uint32_t i, uint32_t j, LoudTrack* rec, double* wt, uint64_t* n_work, uint64_t* n_seg, uint64_t* n_ch, uint32_t* max_c) const {
+        uint64_t w = 0, sg = 0, nc = 0;
         uint32_t mc = 1;
         for (uint32_t q = i; q < j; ++q) {
             const uint32_t sr = sample_rates[q], C = channels[q];
@@ -2599,6 +2618,7 @@ struct LoudnessSink final : ChunkSink {
                 T.frames = frames;
                 T.work = w;
                 T.seg0 = sg;
+                T.ch0 = nc;
                 T.C = C;
                 T.fmt = formats[q];
                 T.S = S;
@@ -2613,28 +2633,36 @@ struct LoudnessSink final : ChunkSink {
                     true_peak_taps(T.L, T.taps);
                 }
             }
+            if (wt)
+                for (uint32_t c = 0; c < C; ++c) wt[nc + c] = chans_.map ? loud_class_weight(chans_.map[chans_.at[q] + c]) : loud_channel_weight(C, c);
             w += (uint64_t)nseg * C;
             sg += nseg;
+            nc += C;
             if (ok) mc = std::max(mc, C);
         }
         *n_work = w;
         *n_seg = sg;
+        *n_ch = nc;
         *max_c = mc;
     }
 
-    size_t ws_bytes(uint64_t n_tracks, uint64_t n_work, uint64_t n_seg) const {
-        return align_up(n_tracks * sizeof(LoudTrack), 256) + align_up(n_tracks * sizeof(LoudOut), 256) + align_up(5 * n_work * sizeof(double), 256) +
-               align_up(4 * n_seg * sizeof(double), 256);
+    // Device work area of a chunk: records and weight table (uploaded together), track then per-channel results (zeroed and read
+    // back together), cascade states and energies, per-segment areas, and with per-channel results their areas.
+    static size_t rec_bytes(uint64_t n_tracks, uint64_t n_ch) { return align_up(n_tracks * sizeof(LoudTrack), 256) + n_ch * sizeof(double); }
+    size_t ws_bytes(uint64_t n_tracks, uint64_t n_work, uint64_t n_seg, uint64_t n_ch) const {
+        return align_up(rec_bytes(n_tracks, n_ch), 256) + align_up((n_tracks + n_ch) * sizeof(LoudOut), 256) + align_up(5 * n_work * sizeof(double), 256) +
+               align_up(4 * n_seg * sizeof(double), 256) + (chans_.out ? align_up(4 * n_work * sizeof(double), 256) : 0);
     }
 
     int open(const std::vector<HostChunk>& chunks) override {
-        size_t need = 0, max_n = 0, blk_bytes = 0;
+        size_t need = 0, rec_max = 0, out_max = 0, blk_bytes = 0;
         for (const HostChunk& ch : chunks) {
-            uint64_t w, sg;
+            uint64_t w, sg, nc;
             uint32_t mc;
-            plan(ch.i, ch.j, nullptr, &w, &sg, &mc);
-            need = std::max(need, ws_bytes(ch.j - ch.i, w, sg));
-            max_n = std::max<size_t>(max_n, ch.j - ch.i);
+            plan(ch.i, ch.j, nullptr, nullptr, &w, &sg, &nc, &mc);
+            need = std::max(need, ws_bytes(ch.j - ch.i, w, sg, nc));
+            rec_max = std::max(rec_max, rec_bytes(ch.j - ch.i, nc));
+            out_max = std::max<size_t>(out_max, (ch.j - ch.i + nc) * sizeof(LoudOut));
             if (has_member(ch.i, ch.j)) blk_bytes = std::max<size_t>(blk_bytes, 2 * sg * sizeof(double));
         }
         for (int b = 0; b < 2 && blk_bytes; ++b)
@@ -2642,10 +2670,8 @@ struct LoudnessSink final : ChunkSink {
                 set_error("pinned host allocation failed");
                 return STRATUM_PROCESSING_ERROR;
             }
-        rec_bytes = max_n * sizeof(LoudTrack);
-        out_bytes = max_n * sizeof(LoudOut);
         for (int b = 0; b < 2; ++b)
-            if (!ctx->loud_rec[b].need(rec_bytes) || !ctx->loud_out[b].need(out_bytes)) {
+            if (!ctx->loud_rec[b].need(rec_max) || !ctx->loud_out[b].need(out_max)) {
                 set_error("pinned host allocation failed");
                 return STRATUM_PROCESSING_ERROR;
             }
@@ -2663,24 +2689,30 @@ struct LoudnessSink final : ChunkSink {
 
     int chunk(size_t k, const HostChunk& ch, const char* d_buf, const std::function<void()>& after_prev) override {
         const uint32_t n = ch.j - ch.i;
-        LoudTrack* h_tr = static_cast<LoudTrack*>(ctx->loud_rec[k & 1].p);
+        char* h_rec = static_cast<char*>(ctx->loud_rec[k & 1].p);
+        LoudTrack* h_tr = reinterpret_cast<LoudTrack*>(h_rec);
         LoudOut* h_out = static_cast<LoudOut*>(ctx->loud_out[k & 1].p);
-        uint64_t n_work, n_seg;
+        const uint64_t wt_off = align_up((uint64_t)n * sizeof(LoudTrack), 256);
+        uint64_t n_work, n_seg, n_ch;
         uint32_t max_c;
-        plan(ch.i, ch.j, h_tr, &n_work, &n_seg, &max_c);
+        plan(ch.i, ch.j, h_tr, reinterpret_cast<double*>(h_rec + wt_off), &n_work, &n_seg, &n_ch, &max_c);
         char* d = ctx->d_loud;
         LoudTrack* d_tr = reinterpret_cast<LoudTrack*>(d);
-        d += align_up((uint64_t)n * sizeof(LoudTrack), 256);
+        const double* d_wt = reinterpret_cast<const double*>(d + wt_off);
+        d += align_up(rec_bytes(n, n_ch), 256);
         LoudOut* d_out = reinterpret_cast<LoudOut*>(d);
-        d += align_up((uint64_t)n * sizeof(LoudOut), 256);
+        LoudOut* d_chout = d_out + n;
+        d += align_up((n + n_ch) * sizeof(LoudOut), 256);
         double* d_st = reinterpret_cast<double*>(d);
         double* d_en = d_st + 4 * n_work;
         d += align_up(5 * n_work * sizeof(double), 256);
         double* d_ws = reinterpret_cast<double*>(d);
+        d += align_up(4 * n_seg * sizeof(double), 256);
+        double* d_cws = chans_.out ? reinterpret_cast<double*>(d) : nullptr;
         cudaStream_t s = stream;
-        CUDA_OK(cudaMemcpyAsync(d_tr, h_tr, (size_t)n * sizeof(LoudTrack), cudaMemcpyHostToDevice, s));
-        CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)n * sizeof(LoudOut), s));
-        g_h2d_bytes.fetch_add((uint64_t)n * sizeof(LoudTrack));
+        CUDA_OK(cudaMemcpyAsync(d_tr, h_rec, rec_bytes(n, n_ch), cudaMemcpyHostToDevice, s));
+        CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)(n + n_ch) * sizeof(LoudOut), s));
+        g_h2d_bytes.fetch_add(rec_bytes(n, n_ch));
         {
             StageTimer tm(s, "loudness_pass1");
             launch_loud_pass1(s, d_buf, d_tr, n, n_work, d_st);
@@ -2691,15 +2723,16 @@ struct LoudnessSink final : ChunkSink {
         }
         {
             StageTimer tm(s, "loudness_pass2");
-            launch_loud_pass2(s, d_buf, d_tr, n, n_work, d_st, d_en, d_out);
+            launch_loud_pass2(s, d_buf, d_tr, n, n_work, d_st, d_en, d_chout);
         }
         {
             StageTimer tm(s, "loudness_gate");
-            launch_loud_gate(s, d_tr, n, d_en, d_ws, n_seg, d_out);
+            launch_loud_gate(s, d_tr, n, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout, chans_.out ? max_c : 0);
         }
         CUDA_OK(cudaGetLastError());
-        CUDA_OK(cudaMemcpyAsync(h_out, d_out, (size_t)n * sizeof(LoudOut), cudaMemcpyDeviceToHost, s));
-        g_d2h_bytes.fetch_add((uint64_t)n * sizeof(LoudOut));
+        const uint64_t n_read = chans_.out ? n + n_ch : n;  // the per-channel results follow the track results
+        CUDA_OK(cudaMemcpyAsync(h_out, d_out, (size_t)n_read * sizeof(LoudOut), cudaMemcpyDeviceToHost, s));
+        g_d2h_bytes.fetch_add(n_read * sizeof(LoudOut));
         const bool blocks = has_member(ch.i, ch.j);
         if (blocks) {  // the momentary and short-term regions of the work area are adjacent: one copy for both
             CUDA_OK(cudaMemcpyAsync(ctx->loud_blk[k & 1].p, d_ws + n_seg, 2 * n_seg * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -2727,27 +2760,13 @@ struct LoudnessSink final : ChunkSink {
         resolve_stage_times(sl.stages);
         const LoudTrack* h_tr = static_cast<const LoudTrack*>(ctx->loud_rec[b].p);
         const LoudOut* h_out = static_cast<const LoudOut*>(ctx->loud_out[b].p);
+        const uint32_t n = sl.j - sl.i;
         for (uint32_t q = sl.i; q < sl.j; ++q) {
             const LoudTrack& T = h_tr[q - sl.i];
-            const LoudOut& o = h_out[q - sl.i];
-            StratumLoudness& r = out[q];
-            memset(&r, 0, sizeof r);
-            r.sample_rate = sample_rates[q];
-            r.channels = channels[q];
-            r.frames = T.frames;
-            r.status = loud_track_status(r.sample_rate, r.frames, r.error, sizeof r.error);
-            if (r.status != STRATUM_OK) continue;
-            r.integrated_lufs = o.integrated;
-            r.momentary_max_lufs = o.momentary_max;
-            r.short_term_max_lufs = o.short_term_max;
-            r.loudness_range_lu = o.loudness_range;
-            float f;
-            memcpy(&f, &o.sample_peak_bits, sizeof f);
-            r.sample_peak = f;
-            memcpy(&f, &o.true_peak_bits, sizeof f);
-            r.true_peak = f;
-            r.n_momentary = T.J;
-            r.n_short_term = T.K;
+            loud_result(T, h_out[q - sl.i], sample_rates[q], channels[q], out[q]);
+            if (chans_.out)
+                for (uint32_t c = 0; c < T.C; ++c) loud_result(T, h_out[n + T.ch0 + c], sample_rates[q], 1, chans_.out[chans_.at[q] + c]);
+            if (out[q].status != STRATUM_OK) continue;
             if (sl.blocks && pools->member(q)) {
                 const double* blk = static_cast<const double*>(ctx->loud_blk[b].p);
                 memcpy(pools->buf.data() + pools->m_at[q], blk + T.seg0, (size_t)T.J * sizeof(double));
@@ -2755,6 +2774,26 @@ struct LoudnessSink final : ChunkSink {
             }
         }
         return STRATUM_OK;
+    }
+
+    static void loud_result(const LoudTrack& T, const LoudOut& o, uint32_t sr, uint32_t C, StratumLoudness& r) {
+        memset(&r, 0, sizeof r);
+        r.sample_rate = sr;
+        r.channels = C;
+        r.frames = T.frames;
+        r.status = loud_track_status(r.sample_rate, r.frames, r.error, sizeof r.error);
+        if (r.status != STRATUM_OK) return;
+        r.integrated_lufs = o.integrated;
+        r.momentary_max_lufs = o.momentary_max;
+        r.short_term_max_lufs = o.short_term_max;
+        r.loudness_range_lu = o.loudness_range;
+        float f;
+        memcpy(&f, &o.sample_peak_bits, sizeof f);
+        r.sample_peak = f;
+        memcpy(&f, &o.true_peak_bits, sizeof f);
+        r.true_peak = f;
+        r.n_momentary = T.J;
+        r.n_short_term = T.K;
     }
 
     int close() override {
@@ -2771,6 +2810,50 @@ static int32_t loudness_validate(const uint64_t* boff, const uint32_t* sample_ra
     }
     bpf.assign(n_tracks, 1);
     return pcm_frame_bytes(boff, channels, formats, n_tracks, bpf);
+}
+
+// Channel classes: every code of the map a StratumChannelClass.  Runs after every other check of the call.
+static int32_t channels_validate(const uint8_t* map, StratumLoudness* channel_out, const uint32_t* channels, uint32_t n_tracks, LoudChannels& lc) {
+    lc.map = map;
+    lc.out = channel_out;
+    lc.at.assign(n_tracks + 1, 0);
+    for (uint32_t q = 0; q < n_tracks; ++q) lc.at[q + 1] = lc.at[q] + channels[q];
+    for (uint32_t q = 0; map && q < n_tracks; ++q)
+        for (uint32_t c = 0; c < channels[q]; ++c)
+            if (map[lc.at[q] + c] > STRATUM_CH_DUAL_MONO) {
+                set_error("track " + std::to_string(q) + " channel " + std::to_string(c) + ": channel class " + std::to_string(map[lc.at[q] + c]) +
+                          " is not one of STRATUM_CH_UNUSED (0) .. STRATUM_CH_DUAL_MONO (3)");
+                return STRATUM_INVALID_INPUT;
+            }
+    return STRATUM_OK;
+}
+
+int32_t stratum_b200_loudness_channel_map(uint32_t wave_mask, uint32_t channels, int32_t dual_mono, uint8_t* map) {
+    if (!map || channels < 1 || channels > 64) {
+        set_error(!map ? "null argument" : "channels outside 1..64");
+        return STRATUM_INVALID_INPUT;
+    }
+    const uint32_t side = 0x200u | 0x400u;  // SPEAKER_SIDE_LEFT, SPEAKER_SIDE_RIGHT
+    uint32_t bits = wave_mask;
+    for (uint32_t c = 0; c < channels; ++c) {
+        uint8_t code;
+        if (wave_mask == 0) {  // the default map of the channel count
+            const double w = loud_channel_weight(channels, c);
+            code = w == 0.0 ? STRATUM_CH_UNUSED : (w == 1.0 ? STRATUM_CH_FRONT : STRATUM_CH_SURROUND);
+        } else if (bits == 0) {
+            code = STRATUM_CH_UNUSED;  // beyond the set bits
+        } else {
+            const uint32_t bit = bits & (~bits + 1u);  // the lowest set bit left
+            bits &= bits - 1u;
+            if (bit == 0x8u || bit > 0x20000u) code = STRATUM_CH_UNUSED;  // SPEAKER_LOW_FREQUENCY; reserved bits and SPEAKER_ALL
+            else if (bit & side) code = STRATUM_CH_SURROUND;
+            else if (bit == 0x10u || bit == 0x20u) code = (wave_mask & side) ? STRATUM_CH_FRONT : STRATUM_CH_SURROUND;  // BACK_LEFT / RIGHT
+            else code = STRATUM_CH_FRONT;
+        }
+        map[c] = code;
+    }
+    if (dual_mono && channels == 1 && map[0] != STRATUM_CH_UNUSED) map[0] = STRATUM_CH_DUAL_MONO;
+    return STRATUM_OK;
 }
 
 // Album ids: each below n_albums or STRATUM_NO_ALBUM.
@@ -2865,30 +2948,36 @@ static int32_t album_phase(int32_t device, AlbumPools& P, uint32_t n_tracks, con
     return STRATUM_OK;
 }
 
-int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+int32_t stratum_b200_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                          const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
-                                         const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out, StratumLoudness* album_out) {
+                                         const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out,
+                                         StratumLoudness* album_out, StratumLoudness* channel_out) {
     std::vector<uint32_t> bpf;
+    LoudChannels lc;
     int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
+    if (st == STRATUM_OK) st = channels_validate(channel_map, channel_out, channels, n_tracks, lc);
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
     AlbumPools* pp = n_albums ? &pools : nullptr;
     if (n_tracks)
         st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
-            return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, pp));
+            return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, pp, lc));
         });
     if (st != STRATUM_OK || n_albums == 0) return st;
     return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, out, album_out);
 }
 
-int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                 const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
-                                                int32_t device_id, StratumLoudness* out, StratumLoudness* album_out) {
+                                                const uint8_t* channel_map, int32_t device_id, StratumLoudness* out, StratumLoudness* album_out,
+                                                StratumLoudness* channel_out) {
     std::vector<uint32_t> bpf;
+    LoudChannels lc;
     int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, d_pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
+    if (st == STRATUM_OK) st = channels_validate(channel_map, channel_out, channels, n_tracks, lc);
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
@@ -2902,7 +2991,7 @@ int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_
         }
         // the whole batch is one chunk: one launch of each kernel
         const std::vector<HostChunk> one{HostChunk{0, n_tracks, byte_offsets[n_tracks] - byte_offsets[0], 0}};
-        LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, n_albums ? &pools : nullptr);
+        LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, n_albums ? &pools : nullptr, lc);
         st = sink.open(one);
         if (st != STRATUM_OK) return st;
         const int s1 = sink.chunk(0, one[0], static_cast<const char*>(d_pcm) + byte_offsets[0], [] {});
@@ -2913,14 +3002,30 @@ int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_
     return album_phase(device_id, pools, n_tracks, out, album_out);
 }
 
+int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out, StratumLoudness* album_out) {
+    return stratum_b200_loudness_mapped_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, album_of_track, n_albums, nullptr, device_ids,
+                                            n_devices, out, album_out, nullptr);
+}
+
+int32_t stratum_b200_loudness_albums_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                int32_t device_id, StratumLoudness* out, StratumLoudness* album_out) {
+    return stratum_b200_loudness_mapped_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, album_of_track, n_albums, nullptr,
+                                                   device_id, out, album_out, nullptr);
+}
+
 int32_t stratum_b200_loudness_batch_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                         const uint32_t* formats, uint32_t n_tracks, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out) {
-    return stratum_b200_loudness_albums_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, device_ids, n_devices, out, nullptr);
+    return stratum_b200_loudness_mapped_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, nullptr, device_ids, n_devices, out,
+                                            nullptr, nullptr);
 }
 
 int32_t stratum_b200_loudness_batch_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                const uint32_t* formats, uint32_t n_tracks, int32_t device_id, StratumLoudness* out) {
-    return stratum_b200_loudness_albums_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, device_id, out, nullptr);
+    return stratum_b200_loudness_mapped_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, nullptr, 0, nullptr, device_id, out,
+                                                   nullptr, nullptr);
 }
 
 // Analysis and loudness of the same staged chunks: one upload feeds both.  The loudness passes of a chunk are queued first, on a
@@ -2932,8 +3037,8 @@ struct AnalysisLoudnessSink final : ChunkSink {
     AnalysisSink ana;
     LoudnessSink loud;
     AnalysisLoudnessSink(DeviceCtx* c, const StratumConfig& cfg, const uint64_t* offs, const std::vector<uint32_t>& bpf, const uint32_t* srs,
-                         const uint32_t* chans, const uint32_t* fmts, StratumResult* o, StratumLoudness* lo, AlbumPools* p)
-        : ana(c, cfg, offs, bpf, srs, chans, fmts, o), loud(c, offs, bpf, srs, chans, fmts, lo, p) {}
+                         const uint32_t* chans, const uint32_t* fmts, StratumResult* o, StratumLoudness* lo, AlbumPools* p, const LoudChannels& lc)
+        : ana(c, cfg, offs, bpf, srs, chans, fmts, o), loud(c, offs, bpf, srs, chans, fmts, lo, p, lc) {}
 
     int open(const std::vector<HostChunk>& chunks) override {
         DeviceCtx* ctx = ana.ctx;
@@ -2963,11 +3068,12 @@ struct AnalysisLoudnessSink final : ChunkSink {
     }
 };
 
-int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
-                                          const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
-                                          uint32_t n_albums, const int32_t* device_ids, uint32_t n_devices, StratumResult* out,
-                                          StratumLoudness* loudness_out, StratumLoudness* album_out) {
-    // the order of stratum_b200_analyze_batch_pcm: NULL pointers, the configuration, the PCM layout; then the album ids
+int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                 const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                                 uint32_t n_albums, const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices,
+                                                 StratumResult* out, StratumLoudness* loudness_out, StratumLoudness* album_out,
+                                                 StratumLoudness* channel_out) {
+    // the order of stratum_b200_analyze_batch_pcm: NULL pointers, the configuration, the PCM layout; then the album ids, the channel map
     if (!byte_offsets || !sample_rates || !channels || !formats || !out || !loudness_out || (!pcm && n_tracks && byte_offsets[n_tracks] > 0)) {
         set_error("null argument");
         return STRATUM_INVALID_INPUT;
@@ -2976,19 +3082,30 @@ int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_
     config_default(&def);
     const StratumConfig& c = cfg ? *cfg : def;
     std::vector<uint32_t> bpf;
+    LoudChannels lc;
     int st = config_validate(c);
     if (st == STRATUM_OK) st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, loudness_out, pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
+    if (st == STRATUM_OK) st = channels_validate(channel_map, channel_out, channels, n_tracks, lc);
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
     AlbumPools* pp = n_albums ? &pools : nullptr;
     if (n_tracks)
         st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
-            return std::unique_ptr<ChunkSink>(new AnalysisLoudnessSink(ctx, c, byte_offsets, bpf, sample_rates, channels, formats, out, loudness_out, pp));
+            return std::unique_ptr<ChunkSink>(
+                new AnalysisLoudnessSink(ctx, c, byte_offsets, bpf, sample_rates, channels, formats, out, loudness_out, pp, lc));
         });
     if (st != STRATUM_OK || n_albums == 0) return st;
     return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, loudness_out, album_out);
+}
+
+int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                          const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                          uint32_t n_albums, const int32_t* device_ids, uint32_t n_devices, StratumResult* out,
+                                          StratumLoudness* loudness_out, StratumLoudness* album_out) {
+    return stratum_b200_analyze_loudness_mapped_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, cfg, album_of_track, n_albums, nullptr,
+                                                    device_ids, n_devices, out, loudness_out, album_out, nullptr);
 }
 
 int32_t stratum_b200_debug_loudness_filters(uint32_t sample_rate, double* kweight10, float* taps49) {

@@ -6,10 +6,13 @@
 //   scan    one CTA per (track, channel) turns the end states into the true start state of every segment
 //           (s[k+1] = M s[k] + e[k], M = A^S computed on the host);
 //   pass 2  each work item re-runs its segment from its start state and writes its sum of y^2; on the same samples it keeps the
-//           sample peak and the 4x / 2x oversampled true peak (49-tap interpolator, 12 / 24 frames of context), reduced per track
-//           by atomicMax on the bit pattern;
-//   gate    one CTA per track: channel-weighted sub-block energies, momentary / short-term powers as in-order sums of 4 / 30
-//           sub-blocks, the absolute and relative gates, the maxima and the loudness range (exact order statistics);
+//           sample peak and the 4x / 2x oversampled true peak (49-tap interpolator, 12 / 24 frames of context), reduced per
+//           (track, channel) by atomicMax on the bit pattern;
+//   gate    one CTA per track: sub-block energies weighted by the track's channel weights (a per-launch table built on the host
+//           from the caller's channel map or the default map), momentary / short-term powers as in-order sums of 4 / 30
+//           sub-blocks, the absolute and relative gates, the maxima and the loudness range (exact order statistics), and the
+//           track peaks as the maxima over its channels; on request one more CTA per (track, channel) gates that channel alone
+//           (stratum_b200_loudness_mapped_pcm: channel_out);
 //   album   one CTA per album: the same gates, maxima and range over the members' momentary / short-term powers, pooled on the
 //           host in ascending track order (stratum_b200_loudness_albums_pcm).
 // The recurrence runs in f64: at 192 kHz the high-pass pole of stage 2 lies 1.2e-3 from the unit circle, and f32 coefficients
@@ -193,14 +196,18 @@ __device__ __forceinline__ void loud_pass2_item(const LoudTrack& T, const unsign
 }
 
 __global__ void __launch_bounds__(256) loud_pass2_kernel(const unsigned char* __restrict__ pcm, const LoudTrack* __restrict__ tr, uint32_t n_tracks,
-                                                         uint64_t n_work, const double* __restrict__ st, double* __restrict__ en, LoudOut* __restrict__ out) {
+                                                         uint64_t n_work, const double* __restrict__ st, double* __restrict__ en, LoudOut* __restrict__ chout) {
     const uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool valid = w < n_work;
     const uint32_t t = valid ? loud_track_of(tr, n_tracks, w) : 0xffffffffu;
     float spk = 0.0f, tpk = 0.0f;
+    uint32_t C = 0;
+    uint64_t slot = 0;  // (track, channel) entry of chout
     if (valid) {
         const LoudTrack& T = tr[t];
         const uint32_t r = (uint32_t)(w - T.work), seg = r / T.C, ch = r % T.C;
+        C = T.C;
+        slot = T.ch0 + ch;
         const uint64_t a = (uint64_t)seg * T.S, b = min(a + T.S, T.frames);
         const bool energy = seg < T.nfull;
         double k[10];
@@ -219,18 +226,20 @@ __global__ void __launch_bounds__(256) loud_pass2_kernel(const unsigned char* __
         if (energy) en[w] = sum;
     }
     tpk = fmaxf(tpk, spk);
-    // one atomic per warp when the warp lies inside one track (the common case), else one per lane
+    // Work items are channel-minor, so lanes l and l ^ o hold the same channel whenever C divides o.  When the warp lies inside one
+    // track (the common case) and C is a power of two dividing 32, xor-shuffles over o = 16 .. C leave lane c < C with its channel's
+    // maximum over the warp and those C lanes issue the atomics; otherwise every lane issues its own.
     const uint32_t t0 = __shfl_sync(0xffffffffu, t, 0);
-    if (__all_sync(0xffffffffu, t == t0)) {
-        for (int o = 16; o > 0; o >>= 1) {
+    if (__all_sync(0xffffffffu, t == t0) && valid && (C & (C - 1)) == 0 && C <= 32) {  // t uniform: valid and C uniform too
+        for (uint32_t o = 16; o >= C; o >>= 1) {
             spk = fmaxf(spk, __shfl_xor_sync(0xffffffffu, spk, o));
             tpk = fmaxf(tpk, __shfl_xor_sync(0xffffffffu, tpk, o));
         }
-        if ((threadIdx.x & 31) != 0) return;
+        if ((threadIdx.x & 31) >= C) return;
     }
     if (valid) {  // values >= 0: bit order == value order
-        atomicMax(&out[t].sample_peak_bits, __float_as_uint(spk));
-        atomicMax(&out[t].true_peak_bits, __float_as_uint(tpk));
+        atomicMax(&chout[slot].sample_peak_bits, __float_as_uint(spk));
+        atomicMax(&chout[slot].true_peak_bits, __float_as_uint(tpk));
     }
 }
 
@@ -338,18 +347,16 @@ __device__ __forceinline__ void loud_gate_lists(const double* __restrict__ m, ui
     }
 }
 
-__global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const LoudTrack* __restrict__ tr, const double* __restrict__ en, double* __restrict__ zs,
-                                                                      double* __restrict__ mom, double* __restrict__ sht, double* __restrict__ keep,
-                                                                      LoudOut* __restrict__ out) {
-    const LoudTrack& T = tr[blockIdx.x];
-    if (T.nseg == 0) return;
+// Track T's channels [c0, c0 + nc) weighted by w[c] (w null: the single channel at weight 1.0, the table entry of a one-channel
+// track, so a channel gated alone reproduces the bits of a one-channel track of its samples): sub-block energies into z, momentary
+// and short-term powers into m and q, then the gates into o.
+__device__ __forceinline__ void loud_gate_track(const LoudTrack& T, const double* __restrict__ w, uint32_t c0, uint32_t nc, const double* __restrict__ en,
+                                                double* __restrict__ z, double* __restrict__ m, double* __restrict__ q, double* __restrict__ kp,
+                                                LoudOut* __restrict__ o) {
     const uint32_t C = T.C, nfull = T.nfull, J = T.J, K = T.K;
-    double* z = zs + T.seg0;
-    double* m = mom + T.seg0;
-    double* q = sht + T.seg0;
     for (uint32_t i = threadIdx.x; i < nfull; i += LOUD_GATE_THREADS) {
         double acc = 0.0;
-        for (uint32_t c = 0; c < C; ++c) acc = acc + loud_channel_weight(C, c) * en[T.work + (uint64_t)i * C + c];
+        for (uint32_t c = c0; c < c0 + nc; ++c) acc = acc + (w ? w[c] : 1.0) * en[T.work + (uint64_t)i * C + c];
         z[i] = acc;
     }
     __syncthreads();
@@ -361,7 +368,34 @@ __global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const Loud
         q[j] = acc / ds;
     }
     __syncthreads();
-    loud_gate_lists(m, J, q, K, keep + T.seg0, out + blockIdx.x);
+    loud_gate_lists(m, J, q, K, kp, o);
+}
+
+// blockIdx.y = 0: track blockIdx.x over its weighted channels, and its peaks as the maxima over its channels' peaks; blockIdx.y =
+// 1 + c: channel c of the track alone (per-channel results).
+__global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const LoudTrack* __restrict__ tr, const double* __restrict__ wt, const double* __restrict__ en,
+                                                                      double* __restrict__ ws, uint64_t n_seg, LoudOut* __restrict__ out, double* __restrict__ cws,
+                                                                      uint64_t n_work, LoudOut* __restrict__ chout) {
+    const LoudTrack& T = tr[blockIdx.x];
+    if (T.nseg == 0) return;
+    if (blockIdx.y == 0) {
+        if (threadIdx.x == 0) {
+            uint32_t sp = 0, tp = 0;
+            for (uint32_t c = 0; c < T.C; ++c) {
+                sp = max(sp, chout[T.ch0 + c].sample_peak_bits);
+                tp = max(tp, chout[T.ch0 + c].true_peak_bits);
+            }
+            out[blockIdx.x].sample_peak_bits = sp;
+            out[blockIdx.x].true_peak_bits = tp;
+        }
+        double* z = ws + T.seg0;
+        loud_gate_track(T, wt + T.ch0, 0, T.C, en, z, z + n_seg, z + 2 * n_seg, z + 3 * n_seg, out + blockIdx.x);
+        return;
+    }
+    const uint32_t c = blockIdx.y - 1;
+    if (c >= T.C) return;
+    double* z = cws + T.work + (uint64_t)c * T.nseg;
+    loud_gate_track(T, nullptr, c, 1, en, z, z + n_work, z + 2 * n_work, z + 3 * n_work, chout + T.ch0 + c);
 }
 
 // One CTA per album over its pooled lists.
@@ -385,15 +419,16 @@ void launch_loud_scan(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, 
 }
 
 void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, const double* d_st, double* d_en,
-                       LoudOut* d_out) {
+                       LoudOut* d_chout) {
     if (n_work == 0) return;
-    loud_pass2_kernel<<<(unsigned)((n_work + 255) / 256), 256, 0, s>>>(static_cast<const unsigned char*>(d_pcm), d_tr, n_tracks, n_work, d_st, d_en, d_out);
+    loud_pass2_kernel<<<(unsigned)((n_work + 255) / 256), 256, 0, s>>>(static_cast<const unsigned char*>(d_pcm), d_tr, n_tracks, n_work, d_st, d_en, d_chout);
     count_launch("loudness");
 }
 
-void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_en, double* d_ws, uint64_t n_seg, LoudOut* d_out) {
+void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_wt, const double* d_en, double* d_ws, uint64_t n_seg,
+                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks) {
     if (n_tracks == 0) return;
-    loud_gate_kernel<<<n_tracks, LOUD_GATE_THREADS, 0, s>>>(d_tr, d_en, d_ws, d_ws + n_seg, d_ws + 2 * n_seg, d_ws + 3 * n_seg, d_out);
+    loud_gate_kernel<<<dim3(n_tracks, 1 + ch_blocks), LOUD_GATE_THREADS, 0, s>>>(d_tr, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout);
     count_launch("loudness");
 }
 

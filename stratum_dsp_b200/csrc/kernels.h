@@ -209,6 +209,7 @@ struct LoudTrack {
     uint64_t frames;
     uint64_t work;         // first work item (segment-major (segment, channel) pairs of the earlier tracks)
     uint64_t seg0;         // first entry in the per-segment work areas (segments of the earlier tracks)
+    uint64_t ch0;          // first entry in the per-channel tables (weights, per-channel results): channels of the earlier tracks
     uint32_t C, fmt;       // channels, STRATUM_PCM_*
     uint32_t S, L;         // sub-block frames (sr + 5) / 10, true-peak oversampling factor
     uint32_t nseg, nfull;  // segments covering the track (0: the track failed and is skipped), whole sub-blocks floor(frames / S)
@@ -222,8 +223,9 @@ struct LoudOut {
     uint32_t sample_peak_bits, true_peak_bits;  // non-negative floats, reduced by atomicMax on the bits
 };
 // libebur128's default channel map: 1 channel L; 4 channels L R Ls Rs; 5 channels L R C Ls Rs; otherwise L R C LFE Ls Rs and unused
-// channels from 6 on.  L, R, C weigh 1, Ls and Rs 1.41, LFE and unused channels 0.
-__host__ __device__ inline double loud_channel_weight(uint32_t C, uint32_t c) {
+// channels from 6 on.  L, R, C weigh 1, Ls and Rs 1.41, LFE and unused channels 0.  The host fills the weight table of a track
+// without a channel map from it (engine.cu: loud_weights).
+inline double loud_channel_weight(uint32_t C, uint32_t c) {
     if (C == 4) return c < 2 ? 1.0 : 1.41;
     if (C == 5) return c < 3 ? 1.0 : 1.41;
     if (c < 3) return 1.0;
@@ -231,10 +233,15 @@ __host__ __device__ inline double loud_channel_weight(uint32_t C, uint32_t c) {
 }
 void launch_loud_pass1(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, double* d_st);
 void launch_loud_scan(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, uint32_t max_channels, double* d_st);
+// Sample and true peaks per (track, channel) into d_chout[T.ch0 + c] (zeroed by the caller); the gate derives the track peaks.
 void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, const double* d_st, double* d_en,
-                       LoudOut* d_out);
-// d_ws: 4 x n_seg doubles (sub-block, momentary and short-term powers, the compacted short-term powers of the loudness range)
-void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_en, double* d_ws, uint64_t n_seg, LoudOut* d_out);
+                       LoudOut* d_chout);
+// d_wt: channel weights, track T's at d_wt[T.ch0 ..).  d_ws: 4 x n_seg doubles (sub-block, momentary and short-term powers, the
+// compacted short-term powers of the loudness range).  With ch_blocks > 0 (the largest channel count of the launch) the launch adds
+// one CTA per (track, channel) that gates the channel alone into d_chout[T.ch0 + c], over d_cws: 4 x n_work doubles laid out like
+// d_ws, channel c of track T at T.work + c * T.nseg.
+void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_wt, const double* d_en, double* d_ws, uint64_t n_seg,
+                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks);
 // One record per album: its pooled momentary powers are mom[m0 .. m0 + J), its short-term powers sht[q0 .. q0 + K) (engine.cu:
 // AlbumPools).  d_keep has the size of d_sht; only the loudness fields of d_out are written.
 struct LoudAlbum {

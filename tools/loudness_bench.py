@@ -2,6 +2,8 @@
 """Throughput of the loudness measurement (stratum_b200_loudness_batch_pcm) on one GPU.
 
     python tools/loudness_bench.py [--tracks N] [--rounds R] [--warmup W] [--albums [M]] [--with-analysis] [--devices D] [--out FILE]
+    python tools/loudness_bench.py --layout [--tracks N] [--rounds R] [--warmup W] [--out FILE]
+    python tools/loudness_bench.py --baseline-lib LIB [--tracks N] [--rounds R] [--warmup W] [--out FILE]
 
 Workload: N (default 1024) stereo three-minute 44.1 kHz PCM16 tracks, each channel a C2 track of tests/synth.py (channel 0 from
 seed i, channel 1 from seed i + 1000), generated on the device and quantised there.  Two legs (three with --albums), timed in
@@ -18,6 +20,14 @@ With --with-analysis four more legs over the same pinned bytes, run with stage t
 Each reports tracks/s, wall time and the host-to-device bytes of one call; one more combined call with stage timing on gives the
 loudness kernel times inside it and the analysis stage total beside them.  --devices D runs every host leg over devices 0..D-1 from
 this process (the device leg stays on device 0).
+--layout measures channel maps instead, on N (default 256) 7.1 three-minute 44.1 kHz PCM16 tracks (about 32 GB; channel c of track i
+the C2 track i + 1000 c): three kinds, each device-resident and from pinned host memory, six legs timed in alternation:
+  default      no channel map (the default map weighs the 7.1 rear pair as Ls Rs and the side pair 0);
+  mapped       the 7.1 map of stratum_b200_loudness_channel_map(0x63F, 8, 0, map) (stratum_b200_loudness_mapped_pcm);
+  per_channel  the same map plus per-channel results (the per-channel CTAs of the gate launch and their read-back).
+Each leg reports tracks/s, wall time, the median pass 2 and gate kernel times and the device-to-host bytes of one call.
+--baseline-lib LIB times the stereo device leg of this build against another build of the library (e.g. the parent commit's), the
+two alternating, and reports each one's median, minimum and maximum pass 2 time and whether the two give the same bits.
 Reports the median over R rounds of tracks/s and wall time per leg, the median kernel times of the device leg (pass 1, the scan,
 pass 2 with the true-peak FIR, the gate), the album gate's kernel time and the device-to-host bytes the album leg adds to the host
 leg (stratum_b200_transfer_bytes), the host-to-device rate of a plain 4 GB pinned copy measured in the same run, and the card's name
@@ -56,45 +66,168 @@ def card() -> dict:
     return out
 
 
-def make_pcm(S, torch, n_tracks: int):
-    """int16 (n_tracks * N_FRAMES * 2) on the device: interleaved stereo, channel c of track i = C2 track i + 1000 c."""
+def make_pcm(S, torch, n_tracks: int, C: int = 2):
+    """int16 (n_tracks * N_FRAMES * C) on the device: interleaved, channel c of track i = C2 track i + 1000 c."""
     import synth
 
-    pcm = torch.empty(n_tracks * N_FRAMES * 2, dtype=torch.int16, device="cuda")
-    group = 32
-    tmp = torch.empty(2 * group * N_FRAMES, dtype=torch.float32, device="cuda")
+    pcm = torch.empty(n_tracks * N_FRAMES * C, dtype=torch.int16, device="cuda")
+    group = 32 if C <= 2 else 8
+    tmp = torch.empty(C * group * N_FRAMES, dtype=torch.float32, device="cuda")
     for g0 in range(0, n_tracks, group):
         n = min(group, n_tracks - g0)
         rows = []
-        for c in range(2):
+        for c in range(C):
             for i in range(g0, g0 + n):
                 p = synth.c2_params(i + 1000 * c, N_FRAMES, SR)
                 rows.append([p.bpm, p.tonic, p.minor, p.phase_frac, p.chord_amp])
-        S.synth_batch(tmp.data_ptr(), 2 * n, N_FRAMES, SR, np.asarray(rows, np.float32), 0)
-        x = tmp[: 2 * n * N_FRAMES].view(2, n, N_FRAMES).permute(1, 2, 0)  # (track, frame, channel)
+        S.synth_batch(tmp.data_ptr(), C * n, N_FRAMES, SR, np.asarray(rows, np.float32), 0)
+        x = tmp[: C * n * N_FRAMES].view(C, n, N_FRAMES).permute(1, 2, 0)  # (track, frame, channel)
         q = torch.clamp(torch.round(x * 32768.0), -32768, 32767).to(torch.int16)
-        pcm[g0 * N_FRAMES * 2:(g0 + n) * N_FRAMES * 2] = q.reshape(-1)
+        pcm[g0 * N_FRAMES * C:(g0 + n) * N_FRAMES * C] = q.reshape(-1)
     del tmp
     torch.cuda.synchronize()
     return pcm
 
 
+def lib_stage_times(L) -> dict:
+    """Stage times of library handle L since its last reset (S.stage_times for another build of the library)."""
+    names = C.create_string_buffer(4096)
+    ms = (C.c_double * 64)()
+    n = L.stratum_b200_stage_times(names, 4096, ms, 64)
+    return {nm: ms[i] for i, nm in enumerate([s for s in names.value.decode().split("\n") if s][:n])}
+
+
+def layout_main(a, S, torch) -> dict:
+    n = a.tracks
+    L = S.lib()
+    d_pcm = make_pcm(S, torch, n, 8)
+    h_pcm = torch.empty(d_pcm.numel(), dtype=torch.int16, pin_memory=True)
+    h_pcm.copy_(d_pcm)
+    bytes_per_track = N_FRAMES * 8 * 2
+    offsets = (np.arange(n + 1, dtype=np.uint64) * np.uint64(bytes_per_track))
+    srs, chans, fmts = np.full(n, SR, np.uint32), np.full(n, 8, np.uint32), np.full(n, S.PCM_S16, np.uint32)
+    u32 = lambda v: v.ctypes.data_as(C.POINTER(C.c_uint32))
+    off = offsets.ctypes.data_as(C.POINTER(C.c_uint64))
+    cmap = np.ascontiguousarray(np.tile(np.asarray(S.channel_map(0x63F, 8), np.uint8), n))
+    mp = cmap.ctypes.data_as(C.POINTER(C.c_uint8))
+    res = (S.StratumLoudness * n)()
+    chout = (S.StratumLoudness * (8 * n))()
+    kinds = {"default": (None, None), "mapped": (mp, None), "per_channel": (mp, chout)}
+
+    def leg(kind, where):
+        m, co = kinds[kind]
+        if where == "device":
+            return lambda: L.stratum_b200_loudness_mapped_pcm_device(C.c_void_p(d_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, None, 0, m, 0,
+                                                                     res, None, co)
+        return lambda: L.stratum_b200_loudness_mapped_pcm(C.c_void_p(h_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, None, 0, m, None, 0, res,
+                                                          None, co)
+
+    legs = {(k, w): leg(k, w) for k in kinds for w in ("device", "host")}
+
+    def timed(fn):
+        S.stage_timing(True)
+        S.stage_times(reset=True)
+        _, d2h0 = S.transfer_bytes()
+        t0 = time.perf_counter()
+        st = fn()
+        wall = time.perf_counter() - t0
+        S.stage_timing(False)
+        if st != S.OK:
+            raise SystemExit(f"loudness call failed: {S.last_error()}")
+        _, d2h1 = S.transfer_bytes()
+        return wall, S.stage_times(), sum(1 for i in range(n) if res[i].status == 0), d2h1 - d2h0, res[0].integrated_lufs
+
+    for _ in range(a.warmup):
+        for fn in legs.values():
+            timed(fn)
+    runs = {key: [] for key in legs}
+    for _ in range(a.rounds):
+        for key, fn in legs.items():
+            runs[key].append(timed(fn))
+    doc = {"workload": f"{n} 7.1 (8-channel) 3-minute 44.1 kHz PCM16 tracks (synthetic C2 tracks per channel)", "card": card(), "rounds": a.rounds,
+           "warmup": a.warmup, "pcm_bytes": n * bytes_per_track, "map": S.channel_map(0x63F, 8)}
+    for (kind, where), rs in runs.items():
+        wall = statistics.median(r[0] for r in rs)
+        doc[f"{kind}_{where}"] = {"tracks_per_s": n / wall, "wall_s": wall,
+                                  "stage_ms": {s: statistics.median(r[1].get(s, 0.0) for r in rs) for s in STAGES},
+                                  "d2h_bytes": statistics.median(r[3] for r in rs), "ok_tracks": min(r[2] for r in rs), "track0_integrated_lufs": rs[-1][4]}
+    return doc
+
+
+def baseline_main(a, S, torch) -> dict:
+    """The stereo device leg of this build and of the library at a.baseline_lib, alternating."""
+    n = a.tracks
+    L = S.lib()
+    B = C.CDLL(str(Path(a.baseline_lib).resolve()))
+    B.stratum_b200_loudness_batch_pcm_device.argtypes = L.stratum_b200_loudness_batch_pcm_device.argtypes
+    B.stratum_b200_loudness_batch_pcm_device.restype = C.c_int32
+    B.stratum_b200_stage_times.argtypes = [C.c_char_p, C.c_size_t, C.POINTER(C.c_double), C.c_int32]
+    B.stratum_b200_stage_times.restype = C.c_int32
+    B.stratum_b200_stage_timing_enable.argtypes = [C.c_int32]
+    d_pcm = make_pcm(S, torch, n)
+    offsets = (np.arange(n + 1, dtype=np.uint64) * np.uint64(N_FRAMES * 2 * 2))
+    srs, chans, fmts = np.full(n, SR, np.uint32), np.full(n, 2, np.uint32), np.full(n, S.PCM_S16, np.uint32)
+    u32 = lambda v: v.ctypes.data_as(C.POINTER(C.c_uint32))
+    off = offsets.ctypes.data_as(C.POINTER(C.c_uint64))
+    out = {"this": (S.StratumLoudness * n)(), "baseline": (S.StratumLoudness * n)()}
+    libs = {"this": L, "baseline": B}
+
+    def timed(key):
+        lb = libs[key]
+        lb.stratum_b200_stage_timing_enable(1)
+        lb.stratum_b200_stage_times_reset()
+        t0 = time.perf_counter()
+        st = lb.stratum_b200_loudness_batch_pcm_device(C.c_void_p(d_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, 0, out[key])
+        wall = time.perf_counter() - t0
+        lb.stratum_b200_stage_timing_enable(0)
+        if st != S.OK:
+            raise SystemExit(f"{key}: loudness call failed")
+        return wall, lib_stage_times(lb)
+
+    for _ in range(a.warmup):
+        for key in libs:
+            timed(key)
+    runs = {key: [] for key in libs}
+    for _ in range(a.rounds):
+        for key in libs:
+            runs[key].append(timed(key))
+    same = C.string_at(C.addressof(out["this"]), C.sizeof(out["this"])) == C.string_at(C.addressof(out["baseline"]), C.sizeof(out["baseline"]))
+    doc = {"workload": f"{n} stereo 3-minute 44.1 kHz PCM16 tracks (synthetic C2 pairs), device-resident", "card": card(), "rounds": a.rounds,
+           "warmup": a.warmup, "baseline_lib": Path(a.baseline_lib).name, "results_bit_identical": same}
+    for key, rs in runs.items():
+        p2 = [r[1].get("loudness_pass2", 0.0) for r in rs]
+        doc[key] = {"wall_s": statistics.median(r[0] for r in rs), "pass2_ms": {"median": statistics.median(p2), "min": min(p2), "max": max(p2)},
+                    "stage_ms": {s: statistics.median(r[1].get(s, 0.0) for r in rs) for s in STAGES}}
+    return doc
+
+
 def main() -> None:
     ap = argparse.ArgumentParser()
-    ap.add_argument("--tracks", type=int, default=1024)
+    ap.add_argument("--tracks", type=int, default=None, help="default 1024 (256 with --layout)")
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--warmup", type=int, default=1)
     ap.add_argument("--albums", type=int, nargs="?", const=12, default=None, metavar="M", help="add the album leg, M tracks per album")
     ap.add_argument("--with-analysis", action="store_true", help="add the analysis, separate and combined legs")
     ap.add_argument("--devices", type=int, default=1, help="host legs over devices 0..D-1")
+    ap.add_argument("--layout", action="store_true", help="time channel maps and per-channel results on 7.1 tracks")
+    ap.add_argument("--baseline-lib", default=None, metavar="LIB", help="time the stereo device leg of this build against the library LIB")
     ap.add_argument("--out", default=None, help="also write the JSON document to this file")
     a = ap.parse_args()
+    a.tracks = a.tracks or (256 if a.layout else 1024)
     import torch
 
     import stratum_dsp_b200 as S
 
     if not torch.cuda.is_available() or S.device_count() < 1:
         raise SystemExit("loudness_bench needs a CUDA device: the measurement has no CPU fallback")
+    if a.layout or a.baseline_lib:
+        doc = layout_main(a, S, torch) if a.layout else baseline_main(a, S, torch)
+        s = json.dumps(doc, indent=1)
+        print(s)
+        if a.out:
+            Path(a.out).parent.mkdir(parents=True, exist_ok=True)
+            Path(a.out).write_text(s + "\n")
+        return
     if not 1 <= a.devices <= S.device_count():
         raise SystemExit(f"--devices {a.devices}: {S.device_count()} CUDA device(s) present")
     n = a.tracks
