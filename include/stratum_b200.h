@@ -369,6 +369,45 @@ int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t
  * one-channel track DUAL_MONO unless it is UNUSED.  Returns STRATUM_OK, or STRATUM_INVALID_INPUT for a NULL map or channels
  * outside 1..64. */
 int32_t stratum_b200_loudness_channel_map(uint32_t wave_mask, uint32_t channels, int32_t dual_mono, uint8_t* map);
+/* Loudness series: the loudness over time that an EBU Tech 3341 meter shows (and `ffmpeg -af ebur128` logs), and where the peaks
+ * lie, at the 100 ms step S of the definitions above.  Per measured track, nseg = ceil(frames / S):
+ *  - momentary series, J entries: entry j is the loudness l of momentary block j (frames [jS, jS + 4S)), -INFINITY for power 0.
+ *    A meter shows it at time (j + 4) S / sr.
+ *  - short-term series, K entries: entry k is the loudness of short-term window k (frames [kS, kS + 30S)), likewise.
+ *  - sample-peak series, nseg entries: entry s is max |x| over all channels and frames [sS, min((s + 1) S, frames)).
+ *  - true-peak series, nseg entries: entry s is the max over all channels of the sample peak and the |u| of the L - 1 interpolated
+ *    phases at those frames (the true_peak definition above, restricted to the segment's frames).
+ * The channel map weighs the momentary and short-term series exactly as it weighs the summary; the peak series are unweighted and
+ * count unused channels, as sample_peak and true_peak do.  The largest entry of each series equals out[i].momentary_max_lufs,
+ * short_term_max_lufs, sample_peak and true_peak bit for bit, so an album's maxima are the maxima over its members' entries.  A
+ * track that fails (status != STRATUM_OK) has no entries.  There are no per-channel or album series.
+ *
+ * The lengths of a track's series (host only, no device work; any pointer may be NULL): J, K and nseg of a track of `frames` frames
+ * at sample_rate Hz.  Returns STRATUM_OK, or the status a loudness entry gives that track, with all three counts 0. */
+int32_t stratum_b200_loudness_series_lengths(uint32_t sample_rate, uint64_t frames, uint32_t* n_momentary, uint32_t* n_short_term, uint32_t* n_peaks);
+/* stratum_b200_loudness_mapped_pcm with the four series.  Each array may be NULL, and then that series is neither produced nor read
+ * back; otherwise it holds the sum over the tracks of that series' lengths, track i's entries starting at the sum of the lengths of
+ * tracks 0 .. i-1 (the layout of channel_out).  Entries of failed tracks are not written.  Every other result is bit-identical with
+ * or without series, and stratum_b200_loudness_mapped_pcm is this entry with four NULLs.  The series add no kernel launch: pass 2
+ * keeps the peaks of each (segment, channel) and the gate writes the series, which are read back with the results. */
+int32_t stratum_b200_loudness_series_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out,
+                                         StratumLoudness* album_out, StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs,
+                                         double* sample_peaks, double* true_peaks);
+/* Same, with the PCM already resident in the memory of device `device_id`. */
+int32_t stratum_b200_loudness_series_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                const uint8_t* channel_map, int32_t device_id, StratumLoudness* out, StratumLoudness* album_out,
+                                                StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs, double* sample_peaks,
+                                                double* true_peaks);
+/* stratum_b200_analyze_loudness_mapped_pcm with the four series as in stratum_b200_loudness_series_pcm. */
+int32_t stratum_b200_analyze_loudness_series_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                 const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                                 uint32_t n_albums, const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices,
+                                                 StratumResult* out, StratumLoudness* loudness_out, StratumLoudness* album_out,
+                                                 StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs, double* sample_peaks,
+                                                 double* true_peaks);
 /* Host-side filters of the loudness measurement (no device work): kweight10 = stage 1 b0 b1 b2 a1 a2, stage 2 b0 b1 b2 a1 a2 (either
  * may be NULL), taps49 = the true-peak interpolator as the device uses it (f32).  Returns the oversampling factor L, or -1 for a
  * sample rate outside 8000..384000 Hz. */

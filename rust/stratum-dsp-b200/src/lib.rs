@@ -264,6 +264,67 @@ pub fn loudness_mapped_pcm(tracks: &[PcmTrack], albums: &[Option<u32>], channel_
     Ok((res.iter().map(loudness_from_c).collect(), alb.iter().map(loudness_from_c).collect(), split_channels(&chout, &chans, per_channel)))
 }
 
+/// The loudness series of one track (`stratum_b200_loudness_series_pcm` in `include/stratum_b200.h`) at a step of `step_seconds` =
+/// S / sr, S = (sr + 5) / 10 frames: `momentary_lufs[j]` is the 400 ms block [jS, jS + 4S) (a meter shows it at (j + 4) S / sr),
+/// `short_term_lufs[k]` the 3 s window [kS, kS + 30S), `sample_peak[s]` / `true_peak[s]` the linear peaks over all channels of the
+/// frames [sS, (s + 1) S).  The largest entries equal the track's maxima and peaks.
+#[derive(Clone, Debug, PartialEq)]
+pub struct LoudnessSeries {
+    pub momentary_lufs: Vec<f64>,
+    pub short_term_lufs: Vec<f64>,
+    pub sample_peak: Vec<f64>,
+    pub true_peak: Vec<f64>,
+    pub step_seconds: f64,
+}
+
+/// `loudness_mapped_pcm` without albums or per-channel results, plus each measured track's loudness series.
+#[allow(clippy::type_complexity)]
+pub fn loudness_series_pcm(tracks: &[PcmTrack], channel_maps: Option<&[Option<Vec<u8>>]>, devices: &[i32])
+    -> Result<Vec<Result<(Loudness, LoudnessSeries), AnalysisError>>, AnalysisError> {
+    check_loudness_abi()?;
+    let n = tracks.len();
+    let (flat, offsets, srs, chans, fmts) = pcm_tables(tracks);
+    let map = flat_channel_map(channel_maps, &chans)?;
+    let mut lens = Vec::with_capacity(n);
+    for (i, t) in tracks.iter().enumerate() {
+        let sample_bytes: u64 = match t.format { 1 => 1, 2 => 2, 3 => 3, 4 | 5 => 4, 6 => 8, _ => 0 };  // an unknown format is rejected by the call
+        let bpf = sample_bytes * t.channels.max(1) as u64;
+        let frames = if bpf > 0 { (offsets[i + 1] - offsets[i]) / bpf } else { 0 };
+        let (mut m, mut q, mut p) = (0u32, 0u32, 0u32);
+        unsafe { stratum_b200_loudness_series_lengths(t.sample_rate, frames, &mut m, &mut q, &mut p) };
+        lens.push((m as usize, q as usize, p as usize));
+    }
+    let mut mom = vec![0.0f64; lens.iter().map(|l| l.0).sum()];
+    let mut sht = vec![0.0f64; lens.iter().map(|l| l.1).sum()];
+    let mut spk = vec![0.0f64; lens.iter().map(|l| l.2).sum()];
+    let mut tpk = vec![0.0f64; spk.len()];
+    let mut res: Vec<StratumLoudness> = vec![unsafe { std::mem::zeroed() }; n];
+    let st = unsafe {
+        stratum_b200_loudness_series_pcm(flat.as_ptr(), offsets.as_ptr(), srs.as_ptr(), chans.as_ptr(), fmts.as_ptr(), n as u32, std::ptr::null(), 0,
+                                         map.as_ref().map_or(std::ptr::null(), |m| m.as_ptr()),
+                                         if devices.is_empty() { std::ptr::null() } else { devices.as_ptr() }, devices.len() as u32,
+                                         res.as_mut_ptr(), std::ptr::null_mut(), std::ptr::null_mut(), mom.as_mut_ptr(), sht.as_mut_ptr(), spk.as_mut_ptr(),
+                                         tpk.as_mut_ptr())
+    };
+    if st != 0 {
+        return Err(to_error(st, last_error()));
+    }
+    let (mut a, mut b, mut c) = (0usize, 0usize, 0usize);
+    Ok(res.iter().zip(lens).map(|(r, (m, q, p))| {
+        let series = LoudnessSeries {
+            momentary_lufs: mom[a..a + m].to_vec(),
+            short_term_lufs: sht[b..b + q].to_vec(),
+            sample_peak: spk[c..c + p].to_vec(),
+            true_peak: tpk[c..c + p].to_vec(),
+            step_seconds: if r.sample_rate > 0 { ((r.sample_rate + 5) / 10) as f64 / r.sample_rate as f64 } else { 0.0 },
+        };
+        a += m;
+        b += q;
+        c += p;
+        loudness_from_c(r).map(|l| (l, series))
+    }).collect())
+}
+
 /// Analysis (as `analyze_batch` gives it) and loudness (as `loudness_albums_pcm` gives it) of the same PCM tracks from one upload of
 /// each byte.  `albums`: as in `loudness_albums_pcm`, or `None` for no albums (the album list is then empty).  A track's analysis
 /// and its loudness fail or succeed independently.

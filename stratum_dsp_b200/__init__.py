@@ -221,6 +221,18 @@ def lib() -> C.CDLL:
     L.stratum_b200_analyze_loudness_mapped_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, C.c_void_p, u32p, _u, u8p, i32p, _u,
                                                            C.POINTER(StratumResult), loudp, loudp, loudp]
     L.stratum_b200_analyze_loudness_mapped_pcm.restype = _i
+    f64p = C.POINTER(C.c_double)
+    L.stratum_b200_loudness_series_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, u8p, i32p, _u, loudp, loudp, loudp, f64p, f64p, f64p,
+                                                   f64p]
+    L.stratum_b200_loudness_series_pcm.restype = _i
+    L.stratum_b200_loudness_series_pcm_device.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, u32p, _u, u8p, _i, loudp, loudp, loudp, f64p, f64p,
+                                                          f64p, f64p]
+    L.stratum_b200_loudness_series_pcm_device.restype = _i
+    L.stratum_b200_analyze_loudness_series_pcm.argtypes = [C.c_void_p, u64p, u32p, u32p, u32p, _u, C.c_void_p, u32p, _u, u8p, i32p, _u,
+                                                           C.POINTER(StratumResult), loudp, loudp, loudp, f64p, f64p, f64p, f64p]
+    L.stratum_b200_analyze_loudness_series_pcm.restype = _i
+    L.stratum_b200_loudness_series_lengths.argtypes = [_u, C.c_uint64, u32p, u32p, u32p]
+    L.stratum_b200_loudness_series_lengths.restype = _i
     L.stratum_b200_loudness_channel_map.argtypes = [_u, _u, _i, u8p]
     L.stratum_b200_loudness_channel_map.restype = _i
     L.stratum_b200_debug_loudness_filters.argtypes = [_u, C.POINTER(C.c_double), f32p]
@@ -620,6 +632,21 @@ class Loudness:
     frames: int
     error: AnalysisError | None = None  # set instead of raising for a track that failed on its own
     per_channel: list | None = None     # per_channel=True: one Loudness per channel, each measured alone at weight 1.0
+    series: LoudnessSeries | None = None  # series=True: the loudness over time and the peaks per 100 ms (tracks only)
+
+
+@dataclass
+class LoudnessSeries:
+    """The loudness series of one track (include/stratum_b200.h: stratum_b200_loudness_series_pcm), float64 arrays at a step of
+    ``step_seconds`` = S / sr (S = (sr + 5) // 10 frames): ``momentary_lufs[j]`` is the 400 ms block [j S, j S + 4 S) (a meter shows
+    it at (j + 4) S / sr), ``short_term_lufs[k]`` the 3 s window [k S, k S + 30 S), ``sample_peak[s]`` / ``true_peak[s]`` the peaks
+    over all channels of the frames [s S, (s + 1) S).  A failed track has empty arrays and ``step_seconds`` 0."""
+
+    momentary_lufs: np.ndarray
+    short_term_lufs: np.ndarray
+    sample_peak: np.ndarray
+    true_peak: np.ndarray
+    step_seconds: float
 
 
 def _loudness(r: StratumLoudness) -> Loudness:
@@ -682,6 +709,46 @@ def _with_channels(loud: list, chout, chans: np.ndarray) -> list:
     return loud
 
 
+def loudness_series_lengths(sample_rate: int, frames: int) -> tuple:
+    """stratum_b200_loudness_series_lengths: (momentary, short-term, peak) series lengths of a track of ``frames`` frames at
+    ``sample_rate`` Hz; (0, 0, 0) for a track the measurement rejects."""
+    n = (C.c_uint32 * 3)()
+    p = C.POINTER(C.c_uint32)
+    lib().stratum_b200_loudness_series_lengths(int(sample_rate), int(frames), C.cast(C.byref(n, 0), p), C.cast(C.byref(n, 4), p), C.cast(C.byref(n, 8), p))
+    return int(n[0]), int(n[1]), int(n[2])
+
+
+def _series_args(series: bool, offsets: np.ndarray, srs: np.ndarray, chans: np.ndarray, fmts: np.ndarray):
+    """(per-track lengths, four float64 arrays) of the series entries; (None, [None] * 4) without series."""
+    if not series:
+        return None, [None] * 4
+    lengths = []
+    for i in range(srs.size):
+        bpf = _PCM_BYTES.get(int(fmts[i]), 0) * max(int(chans[i]), 1)
+        frames = (int(offsets[i + 1]) - int(offsets[i])) // bpf if bpf else 0  # an unknown format is rejected by the call
+        lengths.append(loudness_series_lengths(int(srs[i]), frames))
+    n_m, n_q, n_p = (int(v) for v in np.sum(np.asarray(lengths, np.int64).reshape(-1, 3), axis=0))
+    return lengths, [np.zeros(v, np.float64) for v in (n_m, n_q, n_p, n_p)]
+
+
+def _f64p(a):
+    return a.ctypes.data_as(C.POINTER(C.c_double)) if a is not None else None
+
+
+def _with_series(loud: list, lengths, arrays) -> list:
+    if lengths is not None:
+        at = [0, 0, 0, 0]
+        for g, ln in zip(loud, lengths):
+            parts = []
+            for k in range(4):
+                m = ln[min(k, 2)]
+                parts.append(arrays[k][at[k]:at[k] + m].copy())
+                at[k] += m
+            step = ((g.sample_rate + 5) // 10) / g.sample_rate if g.error is None else 0.0
+            g.series = LoudnessSeries(*parts, step)
+    return loud
+
+
 def _pcm_tables(tracks: Sequence[PcmTrack]):
     n = len(tracks)
     offsets = np.zeros(n + 1, dtype=np.uint64)
@@ -693,23 +760,24 @@ def _pcm_tables(tracks: Sequence[PcmTrack]):
 
 
 def loudness_batch_pcm(tracks: Sequence[PcmTrack], devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None,
-                       per_channel: bool = False) -> list:
+                       per_channel: bool = False, series: bool = False) -> list:
     """stratum_b200_loudness_batch_pcm: integrated loudness, maxima, loudness range and peaks of undecoded PCM tracks, measured on
     the device and sharded over ``devices`` (default: the current device).  A failed track carries ``.error``.
     ``channel_maps``: one list of channel classes (CH_*, e.g. from ``channel_map``) per track, ``None`` for a track's default map;
-    ``per_channel=True`` fills each track's ``.per_channel`` (stratum_b200_loudness_mapped_pcm)."""
+    ``per_channel=True`` fills each track's ``.per_channel`` (stratum_b200_loudness_mapped_pcm); ``series=True`` fills each track's
+    ``.series`` (``LoudnessSeries``: the momentary and short-term loudness and the peaks per 100 ms, stratum_b200_loudness_series_pcm)."""
     if len(tracks) == 0:
         return []
-    return loudness_albums_pcm(tracks, [None] * len(tracks), 0, devices, channel_maps=channel_maps, per_channel=per_channel)[0]
+    return loudness_albums_pcm(tracks, [None] * len(tracks), 0, devices, channel_maps=channel_maps, per_channel=per_channel, series=series)[0]
 
 
 def loudness_batch_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
-                              device: int = -1, *, channel_maps: Sequence | None = None, per_channel: bool = False) -> list:
+                              device: int = -1, *, channel_maps: Sequence | None = None, per_channel: bool = False, series: bool = False) -> list:
     """stratum_b200_loudness_batch_pcm_device: the same with the PCM already in device memory (``d_pcm_ptr`` = device address of the
     concatenated track bytes, e.g. ``tensor.data_ptr()``; track i = bytes [byte_offsets[i], byte_offsets[i + 1]))."""
     n = np.asarray(byte_offsets).size - 1
     return loudness_albums_pcm_device(d_pcm_ptr, byte_offsets, sample_rates, channels, formats, [None] * n, 0, device, channel_maps=channel_maps,
-                                      per_channel=per_channel)[0]
+                                      per_channel=per_channel, series=series)[0]
 
 
 NO_ALBUM = 0xFFFFFFFF  # STRATUM_NO_ALBUM
@@ -727,32 +795,36 @@ def _album_ids(albums: Sequence[int | None], n_tracks: int, n_albums: int | None
 
 
 def loudness_albums_pcm(tracks: Sequence[PcmTrack], albums: Sequence[int | None], n_albums: int | None = None,
-                        devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None, per_channel: bool = False) -> tuple:
+                        devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None, per_channel: bool = False,
+                        series: bool = False) -> tuple:
     """stratum_b200_loudness_albums_pcm: the per-track results of ``loudness_batch_pcm`` and the loudness of albums (ReplayGain /
     R128 album values), each measured over the pooled 400 ms blocks and 3 s windows of its members.  ``albums[i]`` is the album id of
     track i (``None``: no album); ``n_albums`` defaults to the largest id + 1.  Returns ``(tracks, albums)``, two lists of
-    ``Loudness``; an album with a failed member, or one that no track names, carries ``.error``.  ``channel_maps`` and ``per_channel``
-    as in ``loudness_batch_pcm``; albums pool the members' mapped powers."""
+    ``Loudness``; an album with a failed member, or one that no track names, carries ``.error``.  ``channel_maps``, ``per_channel`` and
+    ``series`` as in ``loudness_batch_pcm``; albums pool the members' mapped powers and have no series."""
     n = len(tracks)
     ids, na = _album_ids(albums, n, n_albums)
     flat = [np.ascontiguousarray(t.data, dtype=np.uint8).reshape(-1) for t in tracks]
     cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
     offsets, srs, chans, fmts = _pcm_tables(tracks)
     cmap, chout = _channel_args(channel_maps, per_channel, chans)
+    lengths, ser = _series_args(series, offsets, srs, chans, fmts)
     res = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
     dev = (C.c_int32 * len(devices))(*devices) if devices else None
-    st = lib().stratum_b200_loudness_mapped_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+    st = lib().stratum_b200_loudness_series_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
                                                 srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)), fmts.ctypes.data_as(C.POINTER(_u)),
-                                                n, ids.ctypes.data_as(C.POINTER(_u)), na, _u8p(cmap), dev, len(devices) if devices else 0, res, alb, chout)
+                                                n, ids.ctypes.data_as(C.POINTER(_u)), na, _u8p(cmap), dev, len(devices) if devices else 0, res, alb, chout,
+                                                *[_f64p(a) for a in ser])
     if st != OK:
         _raise(st)
-    return _with_channels([_loudness(res[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
+    loud = _with_series(_with_channels([_loudness(res[i]) for i in range(n)], chout, chans), lengths, ser)
+    return loud, [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_rates: Sequence[int], channels: Sequence[int], formats: Sequence[int],
                                albums: Sequence[int | None], n_albums: int | None = None, device: int = -1, *, channel_maps: Sequence | None = None,
-                               per_channel: bool = False) -> tuple:
+                               per_channel: bool = False, series: bool = False) -> tuple:
     """stratum_b200_loudness_albums_pcm_device: ``loudness_albums_pcm`` with the PCM already in device memory (arguments as
     ``loudness_batch_pcm_device``)."""
     offsets = np.ascontiguousarray(byte_offsets, dtype=np.uint64)
@@ -764,24 +836,27 @@ def loudness_albums_pcm_device(d_pcm_ptr: int, byte_offsets: np.ndarray, sample_
         raise ValueError("one sample rate, channel count and format per track")
     ids, na = _album_ids(albums, n, n_albums)
     cmap, chout = _channel_args(channel_maps, per_channel, chans)
+    lengths, ser = _series_args(series, offsets, srs, chans, fmts)
     res = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
-    st = lib().stratum_b200_loudness_mapped_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+    st = lib().stratum_b200_loudness_series_pcm_device(C.c_void_p(d_pcm_ptr), offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
                                                        srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)),
                                                        fmts.ctypes.data_as(C.POINTER(_u)), n, ids.ctypes.data_as(C.POINTER(_u)), na, _u8p(cmap), device, res,
-                                                       alb, chout)
+                                                       alb, chout, *[_f64p(a) for a in ser])
     if st != OK:
         _raise(st)
-    return _with_channels([_loudness(res[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
+    loud = _with_series(_with_channels([_loudness(res[i]) for i in range(n)], chout, chans), lengths, ser)
+    return loud, [_loudness(alb[a]) for a in range(na)]
 
 
 def analyze_loudness_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | None = None, albums: Sequence[int | None] | None = None,
                          n_albums: int | None = None, devices: Sequence[int] | None = None, *, channel_maps: Sequence | None = None,
-                         per_channel: bool = False) -> tuple:
+                         per_channel: bool = False, series: bool = False) -> tuple:
     """stratum_b200_analyze_loudness_pcm: ``analyze_batch_pcm`` and ``loudness_albums_pcm`` of the same tracks from one upload.
     Returns ``(results, loudness, album_loudness)``: the analysis results as ``analyze_batch_pcm`` returns them, one ``Loudness`` per
     track and one per album (``[]`` without ``albums``).  A track's analysis and its loudness fail or succeed independently.
-    ``channel_maps`` and ``per_channel`` weigh and split the loudness only (stratum_b200_analyze_loudness_mapped_pcm)."""
+    ``channel_maps`` and ``per_channel`` weigh and split the loudness only (stratum_b200_analyze_loudness_mapped_pcm); ``series``
+    as in ``loudness_batch_pcm`` (stratum_b200_analyze_loudness_series_pcm)."""
     n = len(tracks)
     if albums is None:
         if n_albums:
@@ -793,18 +868,20 @@ def analyze_loudness_pcm(tracks: Sequence[PcmTrack], config: AnalysisConfig | No
     cat = np.concatenate(flat) if n > 1 else (flat[0] if n else np.zeros(0, np.uint8))
     offsets, srs, chans, fmts = _pcm_tables(tracks)
     cmap, chout = _channel_args(channel_maps, per_channel, chans)
+    lengths, ser = _series_args(series, offsets, srs, chans, fmts)
     res = (StratumResult * max(n, 1))()
     loud = (StratumLoudness * max(n, 1))()
     alb = (StratumLoudness * max(na, 1))()
     dev = (C.c_int32 * len(devices))(*devices) if devices else None
     cfgp = C.cast(C.byref(config._c), C.c_void_p) if config is not None else None
-    st = lib().stratum_b200_analyze_loudness_mapped_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
+    st = lib().stratum_b200_analyze_loudness_series_pcm(cat.ctypes.data if cat.size else None, offsets.ctypes.data_as(C.POINTER(C.c_uint64)),
                                                         srs.ctypes.data_as(C.POINTER(_u)), chans.ctypes.data_as(C.POINTER(_u)),
                                                         fmts.ctypes.data_as(C.POINTER(_u)), n, cfgp, ids.ctypes.data_as(C.POINTER(_u)) if ids is not None else None,
-                                                        na, _u8p(cmap), dev, len(devices) if devices else 0, res, loud, alb, chout)
+                                                        na, _u8p(cmap), dev, len(devices) if devices else 0, res, loud, alb, chout, *[_f64p(a) for a in ser])
     if st != OK:
         _fail(st, res, n)
-    return _collect(res, n), _with_channels([_loudness(loud[i]) for i in range(n)], chout, chans), [_loudness(alb[a]) for a in range(na)]
+    tracks_loud = _with_series(_with_channels([_loudness(loud[i]) for i in range(n)], chout, chans), lengths, ser)
+    return _collect(res, n), tracks_loud, [_loudness(alb[a]) for a in range(na)]
 
 
 def loudness_filters(sample_rate: int) -> tuple:

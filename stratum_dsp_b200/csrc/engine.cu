@@ -259,6 +259,7 @@ struct DeviceCtx {
     size_t loud_cap = 0;
     PinnedBuf loud_rec[2], loud_out[2];  // pinned track records / results of two chunks (chunk k+1 is queued before chunk k is read)
     PinnedBuf loud_blk[2];    // momentary and short-term powers of the same two chunks (calls with albums only)
+    PinnedBuf loud_ser[2];    // the requested loudness series of the same two chunks (series calls only)
     char* d_album = nullptr;  // album phase: album records, pooled powers, selection scratch, results
     size_t album_cap = 0;
     cudaEvent_t loud_ev[2] = {nullptr, nullptr};
@@ -2564,6 +2565,36 @@ struct LoudChannels {
     std::vector<uint64_t> at;
 };
 
+// The series side of a loudness call (include/stratum_b200.h: stratum_b200_loudness_series_pcm): the caller's arrays in the order of
+// LoudSeries (null: that series is neither produced nor read back), and per series where track q's entries start, at[s][q]: the
+// lengths of the tracks before it.
+struct LoudSeriesOut {
+    double* dst[4] = {nullptr, nullptr, nullptr, nullptr};  // momentary, short-term, sample-peak, true-peak
+    std::vector<uint64_t> at[4];
+    uint32_t count() const { return (dst[0] != nullptr) + (dst[1] != nullptr) + (dst[2] != nullptr) + (dst[3] != nullptr); }
+    bool peaks() const { return dst[2] || dst[3]; }
+    static uint32_t length(const LoudGeom& g, int k) { return k == 0 ? g.J : (k == 1 ? g.K : g.nseg); }
+};
+
+static void series_layout(double* mom, double* sht, double* spk, double* tpk, const uint64_t* offsets, const std::vector<uint32_t>& bpf,
+                          const uint32_t* sample_rates, uint32_t n_tracks, LoudSeriesOut& so) {
+    double* d[4] = {mom, sht, spk, tpk};
+    for (int k = 0; k < 4; ++k) {
+        so.dst[k] = d[k];
+        so.at[k].assign(d[k] ? n_tracks : 0, 0);
+    }
+    if (!so.count()) return;
+    uint64_t next[4] = {0, 0, 0, 0};
+    for (uint32_t q = 0; q < n_tracks; ++q) {
+        const LoudGeom g = loud_geom(sample_rates[q], (offsets[q + 1] - offsets[q]) / bpf[q]);
+        for (int k = 0; k < 4; ++k)
+            if (d[k]) {
+                so.at[k][q] = next[k];
+                next[k] += LoudSeriesOut::length(g, k);
+            }
+    }
+}
+
 // Weight of a channel class (include/stratum_b200.h: StratumChannelClass); codes are checked by channels_validate.
 static double loud_class_weight(uint8_t code) {
     switch (code) {
@@ -2584,6 +2615,7 @@ struct LoudnessSink final : ChunkSink {
     StratumLoudness* out;
     AlbumPools* pools;  // null without albums
     const LoudChannels& chans_;  // channel map, per-channel results
+    const LoudSeriesOut& ser_;  // requested series
     cudaStream_t stream;  // every launch and copy of the sink; ctx->stream unless set before open()
     struct Slot {
         uint32_t i = 0, j = 0;
@@ -2592,8 +2624,8 @@ struct LoudnessSink final : ChunkSink {
         std::vector<PendingStage> stages;
     } slot[2];
     LoudnessSink(DeviceCtx* c, const uint64_t* offs, const std::vector<uint32_t>& bpf_, const uint32_t* srs, const uint32_t* chans, const uint32_t* fmts,
-                 StratumLoudness* o, AlbumPools* p, const LoudChannels& lc)
-        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p), chans_(lc), stream(c->stream) {}
+                 StratumLoudness* o, AlbumPools* p, const LoudChannels& lc, const LoudSeriesOut& so)
+        : ctx(c), offsets(offs), bpf(bpf_), sample_rates(srs), channels(chans), formats(fmts), out(o), pools(p), chans_(lc), ser_(so), stream(c->stream) {}
     bool has_member(uint32_t i, uint32_t j) const {
         for (uint32_t q = i; pools && q < j; ++q)
             if (pools->member(q)) return true;
@@ -2647,15 +2679,17 @@ struct LoudnessSink final : ChunkSink {
     }
 
     // Device work area of a chunk: records and weight table (uploaded together), track then per-channel results (zeroed and read
-    // back together), cascade states and energies, per-segment areas, and with per-channel results their areas.
+    // back together), cascade states and energies, per-segment areas, with per-channel results their areas, with peak series the
+    // work items' peaks, and one region of n_seg doubles per requested series.
     static size_t rec_bytes(uint64_t n_tracks, uint64_t n_ch) { return align_up(n_tracks * sizeof(LoudTrack), 256) + n_ch * sizeof(double); }
     size_t ws_bytes(uint64_t n_tracks, uint64_t n_work, uint64_t n_seg, uint64_t n_ch) const {
         return align_up(rec_bytes(n_tracks, n_ch), 256) + align_up((n_tracks + n_ch) * sizeof(LoudOut), 256) + align_up(5 * n_work * sizeof(double), 256) +
-               align_up(4 * n_seg * sizeof(double), 256) + (chans_.out ? align_up(4 * n_work * sizeof(double), 256) : 0);
+               align_up(4 * n_seg * sizeof(double), 256) + (chans_.out ? align_up(4 * n_work * sizeof(double), 256) : 0) +
+               (ser_.peaks() ? align_up(2 * n_work * sizeof(float), 256) : 0) + ser_.count() * align_up(n_seg * sizeof(double), 256);
     }
 
     int open(const std::vector<HostChunk>& chunks) override {
-        size_t need = 0, rec_max = 0, out_max = 0, blk_bytes = 0;
+        size_t need = 0, rec_max = 0, out_max = 0, blk_bytes = 0, ser_bytes = 0;
         for (const HostChunk& ch : chunks) {
             uint64_t w, sg, nc;
             uint32_t mc;
@@ -2664,9 +2698,10 @@ struct LoudnessSink final : ChunkSink {
             rec_max = std::max(rec_max, rec_bytes(ch.j - ch.i, nc));
             out_max = std::max<size_t>(out_max, (ch.j - ch.i + nc) * sizeof(LoudOut));
             if (has_member(ch.i, ch.j)) blk_bytes = std::max<size_t>(blk_bytes, 2 * sg * sizeof(double));
+            ser_bytes = std::max<size_t>(ser_bytes, ser_.count() * sg * sizeof(double));
         }
-        for (int b = 0; b < 2 && blk_bytes; ++b)
-            if (!ctx->loud_blk[b].need(blk_bytes)) {
+        for (int b = 0; b < 2 && (blk_bytes || ser_bytes); ++b)
+            if ((blk_bytes && !ctx->loud_blk[b].need(blk_bytes)) || (ser_bytes && !ctx->loud_ser[b].need(ser_bytes))) {
                 set_error("pinned host allocation failed");
                 return STRATUM_PROCESSING_ERROR;
             }
@@ -2709,6 +2744,14 @@ struct LoudnessSink final : ChunkSink {
         double* d_ws = reinterpret_cast<double*>(d);
         d += align_up(4 * n_seg * sizeof(double), 256);
         double* d_cws = chans_.out ? reinterpret_cast<double*>(d) : nullptr;
+        if (chans_.out) d += align_up(4 * n_work * sizeof(double), 256);
+        float* d_pk = ser_.peaks() ? reinterpret_cast<float*>(d) : nullptr;
+        if (d_pk) d += align_up(2 * n_work * sizeof(float), 256);
+        double* d_ser[4];
+        for (int q = 0; q < 4; ++q) {
+            d_ser[q] = ser_.dst[q] ? reinterpret_cast<double*>(d) : nullptr;
+            if (d_ser[q]) d += align_up(n_seg * sizeof(double), 256);
+        }
         cudaStream_t s = stream;
         CUDA_OK(cudaMemcpyAsync(d_tr, h_rec, rec_bytes(n, n_ch), cudaMemcpyHostToDevice, s));
         CUDA_OK(cudaMemsetAsync(d_out, 0, (size_t)(n + n_ch) * sizeof(LoudOut), s));
@@ -2723,11 +2766,12 @@ struct LoudnessSink final : ChunkSink {
         }
         {
             StageTimer tm(s, "loudness_pass2");
-            launch_loud_pass2(s, d_buf, d_tr, n, n_work, d_st, d_en, d_chout);
+            launch_loud_pass2(s, d_buf, d_tr, n, n_work, d_st, d_en, d_chout, d_pk);
         }
         {
             StageTimer tm(s, "loudness_gate");
-            launch_loud_gate(s, d_tr, n, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout, chans_.out ? max_c : 0);
+            launch_loud_gate(s, d_tr, n, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout, chans_.out ? max_c : 0, d_pk,
+                             LoudSeries{d_ser[0], d_ser[1], d_ser[2], d_ser[3]});
         }
         CUDA_OK(cudaGetLastError());
         const uint64_t n_read = chans_.out ? n + n_ch : n;  // the per-channel results follow the track results
@@ -2738,6 +2782,13 @@ struct LoudnessSink final : ChunkSink {
             CUDA_OK(cudaMemcpyAsync(ctx->loud_blk[k & 1].p, d_ws + n_seg, 2 * n_seg * sizeof(double), cudaMemcpyDeviceToHost, s));
             g_d2h_bytes.fetch_add(2 * n_seg * sizeof(double));
         }
+        double* h_ser = static_cast<double*>(ctx->loud_ser[k & 1].p);
+        for (int q = 0; q < 4 && n_seg; ++q)  // the requested series one after the other, n_seg doubles each
+            if (d_ser[q]) {
+                CUDA_OK(cudaMemcpyAsync(h_ser, d_ser[q], n_seg * sizeof(double), cudaMemcpyDeviceToHost, s));
+                g_d2h_bytes.fetch_add(n_seg * sizeof(double));
+                h_ser += n_seg;
+            }
         CUDA_OK(cudaEventRecord(ctx->loud_ev[k & 1], s));
         Slot& cur = slot[k & 1];
         cur.i = ch.i;
@@ -2772,6 +2823,13 @@ struct LoudnessSink final : ChunkSink {
                 memcpy(pools->buf.data() + pools->m_at[q], blk + T.seg0, (size_t)T.J * sizeof(double));
                 memcpy(pools->buf.data() + pools->q_at[q], blk + sl.n_seg + T.seg0, (size_t)T.K * sizeof(double));
             }
+            const double* h_ser = static_cast<const double*>(ctx->loud_ser[b].p);
+            const uint32_t len[4] = {T.J, T.K, T.nseg, T.nseg};
+            for (int s = 0; s < 4; ++s)
+                if (ser_.dst[s]) {
+                    memcpy(ser_.dst[s] + ser_.at[s][q], h_ser + T.seg0, (size_t)len[s] * sizeof(double));
+                    h_ser += sl.n_seg;
+                }
         }
         return STRATUM_OK;
     }
@@ -2948,39 +3006,55 @@ static int32_t album_phase(int32_t device, AlbumPools& P, uint32_t n_tracks, con
     return STRATUM_OK;
 }
 
-int32_t stratum_b200_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+int32_t stratum_b200_loudness_series_lengths(uint32_t sample_rate, uint64_t frames, uint32_t* n_momentary, uint32_t* n_short_term, uint32_t* n_peaks) {
+    char msg[128];
+    const int st = loud_track_status(sample_rate, frames, msg, sizeof msg);
+    const LoudGeom g = loud_geom(sample_rate, frames);
+    if (n_momentary) *n_momentary = LoudSeriesOut::length(g, 0);
+    if (n_short_term) *n_short_term = LoudSeriesOut::length(g, 1);
+    if (n_peaks) *n_peaks = LoudSeriesOut::length(g, 2);
+    return st;
+}
+
+int32_t stratum_b200_loudness_series_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                          const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
                                          const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out,
-                                         StratumLoudness* album_out, StratumLoudness* channel_out) {
+                                         StratumLoudness* album_out, StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs,
+                                         double* sample_peaks, double* true_peaks) {
     std::vector<uint32_t> bpf;
     LoudChannels lc;
+    LoudSeriesOut so;
     int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
     if (st == STRATUM_OK) st = channels_validate(channel_map, channel_out, channels, n_tracks, lc);
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    series_layout(momentary_lufs, short_term_lufs, sample_peaks, true_peaks, byte_offsets, bpf, sample_rates, n_tracks, so);
     AlbumPools* pp = n_albums ? &pools : nullptr;
     if (n_tracks)
         st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
-            return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, pp, lc));
+            return std::unique_ptr<ChunkSink>(new LoudnessSink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, pp, lc, so));
         });
     if (st != STRATUM_OK || n_albums == 0) return st;
     return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, out, album_out);
 }
 
-int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+int32_t stratum_b200_loudness_series_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                 const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
                                                 const uint8_t* channel_map, int32_t device_id, StratumLoudness* out, StratumLoudness* album_out,
-                                                StratumLoudness* channel_out) {
+                                                StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs, double* sample_peaks,
+                                                double* true_peaks) {
     std::vector<uint32_t> bpf;
     LoudChannels lc;
+    LoudSeriesOut so;
     int st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, out, d_pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
     if (st == STRATUM_OK) st = channels_validate(channel_map, channel_out, channels, n_tracks, lc);
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    series_layout(momentary_lufs, short_term_lufs, sample_peaks, true_peaks, byte_offsets, bpf, sample_rates, n_tracks, so);
     if (n_tracks) {
         DeviceCtx* ctx = get_ctx(device_id, &st);
         if (!ctx) return st;
@@ -2991,7 +3065,7 @@ int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_
         }
         // the whole batch is one chunk: one launch of each kernel
         const std::vector<HostChunk> one{HostChunk{0, n_tracks, byte_offsets[n_tracks] - byte_offsets[0], 0}};
-        LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, n_albums ? &pools : nullptr, lc);
+        LoudnessSink sink(ctx, byte_offsets, bpf, sample_rates, channels, formats, out, n_albums ? &pools : nullptr, lc, so);
         st = sink.open(one);
         if (st != STRATUM_OK) return st;
         const int s1 = sink.chunk(0, one[0], static_cast<const char*>(d_pcm) + byte_offsets[0], [] {});
@@ -3000,6 +3074,22 @@ int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_
     }
     if (st != STRATUM_OK || n_albums == 0) return st;
     return album_phase(device_id, pools, n_tracks, out, album_out);
+}
+
+int32_t stratum_b200_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                         const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                         const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices, StratumLoudness* out,
+                                         StratumLoudness* album_out, StratumLoudness* channel_out) {
+    return stratum_b200_loudness_series_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, album_of_track, n_albums, channel_map, device_ids,
+                                            n_devices, out, album_out, channel_out, nullptr, nullptr, nullptr, nullptr);
+}
+
+int32_t stratum_b200_loudness_mapped_pcm_device(const void* d_pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                const uint32_t* formats, uint32_t n_tracks, const uint32_t* album_of_track, uint32_t n_albums,
+                                                const uint8_t* channel_map, int32_t device_id, StratumLoudness* out, StratumLoudness* album_out,
+                                                StratumLoudness* channel_out) {
+    return stratum_b200_loudness_series_pcm_device(d_pcm, byte_offsets, sample_rates, channels, formats, n_tracks, album_of_track, n_albums, channel_map,
+                                                   device_id, out, album_out, channel_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int32_t stratum_b200_loudness_albums_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
@@ -3037,8 +3127,9 @@ struct AnalysisLoudnessSink final : ChunkSink {
     AnalysisSink ana;
     LoudnessSink loud;
     AnalysisLoudnessSink(DeviceCtx* c, const StratumConfig& cfg, const uint64_t* offs, const std::vector<uint32_t>& bpf, const uint32_t* srs,
-                         const uint32_t* chans, const uint32_t* fmts, StratumResult* o, StratumLoudness* lo, AlbumPools* p, const LoudChannels& lc)
-        : ana(c, cfg, offs, bpf, srs, chans, fmts, o), loud(c, offs, bpf, srs, chans, fmts, lo, p, lc) {}
+                         const uint32_t* chans, const uint32_t* fmts, StratumResult* o, StratumLoudness* lo, AlbumPools* p, const LoudChannels& lc,
+                         const LoudSeriesOut& so)
+        : ana(c, cfg, offs, bpf, srs, chans, fmts, o), loud(c, offs, bpf, srs, chans, fmts, lo, p, lc, so) {}
 
     int open(const std::vector<HostChunk>& chunks) override {
         DeviceCtx* ctx = ana.ctx;
@@ -3068,11 +3159,12 @@ struct AnalysisLoudnessSink final : ChunkSink {
     }
 };
 
-int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+int32_t stratum_b200_analyze_loudness_series_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
                                                  const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
                                                  uint32_t n_albums, const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices,
                                                  StratumResult* out, StratumLoudness* loudness_out, StratumLoudness* album_out,
-                                                 StratumLoudness* channel_out) {
+                                                 StratumLoudness* channel_out, double* momentary_lufs, double* short_term_lufs, double* sample_peaks,
+                                                 double* true_peaks) {
     // the order of stratum_b200_analyze_batch_pcm: NULL pointers, the configuration, the PCM layout; then the album ids, the channel map
     if (!byte_offsets || !sample_rates || !channels || !formats || !out || !loudness_out || (!pcm && n_tracks && byte_offsets[n_tracks] > 0)) {
         set_error("null argument");
@@ -3083,6 +3175,7 @@ int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t
     const StratumConfig& c = cfg ? *cfg : def;
     std::vector<uint32_t> bpf;
     LoudChannels lc;
+    LoudSeriesOut so;
     int st = config_validate(c);
     if (st == STRATUM_OK) st = loudness_validate(byte_offsets, sample_rates, channels, formats, n_tracks, loudness_out, pcm != nullptr, bpf);
     if (st == STRATUM_OK) st = albums_validate(album_of_track, n_tracks, n_albums, album_out);
@@ -3090,14 +3183,24 @@ int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t
     if (st != STRATUM_OK) return st;
     AlbumPools pools;
     album_layout(album_of_track, n_albums, byte_offsets, bpf, sample_rates, n_tracks, pools);
+    series_layout(momentary_lufs, short_term_lufs, sample_peaks, true_peaks, byte_offsets, bpf, sample_rates, n_tracks, so);
     AlbumPools* pp = n_albums ? &pools : nullptr;
     if (n_tracks)
         st = stream_host_batch(pcm, byte_offsets, bpf, n_tracks, device_ids, n_devices, [&](DeviceCtx* ctx) -> std::unique_ptr<ChunkSink> {
             return std::unique_ptr<ChunkSink>(
-                new AnalysisLoudnessSink(ctx, c, byte_offsets, bpf, sample_rates, channels, formats, out, loudness_out, pp, lc));
+                new AnalysisLoudnessSink(ctx, c, byte_offsets, bpf, sample_rates, channels, formats, out, loudness_out, pp, lc, so));
         });
     if (st != STRATUM_OK || n_albums == 0) return st;
     return album_phase(device_ids && n_devices ? device_ids[0] : -1, pools, n_tracks, loudness_out, album_out);
+}
+
+int32_t stratum_b200_analyze_loudness_mapped_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
+                                                 const uint32_t* formats, uint32_t n_tracks, const StratumConfig* cfg, const uint32_t* album_of_track,
+                                                 uint32_t n_albums, const uint8_t* channel_map, const int32_t* device_ids, uint32_t n_devices,
+                                                 StratumResult* out, StratumLoudness* loudness_out, StratumLoudness* album_out,
+                                                 StratumLoudness* channel_out) {
+    return stratum_b200_analyze_loudness_series_pcm(pcm, byte_offsets, sample_rates, channels, formats, n_tracks, cfg, album_of_track, n_albums, channel_map,
+                                                    device_ids, n_devices, out, loudness_out, album_out, channel_out, nullptr, nullptr, nullptr, nullptr);
 }
 
 int32_t stratum_b200_analyze_loudness_pcm(const void* pcm, const uint64_t* byte_offsets, const uint32_t* sample_rates, const uint32_t* channels,
@@ -3351,6 +3454,7 @@ void stratum_b200_shutdown(void) {
                 c->loud_rec[b].release();
                 c->loud_out[b].release();
                 c->loud_blk[b].release();
+                c->loud_ser[b].release();
                 if (c->loud_ev[b]) cudaEventDestroy(c->loud_ev[b]);
             }
             c->h_count.release();

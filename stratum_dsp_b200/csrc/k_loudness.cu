@@ -13,6 +13,8 @@
 //           sub-blocks, the absolute and relative gates, the maxima and the loudness range (exact order statistics), and the
 //           track peaks as the maxima over its channels; on request one more CTA per (track, channel) gates that channel alone
 //           (stratum_b200_loudness_mapped_pcm: channel_out);
+//   series  on request (stratum_b200_loudness_series_pcm) pass 2 also stores every work item's two peaks and the track's gate CTA
+//           writes the loudness of every momentary / short-term power and the per-segment maxima of those peaks over the channels;
 //   album   one CTA per album: the same gates, maxima and range over the members' momentary / short-term powers, pooled on the
 //           host in ascending track order (stratum_b200_loudness_albums_pcm).
 // The recurrence runs in f64: at 192 kHz the high-pass pole of stage 2 lies 1.2e-3 from the unit circle, and f32 coefficients
@@ -196,7 +198,8 @@ __device__ __forceinline__ void loud_pass2_item(const LoudTrack& T, const unsign
 }
 
 __global__ void __launch_bounds__(256) loud_pass2_kernel(const unsigned char* __restrict__ pcm, const LoudTrack* __restrict__ tr, uint32_t n_tracks,
-                                                         uint64_t n_work, const double* __restrict__ st, double* __restrict__ en, LoudOut* __restrict__ chout) {
+                                                         uint64_t n_work, const double* __restrict__ st, double* __restrict__ en, LoudOut* __restrict__ chout,
+                                                         float* __restrict__ pk) {
     const uint64_t w = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool valid = w < n_work;
     const uint32_t t = valid ? loud_track_of(tr, n_tracks, w) : 0xffffffffu;
@@ -226,6 +229,10 @@ __global__ void __launch_bounds__(256) loud_pass2_kernel(const unsigned char* __
         if (energy) en[w] = sum;
     }
     tpk = fmaxf(tpk, spk);
+    if (pk && valid) {  // the peak series: this segment's peaks of this channel, reduced over the channels by the gate
+        pk[w] = spk;
+        pk[n_work + w] = tpk;
+    }
     // Work items are channel-minor, so lanes l and l ^ o hold the same channel whenever C divides o.  When the warp lies inside one
     // track (the common case) and C is a power of two dividing 32, xor-shuffles over o = 16 .. C leave lane c < C with its channel's
     // maximum over the warp and those C lanes issue the atomics; otherwise every lane issues its own.
@@ -371,11 +378,33 @@ __device__ __forceinline__ void loud_gate_track(const LoudTrack& T, const double
     loud_gate_lists(m, J, q, K, kp, o);
 }
 
-// blockIdx.y = 0: track blockIdx.x over its weighted channels, and its peaks as the maxima over its channels' peaks; blockIdx.y =
-// 1 + c: channel c of the track alone (per-channel results).
+// The requested series of track T from its momentary / short-term powers m, q and the work items' peaks pk (kernels.h: LoudSeries).
+__device__ __forceinline__ void loud_series_track(const LoudTrack& T, const double* __restrict__ m, const double* __restrict__ q, const float* __restrict__ pk,
+                                                  uint64_t n_work, const LoudSeries& ser) {
+    if (ser.mom)
+        for (uint32_t j = threadIdx.x; j < T.J; j += LOUD_GATE_THREADS) ser.mom[T.seg0 + j] = lufs_of(m[j]);
+    if (ser.sht)
+        for (uint32_t j = threadIdx.x; j < T.K; j += LOUD_GATE_THREADS) ser.sht[T.seg0 + j] = lufs_of(q[j]);
+    if (ser.spk || ser.tpk)
+        for (uint32_t s = threadIdx.x; s < T.nseg; s += LOUD_GATE_THREADS) {
+            const float* p = pk + T.work + (uint64_t)s * T.C;
+            float sp = 0.0f, tp = 0.0f;
+            for (uint32_t c = 0; c < T.C; ++c) {
+                sp = fmaxf(sp, p[c]);
+                tp = fmaxf(tp, p[n_work + c]);
+            }
+            if (ser.spk) ser.spk[T.seg0 + s] = sp;
+            if (ser.tpk) ser.tpk[T.seg0 + s] = tp;
+        }
+}
+
+// blockIdx.y = 0: track blockIdx.x over its weighted channels, its peaks as the maxima over its channels' peaks and, with SERIES,
+// the requested series; blockIdx.y = 1 + c: channel c of the track alone (per-channel results).  Without series the launch runs the
+// instance that has no series code at all.
+template <bool SERIES>
 __global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const LoudTrack* __restrict__ tr, const double* __restrict__ wt, const double* __restrict__ en,
                                                                       double* __restrict__ ws, uint64_t n_seg, LoudOut* __restrict__ out, double* __restrict__ cws,
-                                                                      uint64_t n_work, LoudOut* __restrict__ chout) {
+                                                                      uint64_t n_work, LoudOut* __restrict__ chout, const float* __restrict__ pk, LoudSeries ser) {
     const LoudTrack& T = tr[blockIdx.x];
     if (T.nseg == 0) return;
     if (blockIdx.y == 0) {
@@ -390,6 +419,8 @@ __global__ void __launch_bounds__(LOUD_GATE_THREADS) loud_gate_kernel(const Loud
         }
         double* z = ws + T.seg0;
         loud_gate_track(T, wt + T.ch0, 0, T.C, en, z, z + n_seg, z + 2 * n_seg, z + 3 * n_seg, out + blockIdx.x);
+        // m and q are final once loud_gate_track has returned (the gates only read them)
+        if constexpr (SERIES) loud_series_track(T, z + n_seg, z + 2 * n_seg, pk, n_work, ser);
         return;
     }
     const uint32_t c = blockIdx.y - 1;
@@ -419,16 +450,21 @@ void launch_loud_scan(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, 
 }
 
 void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, const double* d_st, double* d_en,
-                       LoudOut* d_chout) {
+                       LoudOut* d_chout, float* d_pk) {
     if (n_work == 0) return;
-    loud_pass2_kernel<<<(unsigned)((n_work + 255) / 256), 256, 0, s>>>(static_cast<const unsigned char*>(d_pcm), d_tr, n_tracks, n_work, d_st, d_en, d_chout);
+    loud_pass2_kernel<<<(unsigned)((n_work + 255) / 256), 256, 0, s>>>(static_cast<const unsigned char*>(d_pcm), d_tr, n_tracks, n_work, d_st, d_en, d_chout,
+                                                                       d_pk);
     count_launch("loudness");
 }
 
 void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_wt, const double* d_en, double* d_ws, uint64_t n_seg,
-                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks) {
+                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks, const float* d_pk, LoudSeries ser) {
     if (n_tracks == 0) return;
-    loud_gate_kernel<<<dim3(n_tracks, 1 + ch_blocks), LOUD_GATE_THREADS, 0, s>>>(d_tr, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout);
+    const dim3 grid(n_tracks, 1 + ch_blocks);
+    if (ser.mom || ser.sht || ser.spk || ser.tpk)
+        loud_gate_kernel<true><<<grid, LOUD_GATE_THREADS, 0, s>>>(d_tr, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout, d_pk, ser);
+    else
+        loud_gate_kernel<false><<<grid, LOUD_GATE_THREADS, 0, s>>>(d_tr, d_wt, d_en, d_ws, n_seg, d_out, d_cws, n_work, d_chout, d_pk, ser);
     count_launch("loudness");
 }
 

@@ -234,14 +234,21 @@ inline double loud_channel_weight(uint32_t C, uint32_t c) {
 void launch_loud_pass1(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, double* d_st);
 void launch_loud_scan(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, uint32_t max_channels, double* d_st);
 // Sample and true peaks per (track, channel) into d_chout[T.ch0 + c] (zeroed by the caller); the gate derives the track peaks.
+// d_pk: null, or 2 x n_work floats that take every work item's sample peak (d_pk[w]) and true peak (d_pk[n_work + w]).
 void launch_loud_pass2(cudaStream_t s, const void* d_pcm, const LoudTrack* d_tr, uint32_t n_tracks, uint64_t n_work, const double* d_st, double* d_en,
-                       LoudOut* d_chout);
+                       LoudOut* d_chout, float* d_pk);
+// The loudness series of a launch (include/stratum_b200.h: stratum_b200_loudness_series_pcm), each null or n_seg doubles with track
+// T's entries from T.seg0: momentary and short-term loudness (J / K entries), sample and true peaks per segment (nseg entries).
+struct LoudSeries {
+    double *mom, *sht, *spk, *tpk;
+};
 // d_wt: channel weights, track T's at d_wt[T.ch0 ..).  d_ws: 4 x n_seg doubles (sub-block, momentary and short-term powers, the
 // compacted short-term powers of the loudness range).  With ch_blocks > 0 (the largest channel count of the launch) the launch adds
 // one CTA per (track, channel) that gates the channel alone into d_chout[T.ch0 + c], over d_cws: 4 x n_work doubles laid out like
-// d_ws, channel c of track T at T.work + c * T.nseg.
+// d_ws, channel c of track T at T.work + c * T.nseg.  The track CTAs write the series of ser; the peak series reduce d_pk, which
+// pass 2 filled.
 void launch_loud_gate(cudaStream_t s, const LoudTrack* d_tr, uint32_t n_tracks, const double* d_wt, const double* d_en, double* d_ws, uint64_t n_seg,
-                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks);
+                      LoudOut* d_out, double* d_cws, uint64_t n_work, LoudOut* d_chout, uint32_t ch_blocks, const float* d_pk, LoudSeries ser);
 // One record per album: its pooled momentary powers are mom[m0 .. m0 + J), its short-term powers sht[q0 .. q0 + K) (engine.cu:
 // AlbumPools).  d_keep has the size of d_sht; only the loudness fields of d_out are written.
 struct LoudAlbum {

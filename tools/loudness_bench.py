@@ -4,6 +4,7 @@
     python tools/loudness_bench.py [--tracks N] [--rounds R] [--warmup W] [--albums [M]] [--with-analysis] [--devices D] [--out FILE]
     python tools/loudness_bench.py --layout [--tracks N] [--rounds R] [--warmup W] [--out FILE]
     python tools/loudness_bench.py --baseline-lib LIB [--tracks N] [--rounds R] [--warmup W] [--out FILE]
+    python tools/loudness_bench.py --series [--tracks N] [--rounds R] [--warmup W] [--out FILE]
 
 Workload: N (default 1024) stereo three-minute 44.1 kHz PCM16 tracks, each channel a C2 track of tests/synth.py (channel 0 from
 seed i, channel 1 from seed i + 1000), generated on the device and quantised there.  Two legs (three with --albums), timed in
@@ -26,6 +27,10 @@ the C2 track i + 1000 c): three kinds, each device-resident and from pinned host
   mapped       the 7.1 map of stratum_b200_loudness_channel_map(0x63F, 8, 0, map) (stratum_b200_loudness_mapped_pcm);
   per_channel  the same map plus per-channel results (the per-channel CTAs of the gate launch and their read-back).
 Each leg reports tracks/s, wall time, the median pass 2 and gate kernel times and the device-to-host bytes of one call.
+--series measures the loudness series on the default stereo workload: without and with all four series
+(stratum_b200_loudness_series_pcm: momentary and short-term loudness, sample and true peaks per 100 ms), each device-resident and
+from pinned host memory, four legs timed in alternation; each reports tracks/s, wall time, the median pass 2 and gate kernel times and
+the device-to-host bytes of one call.
 --baseline-lib LIB times the stereo device leg of this build against another build of the library (e.g. the parent commit's), the
 two alternating, and reports each one's median, minimum and maximum pass 2 time and whether the two give the same bits.
 Reports the median over R rounds of tracks/s and wall time per leg, the median kernel times of the device leg (pass 1, the scan,
@@ -154,6 +159,64 @@ def layout_main(a, S, torch) -> dict:
     return doc
 
 
+def series_main(a, S, torch) -> dict:
+    n = a.tracks
+    L = S.lib()
+    d_pcm = make_pcm(S, torch, n)
+    h_pcm = torch.empty(d_pcm.numel(), dtype=torch.int16, pin_memory=True)
+    h_pcm.copy_(d_pcm)
+    bytes_per_track = N_FRAMES * 2 * 2
+    offsets = (np.arange(n + 1, dtype=np.uint64) * np.uint64(bytes_per_track))
+    srs, chans, fmts = np.full(n, SR, np.uint32), np.full(n, 2, np.uint32), np.full(n, S.PCM_S16, np.uint32)
+    u32 = lambda v: v.ctypes.data_as(C.POINTER(C.c_uint32))
+    off = offsets.ctypes.data_as(C.POINTER(C.c_uint64))
+    _, arrays = S._series_args(True, offsets, srs, chans, fmts)
+    ptrs = [x.ctypes.data_as(C.POINTER(C.c_double)) for x in arrays]
+    res = (S.StratumLoudness * n)()
+    kinds = {"plain": [None] * 4, "series": ptrs}
+
+    def leg(kind, where):
+        p = kinds[kind]
+        if where == "device":
+            return lambda: L.stratum_b200_loudness_series_pcm_device(C.c_void_p(d_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, None, 0, None, 0,
+                                                                     res, None, None, *p)
+        return lambda: L.stratum_b200_loudness_series_pcm(C.c_void_p(h_pcm.data_ptr()), off, u32(srs), u32(chans), u32(fmts), n, None, 0, None, None, 0, res,
+                                                          None, None, *p)
+
+    legs = {(k, w): leg(k, w) for k in kinds for w in ("device", "host")}
+
+    def timed(fn):
+        S.stage_timing(True)
+        S.stage_times(reset=True)
+        _, d2h0 = S.transfer_bytes()
+        t0 = time.perf_counter()
+        st = fn()
+        wall = time.perf_counter() - t0
+        S.stage_timing(False)
+        if st != S.OK:
+            raise SystemExit(f"loudness call failed: {S.last_error()}")
+        _, d2h1 = S.transfer_bytes()
+        return wall, S.stage_times(), sum(1 for i in range(n) if res[i].status == 0), d2h1 - d2h0
+
+    for _ in range(a.warmup):
+        for fn in legs.values():
+            timed(fn)
+    runs = {key: [] for key in legs}
+    for _ in range(a.rounds):
+        for key, fn in legs.items():
+            runs[key].append(timed(fn))
+    doc = {"workload": f"{n} stereo 3-minute 44.1 kHz PCM16 tracks (synthetic C2 pairs)", "card": card(), "rounds": a.rounds, "warmup": a.warmup,
+           "pcm_bytes": n * bytes_per_track, "series_entries": {k: int(x.size) for k, x in zip(("momentary", "short_term", "sample_peak", "true_peak"), arrays)},
+           "track0": {"momentary_max_lufs": res[0].momentary_max_lufs, "series_momentary_max_lufs": float(arrays[0][:res[0].n_momentary].max()),
+                      "true_peak": res[0].true_peak, "series_true_peak": float(arrays[3][:len(arrays[3]) // n].max())}}
+    for (kind, where), rs in runs.items():
+        wall = statistics.median(r[0] for r in rs)
+        doc[f"{kind}_{where}"] = {"tracks_per_s": n / wall, "wall_s": wall,
+                                  "stage_ms": {s: statistics.median(r[1].get(s, 0.0) for r in rs) for s in STAGES},
+                                  "d2h_bytes": statistics.median(r[3] for r in rs), "ok_tracks": min(r[2] for r in rs)}
+    return doc
+
+
 def baseline_main(a, S, torch) -> dict:
     """The stereo device leg of this build and of the library at a.baseline_lib, alternating."""
     n = a.tracks
@@ -210,6 +273,7 @@ def main() -> None:
     ap.add_argument("--with-analysis", action="store_true", help="add the analysis, separate and combined legs")
     ap.add_argument("--devices", type=int, default=1, help="host legs over devices 0..D-1")
     ap.add_argument("--layout", action="store_true", help="time channel maps and per-channel results on 7.1 tracks")
+    ap.add_argument("--series", action="store_true", help="time the loudness series against the plain measurement")
     ap.add_argument("--baseline-lib", default=None, metavar="LIB", help="time the stereo device leg of this build against the library LIB")
     ap.add_argument("--out", default=None, help="also write the JSON document to this file")
     a = ap.parse_args()
@@ -220,8 +284,8 @@ def main() -> None:
 
     if not torch.cuda.is_available() or S.device_count() < 1:
         raise SystemExit("loudness_bench needs a CUDA device: the measurement has no CPU fallback")
-    if a.layout or a.baseline_lib:
-        doc = layout_main(a, S, torch) if a.layout else baseline_main(a, S, torch)
+    if a.layout or a.baseline_lib or a.series:
+        doc = layout_main(a, S, torch) if a.layout else (series_main(a, S, torch) if a.series else baseline_main(a, S, torch))
         s = json.dumps(doc, indent=1)
         print(s)
         if a.out:
